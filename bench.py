@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """Benchmark of the abdpymc inference hot path on B200 (see DESIGN.md, "Measurement").
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (BASELINE.json configs[2], the configuration the metric is quoted on): the simulated
@@ -18,6 +18,9 @@ independent replicas of the cohort + chain state whose total footprint exceeds t
 `e2e` = the same metric through the host-pointer C-ABI call abd_logp_dlogp(q17, i_raw, waner)
 with pinned HOST buffers: every call copies all three inputs to the device and the results back.
 The `gibbs` object reports abd_gibbs_sweep the same way (its own timed regions).
+--dump-outputs DIR writes what the last timed step returned to its caller, DIR/logp.npy (C,) and
+DIR/dlogp.npy (C, 17), float64, all ranks' chains: the inputs are seeded, so two builds can be
+compared output for output.
 """
 from __future__ import annotations
 
@@ -34,6 +37,8 @@ import numpy as np
 
 ROOT = Path(__file__).resolve().parent
 sys.path.insert(0, str(ROOT))
+# the benchmark leaves the tree as it found it (which may be read-only): no __pycache__ directories
+sys.dont_write_bytecode = True
 
 N_INDS = 10_000
 N_CHAINS = 4
@@ -595,6 +600,24 @@ def bench_ess(eng, co, C, dev, rank, world, dist, tune_n, draws_n, cpu):
     return ess
 
 
+def dump_outputs(directory, last_step, dist, rank, world):
+    """logp.npy / dlogp.npy of the last timed step, every rank's chains in rank order (written by rank 0)."""
+    import torch
+
+    arrays = {}
+    for name, t in zip(("logp", "dlogp"), last_step):
+        if dist:
+            parts = [torch.empty_like(t) for _ in range(world)]
+            dist.all_gather(parts, t)
+            t = torch.cat(parts)
+        arrays[name] = t.cpu().numpy()
+    if rank == 0:
+        d = Path(directory)
+        d.mkdir(parents=True, exist_ok=True)
+        for name, a in arrays.items():
+            np.save(d / f"{name}.npy", a.astype(np.float64))
+
+
 # ------------------------------------------------------------------------------------------
 def run_gpu(args):
     import torch
@@ -703,6 +726,7 @@ def run_gpu(args):
         e1.record()
         barrier()
         ms = e0.elapsed_time(e1)
+        last_step = (out.clone(), outg.clone())
         # keep the sampler alive long enough for at least a few samples under load
         t_end = time.time() + max(0.0, 0.6 - ms / 1e3)
         while time.time() < t_end:
@@ -714,6 +738,8 @@ def run_gpu(args):
         t = torch.tensor([ms], dtype=torch.float64, device=dev)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         ms = float(t.item())
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, last_step, dist, rank, world)
     n_launch = K * EVALS_PER_STEP
     value = world * C * n_launch / (ms / 1e3)
     t_kernel = ms / 1e3 / n_launch
@@ -1106,7 +1132,13 @@ def main():
     ap.add_argument("--ess128-draws", type=int, default=2000)
     ap.add_argument("--profile", action="store_true",
                     help="short run for ncu: a few un-captured logp+grad launches and Gibbs sweeps, no JSON line")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed step's logp and gradient of every chain as DIR/logp.npy, DIR/dlogp.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.profile):
+        ap.error("--dump-outputs needs the timed CUDA path (not --impl reference or --profile)")
     # Exactly ONE line goes to stdout (rank 0's JSON): libraries that chat on stdout (NCCL prints its
     # version there) are sent to stderr for the whole run.
     global _REAL_STDOUT

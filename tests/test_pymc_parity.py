@@ -1,39 +1,33 @@
-"""Parity against a LIVE PyMC + the reference package, whenever both are importable.
+"""Parity of the joint logp and its gradient with the reference model (abdpymc's ``abd.model``, PyMC's
+unconstrained space) on the bundled test cohort, for the one-, two- and three-chunk models.
 
-Neither is installable in the offline build image (DESIGN.md section 5), so this file is skipped
-there; it is the test that turns "restated from PyMC's documentation" into "pinned" on any
-machine that has `pip install pymc abdpymc`."""
+The reference's values are stored in tests/golden/model_goldens.npz: tests/golden/make_golden.py evaluated
+the reference's own ``abd.py`` at each point (PyTensor / PyMC primitives restated in NumPy by
+tests/golden/refshim.py and validated by the reference's unit tests; gradient by complex-step
+differentiation), so the comparison needs neither PyMC nor the reference package."""
 import numpy as np
 import pytest
-
-pm = pytest.importorskip("pymc")
-ref = pytest.importorskip("abdpymc")
 
 pytestmark = pytest.mark.gpu
 
 
 @pytest.mark.parametrize("splits", [None, (14,), (14, 20)])
-def test_logp_dlogp_matches_pymc(splits, tmp_path):
-    from abdpymc_b200.cohort import CohortArrays
-    from abdpymc_b200.engine import Q17, AbdEngine
+def test_logp_dlogp_matches_pymc(splits, goldens, cohorts):
+    import torch
 
-    co = CohortArrays.load("test_cohort")
-    co.to_disk(tmp_path / "cohort_data")
-    data = ref.TiterData.from_disk(str(tmp_path / "cohort_data"))
-    model = ref.model(data, splits=splits)
-    fn = model.logp_dlogp_function()
-    rng = np.random.default_rng(0)
-    with AbdEngine(co, splits=splits) as eng:
-        for _ in range(8):
-            point = model.initial_point()
-            for k in point:
-                if point[k].dtype.kind == "f":
-                    point[k] = point[k] + rng.normal(scale=0.3, size=point[k].shape)
-            point["i_raw"] = (rng.random(point["i_raw"].shape) < 0.05).astype(point["i_raw"].dtype)
-            point["ab_s_waner"] = (rng.random(point["ab_s_waner"].shape) < 0.5).astype(point["ab_s_waner"].dtype)
-            fn.set_extra_values(point)
-            q = np.array([float(point[name]) for name in Q17])
-            lp_ref, g_ref = fn(fn.array_to_dict(q) if hasattr(fn, "array_to_dict") else q)
-            lp, g = eng.logp_dlogp(q, point["i_raw"], point["ab_s_waner"])
+    if not torch.cuda.is_available():
+        pytest.skip("no CUDA device")
+    from abdpymc_b200 import build
+    from abdpymc_b200.engine import AbdEngine
+
+    build.build()
+    z, cases = goldens
+    keys = [c["key"] for c in cases
+            if c["cohort"] == "test_cohort" and not c["ignore_pcrpos"] and tuple(c["splits"]) == (splits or ())]
+    assert len(keys) >= 8
+    with AbdEngine(cohorts["test_cohort"], splits=splits) as eng:
+        for k in keys:
+            lp_ref, g_ref = float(z[f"{k}/logp"]), z[f"{k}/grad"]
+            lp, g = eng.logp_dlogp(z[f"{k}/q"], z[f"{k}/i_raw"], z[f"{k}/w"])
             assert abs(lp - lp_ref) <= 1e-10 * abs(lp_ref)
             np.testing.assert_allclose(g, g_ref, rtol=1e-9, atol=1e-9)
