@@ -14,7 +14,7 @@ from pathlib import Path
 PKG = Path(__file__).resolve().parent
 LIB_PATH = Path(os.environ.get("ABD_B200_LIB", PKG / "libabd_b200.so"))  # override: developer builds only
 
-N_THETA, N_Q, N_SUMS, MAX_GAPS = 13, 17, 16, 63
+N_THETA, N_Q, N_SUMS, MAX_GAPS = 13, 17, 16, 127
 GIBBS_METROPOLIS, GIBBS_HEATBATH, GIBBS_BLOCKED = 0, 1, 2
 
 c_double_p = C.POINTER(C.c_double)

@@ -1,10 +1,11 @@
 // libabd_b200.so -- kernels (sm_100a) and the C ABI declared in include/abd_b200.h.
 //
 // HBM layout (all built once in abd_create, see DESIGN.md):
-//   pcr[N], vac[N]              one bit mask over gaps per individual (uint32 if G <= 31)
+//   pcr[N], vac[N]              one bit mask over gaps per individual: uint32 (G <= 31), uint64 (G <= 63) or
+//                               128 bits (G <= 127), see with_mask
 //   per antigen a in {N, S}:    CSR by individual -- rp_a[N+1] (int32), and row arrays sorted by
 //                               (individual, gap): od_a[R_a] f64, x_a[R_a] f64,
-//                               meta_a[R_a] u32 = individual << 6 | gap
+//                               meta_a[R_a] u32 = individual << 6 | gap (<< 7 with 128-bit masks)
 //   per chain (resident state): i_raw[C][G][N] int8, waner[C][N] int8  (the reference layout), and beside it
 //                               PackedState[C][N] (raw bit mask | waner, constrained infections): what the kernels read
 //
@@ -69,7 +70,7 @@ int fail(int code, const std::string& msg) {
 struct abd_handle {
   int device = 0;
   int G = 0, N = 0;
-  bool wide = false;  // uint64 masks
+  int mask_bits = 32;  // gap-mask layout (32, 64 or 128 bits): read through with_mask only
   int64_t R[2] = {0, 0};
   Totals tot{};
   DevCohort dc{};
@@ -139,6 +140,17 @@ struct abd_handle {
 
 namespace {
 
+// The one place that turns a handle's mask layout into the kernels' mask type: returns f(M{}) for M = uint32_t,
+// uint64_t or u128.
+template <typename F>
+auto with_mask(const abd_handle* h, F&& f) {
+  if (h->mask_bits == 128) return f(u128{});
+  if (h->mask_bits == 64) return f(uint64_t{});
+  return f(uint32_t{});
+}
+// mask layout for a cohort of G gaps: the narrowest that holds G gaps and the waner bit
+int mask_bits_for(int G) { return G <= 31 ? 32 : (G <= 63 ? 64 : 128); }
+
 template <typename T>
 int dev_alloc(abd_handle* h, T** p, size_t n, bool owned = true) {
   void* q = nullptr;
@@ -193,6 +205,7 @@ Priors default_priors(int G) {
 int build_rows(abd_handle* h, int a, int64_t R, const double* x, const double* od, const int32_t* gap,
                const int32_t* ind) {
   const int N = h->N, G = h->G;
+  const int gap_bits = with_mask(h, [](auto m) { return kGapBits<decltype(m)>; });
   if (R > 0 && (!x || !od || !gap || !ind)) return fail(ABD_ERR_INVALID, "NULL row array");
   if (R >= (int64_t)1 << 31) return fail(ABD_ERR_INVALID, "too many OD rows for int32 CSR");
   std::vector<int>& rp = h->h_rp[a];
@@ -224,7 +237,7 @@ int build_rows(abd_handle* h, int a, int64_t R, const double* x, const double* o
     perm[(size_t)k] = (int)r;
     xs[(size_t)k] = x[r];
     ods[(size_t)k] = od[r];
-    const uint32_t m = ((uint32_t)ind[r] << 6) | (uint32_t)gap[r];
+    const uint32_t m = ((uint32_t)ind[r] << gap_bits) | (uint32_t)gap[r];
     meta[(size_t)k] = m;
     if (cmeta.empty() || cmeta.back() != m) {
       cmeta.push_back(m);
@@ -362,7 +375,8 @@ int ensure_chains(abd_handle* h, int C) {
   h->pack_valid = 0;
   {
     char* pk = nullptr;
-    if ((rc = dev_alloc(h, &pk, (size_t)C * h->N * (h->wide ? 16 : 8), false))) return rc;
+    const size_t entry = with_mask(h, [](auto m) { return sizeof(PackedState<decltype(m)>); });
+    if ((rc = dev_alloc(h, &pk, (size_t)C * h->N * entry, false))) return rc;
     h->d_pack = pk;
   }
   if ((rc = dev_alloc(h, &h->d_theta, (size_t)C * 17, false))) return rc;
@@ -469,12 +483,11 @@ cudaError_t sums_occupancy(int device, size_t smem, int* occ) {
 }
 // resident CTAs per SM of the plain-evaluation kernel for this handle's mask width / dilution mode
 cudaError_t sums_occupancy_h(const abd_handle* h, bool compact, size_t smem, int* occ) {
-  if (compact) return h->wide ? sums_occupancy<uint64_t, uint8_t, true>(h->device, smem, occ)
-                              : sums_occupancy<uint32_t, uint8_t, true>(h->device, smem, occ);
-  if (h->wide) return h->fx ? sums_occupancy<uint64_t, uint8_t, false>(h->device, smem, occ)
-                            : sums_occupancy<uint64_t, double, false>(h->device, smem, occ);
-  return h->fx ? sums_occupancy<uint32_t, uint8_t, false>(h->device, smem, occ)
-               : sums_occupancy<uint32_t, double, false>(h->device, smem, occ);
+  return with_mask(h, [&](auto m) {
+    using M = decltype(m);
+    if (compact) return sums_occupancy<M, uint8_t, true>(h->device, smem, occ);
+    return h->fx ? sums_occupancy<M, uint8_t, false>(h->device, smem, occ) : sums_occupancy<M, double, false>(h->device, smem, occ);
+  });
 }
 
 // The packed copy of the resident chain state for a launch that reads (i_raw, waner): non-null only
@@ -486,8 +499,10 @@ int resident_pack(abd_handle* h, int C, const int8_t* i_raw, const int8_t* waner
   if (h->pack_valid < C) {
     if (!h->lazy_pack) return ABD_OK;
     dim3 grid((h->N + 127) / 128, C);
-    if (h->wide) k_pack<uint64_t><<<grid, 128, 0, st>>>(h->dc, h->d_iraw, h->d_waner, (PackedState<uint64_t>*)h->d_pack);
-    else k_pack<uint32_t><<<grid, 128, 0, st>>>(h->dc, h->d_iraw, h->d_waner, (PackedState<uint32_t>*)h->d_pack);
+    with_mask(h, [&](auto m) {
+      using M = decltype(m);
+      k_pack<M><<<grid, 128, 0, st>>>(h->dc, h->d_iraw, h->d_waner, (PackedState<M>*)h->d_pack);
+    });
     CU(cudaGetLastError());
     h->launches++;
     h->pack_valid = C;
@@ -619,12 +634,14 @@ int launch_sums(abd_handle* h, int C, const double* theta, int theta_is_q, const
   h->last_plan[3] = (int)(compact ? tl->smem_cp : tl->smem), h->last_plan[4] = compact ? 1 : 0, h->last_plan[5] = tl_occ;
   void* pack = nullptr;
   if ((rc = resident_pack(h, C, i_raw, waner, st, &pack))) return rc;
-#define ABD_LAUNCH_SUMS(M_, XT_, CP_) \
-  launch_sums_t<M_, XT_, CP_>(h, *tl, cfg, grid, theta, theta_is_q, i_raw, waner, pack, sums, fin, traj, st, thin)
-  if (compact) rc = h->wide ? ABD_LAUNCH_SUMS(uint64_t, uint8_t, true) : ABD_LAUNCH_SUMS(uint32_t, uint8_t, true);
-  else if (h->wide) rc = h->fx ? ABD_LAUNCH_SUMS(uint64_t, uint8_t, false) : ABD_LAUNCH_SUMS(uint64_t, double, false);
-  else rc = h->fx ? ABD_LAUNCH_SUMS(uint32_t, uint8_t, false) : ABD_LAUNCH_SUMS(uint32_t, double, false);
+  rc = with_mask(h, [&](auto m) {
+    using M = decltype(m);
+#define ABD_LAUNCH_SUMS(XT_, CP_) \
+  launch_sums_t<M, XT_, CP_>(h, *tl, cfg, grid, theta, theta_is_q, i_raw, waner, pack, sums, fin, traj, st, thin)
+    if (compact) return ABD_LAUNCH_SUMS(uint8_t, true);
+    return h->fx ? ABD_LAUNCH_SUMS(uint8_t, false) : ABD_LAUNCH_SUMS(double, false);
 #undef ABD_LAUNCH_SUMS
+  });
   if (rc) return rc;
   CU(cudaGetLastError());
   h->launches++;
@@ -634,8 +651,8 @@ int launch_sums(abd_handle* h, int C, const double* theta, int theta_is_q, const
 int launch_gibbs(abd_handle* h, int C, const double* theta, int theta_is_q, const double* p,
                  const double* pw, int8_t* i_raw, int8_t* waner, const GibbsCfg& cfg, cudaStream_t st) {
   if (cfg.mode == ABD_GIBBS_BLOCKED) {
-    if (h->wide || h->dc.ch.n < 2) {
-      // no "first raw 1 of the chunk" structure (one chunk) or more options than lanes (wide masks):
+    if (h->mask_bits > 32 || h->dc.ch.n < 2) {
+      // no "first raw 1 of the chunk" structure (one chunk) or more options than lanes (masks wider than 32 bits):
       // single-site exact conditionals instead
       GibbsCfg c2 = cfg;
       c2.mode = ABD_GIBBS_HEATBATH;
@@ -660,10 +677,9 @@ int launch_gibbs(abd_handle* h, int C, const double* theta, int theta_is_q, cons
   }
   if (!h->gibbs_ctas) {
     int occ = 0;
-    if (h->wide)
-      CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_gibbs<uint64_t>, kGibbsWarps * 32, 0));
-    else
-      CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_gibbs<uint32_t>, kGibbsWarps * 32, 0));
+    CU(with_mask(h, [&](auto m) {
+      return cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_gibbs<decltype(m)>, kGibbsWarps * 32, 0);
+    }));
     h->gibbs_ctas = h->n_sms * std::max(occ, 1);
   }
   const long items = (long)C * h->N;
@@ -672,12 +688,11 @@ int launch_gibbs(abd_handle* h, int C, const double* theta, int theta_is_q, cons
   void* pack = nullptr;
   int rcp = resident_pack(h, C, i_raw, waner, st, &pack);
   if (rcp) return rcp;
-  if (h->wide)
-    k_gibbs<uint64_t><<<grid, kGibbsWarps * 32, 0, st>>>(h->dc, h->d_order, C, theta, theta_is_q, p, pw, i_raw, waner,
-                                                          (PackedState<uint64_t>*)pack, h->d_queue, cfg);
-  else
-    k_gibbs<uint32_t><<<grid, kGibbsWarps * 32, 0, st>>>(h->dc, h->d_order, C, theta, theta_is_q, p, pw, i_raw, waner,
-                                                          (PackedState<uint32_t>*)pack, h->d_queue, cfg);
+  with_mask(h, [&](auto m) {
+    using M = decltype(m);
+    k_gibbs<M><<<grid, kGibbsWarps * 32, 0, st>>>(h->dc, h->d_order, C, theta, theta_is_q, p, pw, i_raw, waner,
+                                                   (PackedState<M>*)pack, h->d_queue, cfg);
+  });
   CU(cudaGetLastError());
   h->launches++;
   return ABD_OK;
@@ -745,7 +760,7 @@ int stage_state(abd_handle* h, int C, const int8_t* i_raw, const int8_t* waner) 
 }
 
 // A handle with its device facts, stream and environment switches (everything that does not depend on the cohort)
-int new_handle(abd_handle** out, int device, int G, int N) {
+int new_handle(abd_handle** out, int device, int G, int N, int mask_bits) {
   abd_handle* h = new abd_handle();
   h->device = device;
   if (const char* e = std::getenv("ABD_B200_NO_PDL")) h->use_pdl = !(e[0] == '1');
@@ -761,7 +776,7 @@ int new_handle(abd_handle** out, int device, int G, int N) {
   }
   h->G = G;
   h->N = N;
-  h->wide = G > 31;
+  h->mask_bits = mask_bits;
   if (cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking) != cudaSuccess) {
     abd_destroy(h);
     return fail(ABD_ERR_CUDA, "cudaStreamCreate failed");
@@ -787,13 +802,15 @@ struct CacheHeader {
   char magic[8];           // "ABDB200\0"
   int32_t version, G, N, n_chunks;
   uint64_t chunk_mask[3];
-  int32_t wide, fx, n_xlev, has_pcr;
+  int32_t wide, fx, n_xlev, has_pcr;   // wide: mask layout, 0 = 32, 1 = 64, 2 = 128 bits
   int64_t R[2], K[2];      // OD rows / (individual, gap) cells per antigen (N, S)
   double tot[4];
   uint32_t ind_offset, pad;
   double xlev[kMaxXLevels];
 };
-constexpr int kCacheVersion = 2;
+// Version 2: 32- and 64-bit masks.  Version 3 (128-bit masks): the same header, then the chunk masks' high words
+// (gaps 64..127) before the arrays.
+constexpr int kCacheVersion = 2, kCacheVersionWide = 3;
 
 struct CacheIo {
   FILE* f = nullptr;
@@ -831,15 +848,17 @@ int cache_array(abd_handle* h, CacheIo& io, T** dptr, size_t n, std::vector<T>* 
 int cache_body(abd_handle* h, CacheIo& io, const CacheHeader& hd) {
   int rc;
   const size_t N = (size_t)hd.N;
-  if (hd.wide) {
-    uint64_t *p = (uint64_t*)h->dc.pcr, *v = (uint64_t*)h->dc.vac;
-    if ((rc = cache_array(h, io, &p, N)) || (rc = cache_array(h, io, &v, N))) return rc;
-    h->dc.pcr = p, h->dc.vac = v;
-  } else {
-    uint32_t *p = (uint32_t*)h->dc.pcr, *v = (uint32_t*)h->dc.vac;
-    if ((rc = cache_array(h, io, &p, N)) || (rc = cache_array(h, io, &v, N))) return rc;
-    h->dc.pcr = p, h->dc.vac = v;
-  }
+  rc = with_mask(h, [&](auto m) {
+    using M = decltype(m);
+    M *p = (M*)h->dc.pcr, *v = (M*)h->dc.vac;
+    const int r = cache_array(h, io, &p, N);
+    if (r) return r;
+    h->dc.pcr = p;
+    const int r2 = cache_array(h, io, &v, N);
+    h->dc.vac = v;
+    return r2;
+  });
+  if (rc) return rc;
   for (int a = 0; a < 2; ++a) {
     const size_t R = (size_t)hd.R[a], K = (size_t)hd.K[a];
     int* rp = (int*)h->dc.rp[a];
@@ -915,8 +934,13 @@ int abd_create(abd_handle** out, const abd_cohort* co, int device) {
   if (!out || !co) return fail(ABD_ERR_INVALID, "NULL argument");
   *out = nullptr;
   const int G = co->n_gaps, N = co->n_inds;
-  if (G < 1 || G > ABD_MAX_GAPS) return fail(ABD_ERR_INVALID, "n_gaps must be in [1, 63]");
+  if (G < 1 || G > ABD_MAX_GAPS) return fail(ABD_ERR_INVALID, "n_gaps must be in [1, 127]");
   if (N < 1 || N >= (1 << 26)) return fail(ABD_ERR_INVALID, "n_inds must be in [1, 2^26)");
+  // ABD_B200_MASK_BITS=128 (tests, measurements): the 128-bit layout whatever G
+  const char* mb = std::getenv("ABD_B200_MASK_BITS");
+  const int mask_bits = (mb && std::strcmp(mb, "128") == 0) ? 128 : mask_bits_for(G);
+  if (mask_bits == 128 && N >= (1 << 25))
+    return fail(ABD_ERR_INVALID, "n_inds must be < 2^25 with more than 63 gaps (128-bit masks)");
   if (!co->vacs) return fail(ABD_ERR_INVALID, "vacs is NULL");
   // check_splits, abd.py:604-622
   if (co->n_splits < 0 || co->n_splits > 2)
@@ -936,7 +960,7 @@ int abd_create(abd_handle** out, const abd_cohort* co, int device) {
 
   abd_handle* h = nullptr;
   {
-    int rc0 = new_handle(&h, device, G, N);
+    int rc0 = new_handle(&h, device, G, N, mask_bits);
     if (rc0) return rc0;
   }
   auto bail = [&](int rc) {
@@ -945,25 +969,23 @@ int abd_create(abd_handle** out, const abd_cohort* co, int device) {
   };
 
   // bit masks per individual
-  std::vector<uint64_t> pcr((size_t)N, 0), vac((size_t)N, 0);
+  std::vector<u128> pcr((size_t)N, 0), vac((size_t)N, 0);
   for (int t = 0; t < G; ++t)
     for (int n = 0; n < N; ++n) {
-      if (co->pcrpos && co->pcrpos[(size_t)t * N + n]) pcr[n] |= 1ull << t;
-      if (co->vacs[(size_t)t * N + n]) vac[n] |= 1ull << t;
+      if (co->pcrpos && co->pcrpos[(size_t)t * N + n]) pcr[n] |= (u128)1 << t;
+      if (co->vacs[(size_t)t * N + n]) vac[n] |= (u128)1 << t;
     }
-  int rc;
-  if (h->wide) {
-    uint64_t *dp, *dv;
-    if ((rc = upload(h, &dp, pcr)) || (rc = upload(h, &dv, vac))) return bail(rc);
+  int rc = with_mask(h, [&](auto m) {
+    using M = decltype(m);
+    std::vector<M> pm(pcr.begin(), pcr.end()), vm(vac.begin(), vac.end());
+    M *dp, *dv;
+    int r;
+    if ((r = upload(h, &dp, pm)) || (r = upload(h, &dv, vm))) return r;
     h->dc.pcr = dp;
     h->dc.vac = dv;
-  } else {
-    std::vector<uint32_t> p32(pcr.begin(), pcr.end()), v32(vac.begin(), vac.end());
-    uint32_t *dp, *dv;
-    if ((rc = upload(h, &dp, p32)) || (rc = upload(h, &dv, v32))) return bail(rc);
-    h->dc.pcr = dp;
-    h->dc.vac = dv;
-  }
+    return ABD_OK;
+  });
+  if (rc) return bail(rc);
   h->dc.G = G;
   h->dc.N = N;
   h->dc.ind_offset = (unsigned)co->ind_offset;
@@ -974,9 +996,9 @@ int abd_create(abd_handle** out, const abd_cohort* co, int device) {
     int edges[4] = {0, 0, 0, 0};
     for (int k = 0; k < co->n_splits; ++k) edges[k + 1] = co->splits[k];
     edges[co->n_splits + 1] = G;
-    for (int k = 0; k < 3; ++k) h->dc.ch.mask[k] = 0;
+    for (int k = 0; k < 3; ++k) h->dc.ch.mask[k] = h->dc.ch.mask_hi[k] = 0;
     for (int k = 0; k <= co->n_splits; ++k)
-      for (int t = edges[k]; t < edges[k + 1]; ++t) h->dc.ch.mask[k] |= 1ull << t;
+      for (int t = edges[k]; t < edges[k + 1]; ++t) (t < 64 ? h->dc.ch.mask[k] : h->dc.ch.mask_hi[k]) |= 1ull << (t & 63);
   }
   // distinct dilutions over both antigens: <= 32 of them (and no NaN) enables the factored mode
   {
@@ -1038,9 +1060,10 @@ int abd_save_cache(abd_handle* h, const char* path) {
   CU(cudaStreamSynchronize(h->stream));
   CacheHeader hd{};
   std::memcpy(hd.magic, "ABDB200", 8);
-  hd.version = kCacheVersion, hd.G = h->G, hd.N = h->N, hd.n_chunks = h->dc.ch.n;
+  const bool v3 = h->mask_bits == 128;
+  hd.version = v3 ? kCacheVersionWide : kCacheVersion, hd.G = h->G, hd.N = h->N, hd.n_chunks = h->dc.ch.n;
   for (int k = 0; k < 3; ++k) hd.chunk_mask[k] = h->dc.ch.mask[k];
-  hd.wide = h->wide, hd.fx = h->fx, hd.n_xlev = h->dc.n_xlev, hd.has_pcr = h->has_pcr;
+  hd.wide = h->mask_bits == 128 ? 2 : (h->mask_bits == 64 ? 1 : 0), hd.fx = h->fx, hd.n_xlev = h->dc.n_xlev, hd.has_pcr = h->has_pcr;
   for (int a = 0; a < 2; ++a) hd.R[a] = h->R[a], hd.K[a] = h->h_cp[a].empty() ? 0 : h->h_cp[a].back();
   hd.tot[0] = h->tot.rows_n, hd.tot[1] = h->tot.rows_s, hd.tot[2] = h->tot.bits_i, hd.tot[3] = h->tot.bits_w;
   hd.ind_offset = h->dc.ind_offset;
@@ -1050,6 +1073,7 @@ int abd_save_cache(abd_handle* h, const char* path) {
   io.f = std::fopen(path, "wb");
   if (!io.f) return fail(ABD_ERR_INVALID, std::string("cannot write ") + path);
   io.raw(&hd, sizeof(hd));
+  if (v3) io.raw(h->dc.ch.mask_hi, sizeof(h->dc.ch.mask_hi));
   if ((rc = cache_body(h, io, hd))) return rc;
   return io.ok ? ABD_OK : fail(ABD_ERR_INVALID, "cache file I/O error");
 }
@@ -1063,8 +1087,14 @@ int abd_create_from_cache(abd_handle** out, const char* path, int device) {
   CacheHeader hd{};
   io.raw(&hd, sizeof(hd));
   if (!io.ok || std::memcmp(hd.magic, "ABDB200", 8) != 0) return fail(ABD_ERR_INVALID, "not an abd_b200 cache file");
-  if (hd.version != kCacheVersion) return fail(ABD_ERR_INVALID, "cache file of another version: rebuild it");
-  if (hd.G < 1 || hd.G > ABD_MAX_GAPS || hd.N < 1 || hd.N >= (1 << 26) || hd.n_chunks < 1 || hd.n_chunks > 3 ||
+  if (hd.version != kCacheVersion && hd.version != kCacheVersionWide)
+    return fail(ABD_ERR_INVALID, "cache file of another version: rebuild it");
+  const bool v3 = hd.version == kCacheVersionWide;
+  const int mask_bits = v3 ? 128 : (hd.wide ? 64 : 32);
+  uint64_t mask_hi[3] = {0, 0, 0};
+  if (v3) io.raw(mask_hi, sizeof(mask_hi));
+  if (!io.ok || hd.G < 1 || hd.G > ABD_MAX_GAPS || hd.N < 1 || hd.N >= (mask_bits == 128 ? (1 << 25) : (1 << 26)) ||
+      hd.n_chunks < 1 || hd.n_chunks > 3 || hd.wide != (v3 ? 2 : (hd.G > 31 ? 1 : 0)) || (!v3 && hd.G > 63) ||
       hd.R[0] < 0 || hd.R[1] < 0 || hd.K[0] < 0 || hd.K[1] < 0 || hd.n_xlev < 0 || hd.n_xlev > kMaxXLevels)
     return fail(ABD_ERR_INVALID, "corrupt cache header");
   int ndev = 0;
@@ -1072,7 +1102,7 @@ int abd_create_from_cache(abd_handle** out, const char* path, int device) {
   if (device < 0 || device >= ndev) return fail(ABD_ERR_CUDA, "no such CUDA device");
   CU(cudaSetDevice(device));
   abd_handle* h = nullptr;
-  int rc = new_handle(&h, device, hd.G, hd.N);
+  int rc = new_handle(&h, device, hd.G, hd.N, mask_bits);
   if (rc) return rc;
   auto bail = [&](int r) {
     abd_destroy(h);
@@ -1080,7 +1110,7 @@ int abd_create_from_cache(abd_handle** out, const char* path, int device) {
   };
   h->dc.G = hd.G, h->dc.N = hd.N, h->dc.ind_offset = hd.ind_offset, h->dc.chain_offset = 0;
   h->dc.ch.n = hd.n_chunks;
-  for (int k = 0; k < 3; ++k) h->dc.ch.mask[k] = hd.chunk_mask[k];
+  for (int k = 0; k < 3; ++k) h->dc.ch.mask[k] = hd.chunk_mask[k], h->dc.ch.mask_hi[k] = mask_hi[k];
   h->fx = hd.fx != 0, h->has_pcr = hd.has_pcr != 0;
   h->x_levels.assign(hd.xlev, hd.xlev + hd.n_xlev);
   {
@@ -1101,7 +1131,10 @@ int abd_cohort_info(const abd_handle* h, int32_t* n_splits, int32_t* splits, int
   const int ns = h->dc.ch.n - 1;
   if (n_splits) *n_splits = ns;
   if (splits)
-    for (int k = 0; k < ns; ++k) splits[k] = h->dc.ch.mask[k + 1] ? __builtin_ctzll(h->dc.ch.mask[k + 1]) : h->G;
+    for (int k = 0; k < ns; ++k) {
+      const uint64_t lo = h->dc.ch.mask[k + 1], hi = h->dc.ch.mask_hi[k + 1];
+      splits[k] = lo ? __builtin_ctzll(lo) : (hi ? 64 + __builtin_ctzll(hi) : h->G);
+    }
   if (has_pcrpos) *has_pcrpos = h->has_pcr ? 1 : 0;
   return ABD_OK;
 }
@@ -1434,8 +1467,9 @@ int abd_loglik_rows_dev(abd_handle* h, int C, const double* theta13, const int8_
     double* out = a ? out_s : out_n;
     if (!out || h->R[a] == 0) continue;
     dim3 grid((unsigned)((h->R[a] + 255) / 256), C);
-    if (h->wide) k_loglik_rows<uint64_t><<<grid, 256, 0, st>>>(h->dc, a, (int)h->R[a], theta13, i_raw, waner, out);
-    else k_loglik_rows<uint32_t><<<grid, 256, 0, st>>>(h->dc, a, (int)h->R[a], theta13, i_raw, waner, out);
+    with_mask(h, [&](auto m) {
+      k_loglik_rows<decltype(m)><<<grid, 256, 0, st>>>(h->dc, a, (int)h->R[a], theta13, i_raw, waner, out);
+    });
     CU(cudaGetLastError());
     h->launches++;
   }
@@ -1511,13 +1545,11 @@ int abd_deterministics_dev(abd_handle* h, int C, const double* theta13, const in
   dim3 grid((h->N + 127) / 128, C);
   const cudaStream_t st = (cudaStream_t)stream;
   const bool big = (size_t)C * 17 * h->G * h->N > ((size_t)64 << 20);  // outputs beyond half the L2: stream them
-  if (h->wide) {
-    if (big) k_determ<uint64_t, true><<<grid, 128, 0, st>>>(h->dc, theta13, i_raw, waner, out_i, out_mu_n, out_mu_s);
-    else k_determ<uint64_t, false><<<grid, 128, 0, st>>>(h->dc, theta13, i_raw, waner, out_i, out_mu_n, out_mu_s);
-  } else {
-    if (big) k_determ<uint32_t, true><<<grid, 128, 0, st>>>(h->dc, theta13, i_raw, waner, out_i, out_mu_n, out_mu_s);
-    else k_determ<uint32_t, false><<<grid, 128, 0, st>>>(h->dc, theta13, i_raw, waner, out_i, out_mu_n, out_mu_s);
-  }
+  with_mask(h, [&](auto m) {
+    using M = decltype(m);
+    if (big) k_determ<M, true><<<grid, 128, 0, st>>>(h->dc, theta13, i_raw, waner, out_i, out_mu_n, out_mu_s);
+    else k_determ<M, false><<<grid, 128, 0, st>>>(h->dc, theta13, i_raw, waner, out_i, out_mu_n, out_mu_s);
+  });
   CU(cudaGetLastError());
   h->launches++;
   return ABD_OK;
@@ -1529,10 +1561,9 @@ int abd_deterministics_accum_dev(abd_handle* h, int C, const double* theta, int 
   if (!theta || !i_raw || !waner) return fail(ABD_ERR_INVALID, "NULL argument");
   const int grid = (h->N + 127) / 128;
   const cudaStream_t st = (cudaStream_t)stream;
-  if (h->wide)
-    k_determ_accum<uint64_t><<<grid, 128, 0, st>>>(h->dc, C, theta, theta_is_q17, i_raw, waner, sum_i, sum_mu_n, sum_mu_s);
-  else
-    k_determ_accum<uint32_t><<<grid, 128, 0, st>>>(h->dc, C, theta, theta_is_q17, i_raw, waner, sum_i, sum_mu_n, sum_mu_s);
+  with_mask(h, [&](auto m) {
+    k_determ_accum<decltype(m)><<<grid, 128, 0, st>>>(h->dc, C, theta, theta_is_q17, i_raw, waner, sum_i, sum_mu_n, sum_mu_s);
+  });
   CU(cudaGetLastError());
   h->launches++;
   return ABD_OK;

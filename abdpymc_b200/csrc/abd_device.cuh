@@ -13,7 +13,14 @@
 
 namespace abd {
 
-constexpr int kMaxGaps = 64;   // mask width; usable gaps <= 63 (one lane slot is the waner bit)
+// Gap masks are uint32_t (G <= 31), uint64_t (G <= 63) or u128 (G <= 127): the top bit of a mask word carries the
+// waner bit (PackedState.rw, IndState.vacw).
+using u128 = unsigned __int128;
+// Length of the per-gap tables a kernel instantiated for mask type M keeps in shared memory (powers of rho, visiting
+// order): one entry per mask bit, but at least 64, the size the 32- and 64-bit kernels were tuned with (the grid
+// planner derives tiles and chains per CTA from their occupancy).
+template <typename M>
+constexpr int kGapTab = sizeof(M) * 8 > 64 ? (int)sizeof(M) * 8 : 64;
 constexpr int kNSums = 16;
 constexpr double kHalfLog2Pi = 0.918938533204672741780329736406;  // log(sqrt(2 pi))
 
@@ -38,6 +45,7 @@ constexpr int kQ_P = 0, kQ_PW = 7;
 struct Chunks {
   int n;               // number of time chunks (1 => OneTimeChunk rule)
   uint64_t mask[3];    // bit t set <=> gap t belongs to the chunk
+  uint64_t mask_hi[3]; // the same for gaps 64..127 (128-bit layout only)
 };
 
 struct Totals {        // sizes over ALL shards (Bernoulli terms and likelihood constants)
@@ -59,6 +67,26 @@ __device__ __forceinline__ int ctz(uint32_t v) { return __ffs((int)v) - 1; }
 __device__ __forceinline__ int ctz(uint64_t v) { return __ffsll((long long)v) - 1; }
 __device__ __forceinline__ int popc(uint32_t v) { return __popc(v); }
 __device__ __forceinline__ int popc(uint64_t v) { return __popcll(v); }
+__device__ __forceinline__ int ctz(u128 v) {
+  const int lo = __ffsll((long long)(uint64_t)v), hi = __ffsll((long long)(uint64_t)(v >> 64));
+  return lo ? lo - 1 : (hi ? 63 + hi : -1);
+}
+__device__ __forceinline__ int popc(u128 v) { return __popcll((uint64_t)v) + __popcll((uint64_t)(v >> 64)); }
+// warp shuffle of a mask (two 64-bit shuffles for the 128-bit layout)
+template <typename M>
+__device__ __forceinline__ M shfl_mask(M v, int src) {
+  if constexpr (sizeof(M) > 8) {
+    const uint64_t lo = __shfl_sync(0xffffffffu, (uint64_t)v, src), hi = __shfl_sync(0xffffffffu, (uint64_t)(v >> 64), src);
+    return ((M)hi << 64) | lo;
+  } else {
+    return __shfl_sync(0xffffffffu, v, src);
+  }
+}
+template <typename M>
+__device__ __forceinline__ M chunk_mask(const Chunks& ch, int k) {
+  if constexpr (sizeof(M) > 8) return ((M)ch.mask_hi[k] << 64) | ch.mask[k];
+  else return (M)ch.mask[k];
+}
 template <typename M>
 __device__ __forceinline__ M low_mask(int t) {  // bits 0..t inclusive
   return (M)(~(M)0) >> (sizeof(M) * 8 - 1 - t);
@@ -80,7 +108,7 @@ __device__ __forceinline__ M constrain(M raw, M pcr, const Chunks& ch) {
 #pragma unroll
     for (int k = 0; k < 3; ++k) {
       if (k < ch.n) {
-        const M cm = (M)ch.mask[k];
+        const M cm = chunk_mask<M>(ch, k);
         const M p = pcr & cm, r = raw & cm;
         m |= p ? p : (r & (~r + 1));
       }

@@ -9,6 +9,13 @@ using namespace abd;
 // ------------------------------------------------------------------------------------------
 // device-side view of the cohort
 // ------------------------------------------------------------------------------------------
+// The (individual, gap) words meta / cmeta: individual << kGapBits<M> | gap.  Six gap bits leave 26 for the individual;
+// the 128-bit layout needs seven (individuals < 2^25).
+template <typename M>
+constexpr int kGapBits = sizeof(M) > 8 ? 7 : 6;
+template <typename M>
+constexpr uint32_t kGapMask = (1u << kGapBits<M>) - 1u;
+
 struct DevCohort {
   int G, N;
   unsigned ind_offset;       // global index of this shard's first individual (RNG streams)
@@ -22,9 +29,9 @@ struct DevCohort {
   const uint32_t* rcx[2];      // per row: cell index << 5 | index of its dilution in xlev
   const double* xlev;          // [32] the distinct dilutions, ascending (padded with 0)
   int n_xlev;                  // 0: not available (k_sums stages the dilutions as doubles)
-  const uint32_t* meta[2];     // per row: individual << 6 | gap
+  const uint32_t* meta[2];     // per row: individual << kGapBits<M> | gap
   const uint32_t* rowcell[2];  // per row: index of its (individual, gap) cell
-  const uint32_t* cmeta[2];    // per cell: individual << 6 | gap
+  const uint32_t* cmeta[2];    // per cell: individual << kGapBits<M> | gap
   const int* rowperm[2];       // per (sorted) row: its index among the antigen's rows as the caller passed them
   Chunks ch;
 };
@@ -40,6 +47,13 @@ constexpr int kTileMaxInds = 128;
 #define ABD_GIBBS_MINB 4
 #endif
 constexpr int kGibbsWarps = ABD_GIBBS_WARPS;  // warps per CTA of the Gibbs kernels; ABD_GIBBS_MINB CTAs per SM
+// k_gibbs on 128-bit masks: four proposal slots per lane (two for 64-bit masks) do not fit the 64 registers that 4 CTAs
+// per SM leave (see DESIGN.md section 4)
+#ifndef ABD_GIBBS_MINB128
+#define ABD_GIBBS_MINB128 2
+#endif
+template <typename M>
+constexpr int kGibbsMinB = sizeof(M) > 8 ? ABD_GIBBS_MINB128 : ABD_GIBBS_MINB;
 
 // per-individual state staged in shared memory: constrained infections, vaccinations, waner
 // (packed in the top bit of the vaccination mask; usable gaps <= width - 1)
@@ -60,6 +74,42 @@ template <typename M>
 struct __align__(2 * sizeof(M)) PackedState {
   M rw, inf;
 };
+
+// One thread's i_raw column (gaps 0..G-1, stride N) as a bit mask.  Unpredicated loads along an address chain that
+// stops at the last row, masked afterwards: every load in flight at once, and the compiler cannot precompute (and
+// spill) one 64-bit address per gap.  (A load guarded by `t < G` needs a predicate register each, and there are only
+// seven: the compiler then keeps ~6 loads in flight.)  The 128-bit layout loads in blocks of 32 gaps, skipping the
+// blocks beyond the last gap: 128 bytes in flight per thread would not fit in registers.
+template <typename M>
+__device__ __forceinline__ M load_column(const int8_t* col, int G, int N) {
+  M raw = 0;
+  if constexpr (sizeof(M) > 8) {
+#pragma unroll 1
+    for (int b = 0; b * 32 < G; ++b) {
+      const int8_t* p = col + (size_t)b * 32 * N;
+      int8_t bytes[32];
+#pragma unroll
+      for (int t = 0; t < 32; ++t) {
+        bytes[t] = __ldg(p);
+        p += (b * 32 + t + 1 < G) ? (size_t)N : (size_t)0;
+      }
+      uint32_t bits = 0;
+#pragma unroll
+      for (int t = 0; t < 32; ++t) bits |= (uint32_t)(bytes[t] != 0) << t;
+      raw |= (M)bits << (32 * b);
+    }
+  } else {
+    int8_t bytes[sizeof(M) * 8];
+#pragma unroll
+    for (int t = 0; t < (int)sizeof(M) * 8; ++t) {
+      bytes[t] = __ldg(col);
+      col += (t + 1 < G) ? (size_t)N : (size_t)0;
+    }
+#pragma unroll
+    for (int t = 0; t < (int)sizeof(M) * 8; ++t) raw |= (M)(bytes[t] != 0) << t;
+  }
+  return raw & low_mask<M>(G - 1);
+}
 
 __device__ __forceinline__ double load_param(const double* theta, int theta_is_q, int c, int k13) {
   if (theta_is_q) {
@@ -84,13 +134,14 @@ __device__ __forceinline__ void fill_pow_warp(double rho, int G, int lane, doubl
     pw[0] = 1.0;
     if (dpw) dpw[0] = 0.0;
   }
+  double scale = 1.0;  // rho^(32 blk)
   for (int blk = 0; blk * 32 < G; ++blk) {
     const int k = blk * 32 + lane + 1;
-    const double scale = blk ? r32 : 1.0;  // G <= 63: at most two blocks
     if (k < G) {
       pw[k] = v * scale;
       if (dpw) dpw[k] = (double)k * prev * scale;
     }
+    scale *= r32;
   }
 }
 
@@ -108,10 +159,11 @@ __device__ __forceinline__ void fill_pow2_warp(double rho, int G, int lane, doub
     prev = 1.0;
     tab[0] = make_double2(1.0, 0.0);
   }
+  double scale = 1.0;  // rho^(32 blk)
   for (int blk = 0; blk * 32 < G; ++blk) {
     const int k = blk * 32 + lane + 1;
-    const double scale = blk ? r32 : 1.0;  // G <= 63: at most two blocks
     if (k < G) tab[k] = make_double2(v * scale, (double)k * prev * scale);
+    scale *= r32;
   }
 }
 

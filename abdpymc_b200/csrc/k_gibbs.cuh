@@ -24,7 +24,7 @@ struct RowPar {
 };
 template <typename M>
 __device__ __forceinline__ double gibbs_row(double x, double od, int t, bool is_s, M inf, M vac, int w,
-                                            const RowPar& rp, const double (*s_pw)[kMaxGaps],
+                                            const RowPar& rp, const double (*s_pw)[kGapTab<M>],
                                             const double* __restrict__ s_tab) {
   const M lm = low_mask<M>(t);
   M e = inf & lm, v = is_s ? (vac & lm) : (M)0;
@@ -45,7 +45,7 @@ __device__ __forceinline__ double gibbs_row(double x, double od, int t, bool is_
 // The vaccinations' share of an S row's decaying response, sum_{s in vac, s <= t} rho_ind^(t - s): it only changes with
 // ab_s_waner, so a lane keeps it for its row instead of re-summing it in every candidate evaluation.
 template <typename M>
-__device__ __forceinline__ double gibbs_vac_sum(int t, M vac, int w, const double (*s_pw)[kMaxGaps]) {
+__device__ __forceinline__ double gibbs_vac_sum(int t, M vac, int w, const double (*s_pw)[kGapTab<M>]) {
   M v = vac & low_mask<M>(t);
   const double* pw = w ? s_pw[1] : s_pw[2];
   double T = 0.0;
@@ -58,7 +58,7 @@ __device__ __forceinline__ double gibbs_vac_sum(int t, M vac, int w, const doubl
 // gibbs_row with the vaccinations' share handed in (tv; any_v: a vaccination at or before t)
 template <typename M>
 __device__ __forceinline__ double gibbs_row_tv(double x, double od, int t, bool is_s, M inf, double tv, bool any_v, int w,
-                                               const RowPar& rp, const double (*s_pw)[kMaxGaps],
+                                               const RowPar& rp, const double (*s_pw)[kGapTab<M>],
                                                const double* __restrict__ s_tab) {
   M e = inf & low_mask<M>(t);
   const double P = (e != 0 || any_v) ? rp.perm : 0.0;
@@ -76,7 +76,7 @@ __device__ __forceinline__ double gibbs_row_tv(double x, double od, int t, bool 
 //   [17], [18] sigmoid of those, [19], [20], [21] log p, log(1 - p), p; s_pw[0] = rho_n^k, s_pw[1] = rho_s^k.
 __device__ __forceinline__ void gibbs_load_chain(const double* __restrict__ theta, int theta_is_q,
                                                  const double* __restrict__ p_arr, const double* __restrict__ pw_arr,
-                                                 int c, int G, int lane, double* s_th, double (*s_pw)[kMaxGaps]) {
+                                                 int c, int G, int lane, double* s_th, double (*s_pw)[kGapTab<uint32_t>]) {
   __syncwarp();
   fill_pow_warp(load_param(theta, theta_is_q, c, N_RHO), G, lane, s_pw[0], nullptr);
   fill_pow_warp(load_param(theta, theta_is_q, c, S_RHO), G, lane, s_pw[1], nullptr);
@@ -113,7 +113,7 @@ template <typename M>
 struct GibbsRows {
   const DevCohort& dc;
   const double* s_th;
-  const double (*s_pw)[kMaxGaps];
+  const double (*s_pw)[kGapTab<M>];
   const double* s_tab;
   int lane, rn0, cnt_n, rs0, cnt_s, nrows;
   double x0, od0;
@@ -127,7 +127,7 @@ struct GibbsRows {
   int t_last, t_last_s;  // latest sampled gap of either antigen / of the S antigen (rows are sorted by gap)
 
   __device__ __forceinline__ GibbsRows(const DevCohort& dc_, int n, int lane_, const double* s_th_,
-                                       const double (*s_pw_)[kMaxGaps], const double* s_tab_)
+                                       const double (*s_pw_)[kGapTab<M>], const double* s_tab_)
       : dc(dc_), s_th(s_th_), s_pw(s_pw_), s_tab(s_tab_), lane(lane_) {
     rn0 = dc.rp[0][n], cnt_n = dc.rp[0][n + 1] - rn0;
     rs0 = dc.rp[1][n], cnt_s = dc.rp[1][n + 1] - rs0;
@@ -138,7 +138,7 @@ struct GibbsRows {
     for (int l = lane + 32; l < nrows; l += 32) {
       const bool is_s = l >= cnt_n;
       const int r = is_s ? rs0 + (l - cnt_n) : rn0 + l;
-      const int t = (int)((is_s ? dc.meta[1] : dc.meta[0])[r] & 63u);
+      const int t = (int)((is_s ? dc.meta[1] : dc.meta[0])[r] & kGapMask<M>);
       t_last = max(t_last, t);
       if (is_s) t_last_s = max(t_last_s, t);
     }
@@ -159,7 +159,7 @@ struct GibbsRows {
     if (l < nrows) {
       x = (is_s ? dc.x[1] : dc.x[0])[r];
       od = (is_s ? dc.od[1] : dc.od[0])[r];
-      t = (int)((is_s ? dc.meta[1] : dc.meta[0])[r] & 63u);
+      t = (int)((is_s ? dc.meta[1] : dc.meta[0])[r] & kGapMask<M>);
     } else {
       x = 0.0;
       od = 0.0;
@@ -195,6 +195,20 @@ struct GibbsRows {
   }
 };
 
+// a[i] of a per-lane array of proposal slots (i uniform over the warp), by selects: a dynamic index would put the
+// array in local memory
+template <int NS, typename T>
+__device__ __forceinline__ T slot(const T (&a)[NS], int i) {
+  if constexpr (NS <= 2) {
+    return (NS > 1 && i) ? a[NS - 1] : a[0];
+  } else {
+    T v = a[0];
+#pragma unroll
+    for (int s = 1; s < NS; ++s) v = (i == s) ? a[s] : v;
+    return v;
+  }
+}
+
 // (k_gibbs below keeps its own hand-inlined copy of these two: going through the helpers costs it
 // 4 % -- 274 instead of 264 us per sweep, a few more spilled registers under its 64-register cap.)
 // Persistent warps: every warp repeatedly claims the next (chain, individual) from a global
@@ -204,7 +218,7 @@ struct GibbsRows {
 // measured and dropped: patching each row's decaying response for a candidate instead of summing
 // it again (no gain: the extra live registers cost what the shorter loops save).
 template <typename M>
-__global__ void __launch_bounds__(kGibbsWarps * 32, ABD_GIBBS_MINB)
+__global__ void __launch_bounds__(kGibbsWarps * 32, kGibbsMinB<M>)
 k_gibbs(const DevCohort dc, const int* __restrict__ order, const int C,
         const double* __restrict__ theta, const int theta_is_q,
         const double* __restrict__ p_arr, const double* __restrict__ pw_arr,
@@ -216,13 +230,13 @@ k_gibbs(const DevCohort dc, const int* __restrict__ order, const int C,
 
   __shared__ double s_tab[kExpTab];
   __shared__ double s_th_all[kGibbsWarps][20];            // theta13, -1/(2 sigma^2) x 2, logit p / p_w, p / p_w
-  __shared__ double s_pw_all[kGibbsWarps][3][kMaxGaps];   // rho_n^k, rho_s^k, ones
-  __shared__ unsigned char s_ord[kGibbsWarps][kMaxGaps];
+  __shared__ double s_pw_all[kGibbsWarps][3][kGapTab<M>];   // rho_n^k, rho_s^k, ones
+  __shared__ unsigned char s_ord[kGibbsWarps][kGapTab<M>];
   double* s_th = s_th_all[warp];
-  const double (*s_pw)[kMaxGaps] = s_pw_all[warp];
+  const double (*s_pw)[kGapTab<M>] = s_pw_all[warp];
 
   fill_exp_table(s_tab, tid, kGibbsWarps * 32);
-  for (int k = lane; k < kMaxGaps; k += 32) s_pw_all[warp][2][k] = 1.0;
+  for (int k = lane; k < kGapTab<M>; k += 32) s_pw_all[warp][2][k] = 1.0;
   __syncthreads();
 
   const int nprop = G + 1;  // proposal j < G flips i_raw[j, n]; j == G flips waner[n]
@@ -310,7 +324,7 @@ k_gibbs(const DevCohort dc, const int* __restrict__ order, const int C,
       if (l < nrows) {
         x = (is_s ? dc.x[1] : dc.x[0])[r];
         od = (is_s ? dc.od[1] : dc.od[0])[r];
-        t = (int)((is_s ? dc.meta[1] : dc.meta[0])[r] & 63u);
+        t = (int)((is_s ? dc.meta[1] : dc.meta[0])[r] & kGapMask<M>);
       } else {
         x = 0.0;
         od = 0.0;
@@ -337,7 +351,7 @@ k_gibbs(const DevCohort dc, const int* __restrict__ order, const int C,
     for (int l = lane + 32; l < nrows; l += 32) {
       const bool is_s = l >= cnt_n;
       const int r = is_s ? rs0 + (l - cnt_n) : rn0 + l;
-      const int t = (int)((is_s ? dc.meta[1] : dc.meta[0])[r] & 63u);
+      const int t = (int)((is_s ? dc.meta[1] : dc.meta[0])[r] & kGapMask<M>);
       t_last = max(t_last, t);
       if (is_s) t_last_s = max(t_last_s, t);
     }
@@ -384,7 +398,7 @@ k_gibbs(const DevCohort dc, const int* __restrict__ order, const int C,
         rank[sl] = 0;
       }
       for (int jj = 0; jj < nprop; ++jj) {
-        const uint32_t kj = __shfl_sync(0xffffffffu, key[jj >> 5], jj & 31);
+        const uint32_t kj = __shfl_sync(0xffffffffu, NSLOT <= 2 ? key[(jj >> 5) & 1] : slot(key, jj >> 5), jj & 31);
 #pragma unroll
         for (int sl = 0; sl < NSLOT; ++sl) {
           const int me = lane + 32 * sl;
@@ -405,9 +419,10 @@ k_gibbs(const DevCohort dc, const int* __restrict__ order, const int C,
         const int jp = (step < nprop) ? (int)s_ord[warp][step] : 0;
         jp_step[sl] = jp;
         bool sk = __shfl_sync(0xffffffffu, (int)skip[0], jp & 31);
-        if (NSLOT > 1) {
-          const bool sk1 = __shfl_sync(0xffffffffu, (int)skip[NSLOT - 1], jp & 31);
-          if (jp >> 5) sk = sk1;
+#pragma unroll
+        for (int s2 = 1; s2 < NSLOT; ++s2) {  // (jp >> 5 differs between lanes: every slot is shuffled)
+          const bool sk1 = __shfl_sync(0xffffffffu, (int)skip[s2], jp & 31);
+          if (NSLOT <= 2 ? (jp >> 5) != 0 : (jp >> 5) == s2) sk = sk1;
         }
         act |= (M)__ballot_sync(0xffffffffu, step < nprop && !sk) << (32 * sl);
       }
@@ -458,18 +473,15 @@ k_gibbs(const DevCohort dc, const int* __restrict__ order, const int C,
     while (act) {
       const int step = ctz(act);
       act &= act - 1;
-      int jp = jp_step[0];
-      if (NSLOT > 1 && (step >> 5)) jp = jp_step[NSLOT - 1];
-      jp = __shfl_sync(0xffffffffu, jp, step & 31);
-      const int owner = jp & 31;
-      const bool hi = NSLOT > 1 && (jp >> 5);
-      const int code = __shfl_sync(0xffffffffu, hi ? code_own[NSLOT - 1] : code_own[0], owner);
+      const int jp = __shfl_sync(0xffffffffu, slot(jp_step, step >> 5), step & 31);
+      const int owner = jp & 31, jb = jp >> 5;
+      const int code = __shfl_sync(0xffffffffu, slot(code_own, jb), owner);
       const bool is_w = (jp == G);
       if (cfg.mode >= 0) {
         ++n_prop;
         if (code == 0) continue;
       }
-      const M inf2 = __shfl_sync(0xffffffffu, hi ? inf2_own[NSLOT - 1] : inf2_own[0], owner);
+      const M inf2 = shfl_mask(slot(inf2_own, jb), owner);
       const int w2 = is_w ? (w ^ 1) : w;
       double ll2 = ll;
       bool flip = true;
@@ -485,7 +497,7 @@ k_gibbs(const DevCohort dc, const int* __restrict__ order, const int C,
           }
           continue;
         }
-        const double au = __shfl_sync(0xffffffffu, hi ? acc_u[NSLOT - 1] : acc_u[0], owner);
+        const double au = __shfl_sync(0xffffffffu, slot(acc_u, jb), owner);
         if (cfg.mode == ABD_GIBBS_METROPOLIS) {
           const double delta = cur_bit ? -d10 : d10;  // logp(proposed) - logp(current)
           flip = isfinite(delta) && (au < delta);

@@ -37,12 +37,12 @@ k_gibbs_blk(const DevCohort dc, const int* __restrict__ order, const int C,
 
   __shared__ double s_tab[kExpTab];
   __shared__ double s_th_all[kGibbsWarps][24];            // see gibbs_load_chain
-  __shared__ double s_pw_all[kGibbsWarps][3][kMaxGaps];   // rho_n^k, rho_s^k, ones
+  __shared__ double s_pw_all[kGibbsWarps][3][kGapTab<M>];   // rho_n^k, rho_s^k, ones
   double* s_th = s_th_all[warp];
-  const double (*s_pw)[kMaxGaps] = s_pw_all[warp];
+  const double (*s_pw)[kGapTab<M>] = s_pw_all[warp];
 
   fill_exp_table(s_tab, tid, kGibbsWarps * 32);
-  for (int k = lane; k < kMaxGaps; k += 32) s_pw_all[warp][2][k] = 1.0;
+  for (int k = lane; k < kGapTab<M>; k += 32) s_pw_all[warp][2][k] = 1.0;
   __syncthreads();
 
   unsigned n_prop = 0, n_acc = 0;

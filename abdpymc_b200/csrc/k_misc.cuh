@@ -98,18 +98,7 @@ k_determ(const DevCohort dc, const double* __restrict__ theta13, const int8_t* _
   if (threadIdx.x < 13) s_th[threadIdx.x] = theta13[(size_t)c * 13 + threadIdx.x];
   __syncthreads();
   if (n >= N) return;
-  // unpredicated loads along an address chain, masked afterwards: all in flight (see k_sums)
-  M raw = 0;
-  const int8_t* col = i_raw + (size_t)c * G * N + n;
-  int8_t bytes[sizeof(M) * 8];
-#pragma unroll
-  for (int t = 0; t < (int)sizeof(M) * 8; ++t) {
-    bytes[t] = __ldg(col);
-    col += (t + 1 < G) ? (size_t)N : (size_t)0;
-  }
-#pragma unroll
-  for (int t = 0; t < (int)sizeof(M) * 8; ++t) raw |= (M)(bytes[t] != 0) << t;
-  raw &= low_mask<M>(G - 1);
+  const M raw = load_column<M>(i_raw + (size_t)c * G * N + n, G, N);
   const int w = waner[(size_t)c * N + n] != 0;
   const M inf = constrain<M>(raw, reinterpret_cast<const M*>(dc.pcr)[n], dc.ch);
   const M vac = reinterpret_cast<const M*>(dc.vac)[n];
@@ -216,7 +205,7 @@ k_loglik_rows(const DevCohort dc, const int a, const int R, const double* __rest
   __syncthreads();
   if (r >= R) return;
   const uint32_t mt = dc.meta[a][r];
-  const int n = (int)(mt >> 6), t = (int)(mt & 63u);
+  const int n = (int)(mt >> kGapBits<M>), t = (int)(mt & kGapMask<M>);
   M raw = 0;
   const int8_t* col = i_raw + (size_t)c * G * N + n;
   for (int g = 0; g < G; ++g) raw |= (M)(col[(size_t)g * N] != 0) << g;   // (the whole column: the constraints are per chunk)
@@ -242,17 +231,7 @@ k_pack(const DevCohort dc, const int8_t* __restrict__ i_raw, const int8_t* __res
   const int c = blockIdx.y, n = blockIdx.x * blockDim.x + threadIdx.x;
   const int G = dc.G, N = dc.N;
   if (n >= N) return;
-  M raw = 0;
-  const int8_t* col = i_raw + (size_t)c * G * N + n;
-  int8_t bytes[sizeof(M) * 8];
-#pragma unroll
-  for (int t = 0; t < (int)sizeof(M) * 8; ++t) {  // unpredicated loads along an address chain (see k_sums)
-    bytes[t] = __ldg(col);
-    col += (t + 1 < G) ? (size_t)N : (size_t)0;
-  }
-#pragma unroll
-  for (int t = 0; t < (int)sizeof(M) * 8; ++t) raw |= (M)(bytes[t] != 0) << t;
-  raw &= low_mask<M>(G - 1);
+  const M raw = load_column<M>(i_raw + (size_t)c * G * N + n, G, N);
   PackedState<M> ps;
   ps.inf = constrain<M>(raw, reinterpret_cast<const M*>(dc.pcr)[n], dc.ch);
   ps.rw = raw | (waner[(size_t)c * N + n] != 0 ? top_bit<M>() : (M)0);

@@ -195,7 +195,7 @@ k_sums(const DevCohort dc, const TileDesc* __restrict__ tiles, const SumsCfg cfg
   uint32_t* s_cm_s = s_cm_n + cfg.capk_n;
 
   __shared__ double s_th[16];
-  __shared__ double2 s_pw[2][kMaxGaps];  // {rho^k, k rho^(k-1)} for rho_n, rho_s
+  __shared__ double2 s_pw[2][kGapTab<M>];  // {rho^k, k rho^(k-1)} for rho_n, rho_s
   __shared__ double s_tab[kExpTab];
   __shared__ IndState<M> s_ind[kTileMaxInds];
   __shared__ double s_red[kSumsWarps][kNSums];
@@ -378,22 +378,8 @@ k_sums(const DevCohort dc, const TileDesc* __restrict__ tiles, const SumsCfg cfg
       cnt_i = (double)popc(ps.rw & ~top_bit<M>());
       cnt_w = w ? 1.0 : 0.0;
     } else if (tid < ni) {
-      // Unpredicated loads: gaps beyond G - 1 re-read the last row and are masked off afterwards.
-      // (A load guarded by `t < G` needs a predicate register each, and there are only seven: the
-      // compiler then keeps ~6 loads in flight and the column costs 5 memory round trips.)
-      const int8_t* col = i_raw + (size_t)c * G * N + i0 + tid;
-      // (The address walks down the column and stops at the last row: a chain of adds, so that the
-      // compiler cannot precompute -- and spill -- 32 / 64 independent 64-bit addresses.)
-      int8_t bytes[sizeof(M) * 8];
-#pragma unroll
-      for (int t = 0; t < (int)sizeof(M) * 8; ++t) {
-        bytes[t] = __ldg(col);
-        col += (t + 1 < G) ? (size_t)N : (size_t)0;
-      }
-      M raw = 0;
-#pragma unroll
-      for (int t = 0; t < (int)sizeof(M) * 8; ++t) raw |= (M)(bytes[t] != 0) << t;
-      raw &= low_mask<M>(G - 1);
+      // (unpredicated loads, all in flight: see load_column; without them the column costs 5 memory round trips)
+      const M raw = load_column<M>(i_raw + (size_t)c * G * N + i0 + tid, G, N);
       const int w = waner[(size_t)c * N + i0 + tid] != 0;
       IndState<M> st;
       st.inf = constrain<M>(raw, my_pcr, dc.ch);
@@ -529,7 +515,7 @@ k_sums(const DevCohort dc, const TileDesc* __restrict__ tiles, const SumsCfg cfg
 #pragma unroll kCellUnroll
       for (int k = cn0 + tid; k < cn1 && tid < nwork; k += nwork) {
         const uint32_t mt = s_cm_n[k - kn0];
-        const int t = mt & 63, li = (int)(mt >> 6) - i0;
+        const int t = mt & kGapMask<M>, li = (int)(mt >> kGapBits<M>) - i0;
         double P, T, dT;
         traj_n<M>(s_ind[li].inf, t, s_pw[0], P, T, dT);
         CellVal cv;
@@ -552,7 +538,7 @@ k_sums(const DevCohort dc, const TileDesc* __restrict__ tiles, const SumsCfg cfg
 #pragma unroll kCellUnroll
       for (int k = cs0 + tid; k < cs1 && tid < nwork; k += nwork) {
         const uint32_t mt = s_cm_s[k - ks0];
-        const int t = mt & 63, li = (int)(mt >> 6) - i0;
+        const int t = mt & kGapMask<M>, li = (int)(mt >> kGapBits<M>) - i0;
         const IndState<M> st = s_ind[li];
         double P, U, dU;
         traj_s<M>(st.inf, st.vacw & ~top_bit<M>(), (st.vacw & top_bit<M>()) != 0, t, s_pw[1], P, U, dU);

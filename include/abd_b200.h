@@ -51,7 +51,7 @@ extern "C" {
 #define ABD_N_THETA 13
 #define ABD_N_Q 17
 #define ABD_N_SUMS 16
-#define ABD_MAX_GAPS 63
+#define ABD_MAX_GAPS 127 /* gap masks of 32, 64 or 128 bits; the top bit holds the waner bit */
 
 /* abd_gibbs_sweep modes */
 #define ABD_GIBBS_METROPOLIS 0 /* PyMC BinaryGibbsMetropolis semantics: propose the flip w.p.
@@ -103,7 +103,12 @@ int abd_version(void);
 
 /* Builds the device-resident cohort on CUDA device `device`.  Replaces the data side of
  * abd.model(): as_tensor(data.vacs.T), pcrpos (abd.py:413-418), make_time_chunks
- * (abd.py:865-882), the gather indices (abd.py:343,393) and check_splits (abd.py:604-622).  */
+ * (abd.py:865-882), the gather indices (abd.py:343,393) and check_splits (abd.py:604-622).
+ * Limits: 1 <= n_gaps <= ABD_MAX_GAPS, n_inds < 2^26 (< 2^25 when n_gaps > 63).  Layout on the device: per
+ * individual, the PCR+ and vaccination months as one bit mask over gaps of 32 bits (n_gaps <= 31), 64 bits
+ * (<= 63) or 128 bits (<= 127); the packed resident state (abd_state_dev) holds two such masks per chain and
+ * individual (8, 16 or 32 bytes).  The environment variable ABD_B200_MASK_BITS=128 selects the 128-bit layout
+ * for any n_gaps (tests and measurements: same results, other kernels).                                    */
 int abd_create(abd_handle** out, const abd_cohort* cohort, int device);
 int abd_destroy(abd_handle* h);
 
