@@ -67,6 +67,51 @@ int fail(int code, const std::string& msg) {
 // ------------------------------------------------------------------------------------------
 // host side
 // ------------------------------------------------------------------------------------------
+namespace {
+
+// Device allocations released together: a handle's cohort arrays, its per-chain buffers, or one call's temporaries
+// (cudaFree waits for the device, so temporaries may go out of scope while work that uses them is still queued)
+struct DevBufs {
+  std::vector<void*> ptrs;
+  template <typename T>
+  int alloc(T** p, size_t n) {
+    void* q = nullptr;
+    cudaError_t e = cudaMalloc(&q, std::max<size_t>(n, 1) * sizeof(T));
+    if (e != cudaSuccess) return fail(ABD_ERR_ALLOC, std::string("cudaMalloc: ") + cudaGetErrorString(e));
+    ptrs.push_back(q);
+    *p = (T*)q;
+    return ABD_OK;
+  }
+  void release() {
+    for (void* p : ptrs) cudaFree(p);
+    ptrs.clear();
+  }
+  ~DevBufs() { release(); }
+};
+
+// Preprocessed-cohort cache file (SURVEY 8f-4: TiterData -> device upload format).  Its header is also the
+// description of the cohort every handle is built from (new_handle), whether abd_create derived it or a file carried it.
+struct CacheHeader {
+  char magic[8];           // "ABDB200\0"
+  int32_t version, G, N, n_chunks;
+  uint64_t chunk_mask[3];
+  int32_t wide, fx, n_xlev, has_pcr;   // wide: mask layout, 0 = 32, 1 = 64, 2 = 128 bits
+  int64_t R[2], K[2];      // OD rows / (individual, gap) cells per antigen (N, S)
+  double tot[4];
+  uint32_t ind_offset, pad;
+  double xlev[kMaxXLevels];
+};
+// Version 2: 32- and 64-bit masks.  Version 3 (128-bit masks): the same header, then the chunk masks' high words
+// (gaps 64..127) before the arrays.
+constexpr int kCacheVersion = 2, kCacheVersionWide = 3;
+
+struct CohortDesc {
+  CacheHeader hd;
+  uint64_t mask_hi[3];  // the chunk masks' high words
+};
+
+}  // namespace
+
 struct abd_handle {
   int device = 0;
   int G = 0, N = 0;
@@ -74,7 +119,8 @@ struct abd_handle {
   int64_t R[2] = {0, 0};
   Totals tot{};
   DevCohort dc{};
-  std::vector<void*> owned;   // device allocations freed in abd_destroy
+  CohortDesc desc{};          // what the handle was built from (abd_save_cache writes it)
+  DevBufs owned;              // cohort arrays and other allocations that live as long as the handle
   std::vector<int> h_rp[2];   // host copy of the row CSR pointers (for tilings)
   std::vector<int> h_cp[2];   // host copy of the cell CSR pointers
   cudaStream_t stream = nullptr;
@@ -98,31 +144,23 @@ struct abd_handle {
   int n_sms = 148;
   size_t smem_optin = 0;
   int* d_order = nullptr;       // individuals by decreasing OD-row count (Gibbs work queue)
-  unsigned* d_queue = nullptr;  // Gibbs work queues: one counter per chain (per-handle scratch, allocated with the chains)
   int gibbs_ctas = 0;
   int gibbs_blk_ctas = 0;
   ThetaInline thin{};           // parameters passed by value with the next k_sums launch (n = 0: none)
   // peer exchange (individual sharding over NVLink)
   XchCfg xch{};
   void* xch_local = nullptr;
-  bool xch_active = false;  // set for the duration of a fused sharded launch
   void* xch_peer[kMaxPeers] = {};
-  std::vector<double> x_levels; // distinct log_dilution values (ascending) when there are <= 32 of them
   bool fx = false;              // factored mode: rows carry (cell, dilution index), see k_sums
-  bool use_pdl = true;          // programmatic dependent launch (ABD_B200_NO_PDL=1 disables)
-  bool use_pull = true;         // SM-driven upload of pinned chain state (ABD_B200_NO_PULL=1 disables)
-  bool use_poll = true;         // host-pointer logp call: watch the pinned result slots instead of cudaStreamSynchronize (ABD_B200_NO_POLL=1 disables)
-  bool use_inline = true;       // <= 8 chains: parameters by value in the launch (ABD_B200_NO_INLINE=1 disables)
 
-  // per-chain scratch
+  // per-chain buffers for cap_chains chains: allocated by ensure_chains, released by free_chains
   int cap_chains = 0;
+  DevBufs chain_bufs;
   int8_t* d_iraw = nullptr;
   int8_t* d_waner = nullptr;
   void* d_pack = nullptr;      // PackedState<M>[C][N] beside the int8 state (see abd_kernels_common.cuh)
   int pack_valid = 0;          // leading chains whose packed entries mirror d_iraw / d_waner
   bool lazy_pack = true;       // a launch on the resident state may (re)build the packed copy first
-  bool use_pack = true;        // ABD_B200_NO_PACK=1: always read the int8 arrays
-  bool has_pcr = true;         // built with PCR+ data (false: ignore_pcrpos)
   double* d_theta = nullptr;   // [C][17]
   double* d_p = nullptr;       // [C][2]
   double* d_sums = nullptr;    // [C][16]
@@ -132,10 +170,13 @@ struct abd_handle {
   double* d_traj = nullptr;    // [C][34] trajectory-mode scratch (position, half-step momentum)
   unsigned* d_gen = nullptr;   // [C + 1] generation counters + error flag
   unsigned long long* d_stats = nullptr;
-  double* d_partial = nullptr;
-  size_t cap_partial = 0;
+  unsigned* d_queue = nullptr; // Gibbs work queues: one counter per chain
   double* h_pin = nullptr;     // pinned staging [C][40]
   double* h_pin_dev = nullptr; // the same buffer as the device sees it
+  // k_sums' partial sums, sized by the grid plan
+  DevBufs partial_buf;
+  double* d_partial = nullptr;
+  size_t cap_partial = 0;
 };
 
 namespace {
@@ -148,22 +189,13 @@ auto with_mask(const abd_handle* h, F&& f) {
   if (h->mask_bits == 64) return f(uint64_t{});
   return f(uint32_t{});
 }
-// mask layout for a cohort of G gaps: the narrowest that holds G gaps and the waner bit
-int mask_bits_for(int G) { return G <= 31 ? 32 : (G <= 63 ? 64 : 128); }
-
-template <typename T>
-int dev_alloc(abd_handle* h, T** p, size_t n, bool owned = true) {
-  void* q = nullptr;
-  cudaError_t e = cudaMalloc(&q, std::max<size_t>(n, 1) * sizeof(T));
-  if (e != cudaSuccess) return fail(ABD_ERR_ALLOC, std::string("cudaMalloc: ") + cudaGetErrorString(e));
-  *p = (T*)q;
-  if (owned) h->owned.push_back(q);
-  return ABD_OK;
-}
+// mask layout for a cohort of G gaps, as the cache header's `wide` field: the narrowest that holds G gaps and the waner
+// bit (new_handle turns it into mask_bits)
+int wide_for(int G) { return G <= 31 ? 0 : (G <= 63 ? 1 : 2); }
 
 template <typename T>
 int upload(abd_handle* h, T** dptr, const std::vector<T>& v) {
-  int rc = dev_alloc(h, dptr, v.size());
+  int rc = h->owned.alloc(dptr, v.size());
   if (rc) return rc;
   if (!v.empty()) CU(cudaMemcpy(*dptr, v.data(), v.size() * sizeof(T), cudaMemcpyHostToDevice));
   return ABD_OK;
@@ -266,7 +298,8 @@ int build_rows(abd_handle* h, int a, int64_t R, const double* x, const double* o
   if (h->fx) {
     std::vector<uint32_t> rcx((size_t)R + 4, 0u);
     for (int64_t k = 0; k < R; ++k) {
-      const int xi = (int)(std::lower_bound(h->x_levels.begin(), h->x_levels.end(), xs[(size_t)k]) - h->x_levels.begin());
+      const double* lv = h->desc.hd.xlev;
+      const int xi = (int)(std::lower_bound(lv, lv + h->desc.hd.n_xlev, xs[(size_t)k]) - lv);
       rcx[(size_t)k] = (rowcell[(size_t)k] << 5) | (uint32_t)xi;
     }
     uint32_t* d_rcx;
@@ -279,7 +312,6 @@ int build_rows(abd_handle* h, int a, int64_t R, const double* x, const double* o
   h->dc.meta[a] = d_meta;
   h->dc.rowcell[a] = d_rowcell;
   h->dc.cmeta[a] = d_cmeta;
-  h->R[a] = R;
   return ABD_OK;
 }
 
@@ -346,53 +378,49 @@ int get_tiling(abd_handle* h, int want, abd_handle::Tiling** out) {
   return ABD_OK;
 }
 
+void free_chains(abd_handle* h) {
+  h->chain_bufs.release();
+  if (h->h_pin) cudaFreeHost(h->h_pin);
+  h->h_pin = h->h_pin_dev = nullptr;
+  h->cap_chains = h->pack_valid = 0;
+}
+
 int ensure_chains(abd_handle* h, int C) {
   if (C <= 0) return fail(ABD_ERR_INVALID, "n_chains must be positive");
   if (C > 65535) return fail(ABD_ERR_INVALID, "n_chains must be <= 65535");
   if (C <= h->cap_chains) return ABD_OK;
   CU(cudaStreamSynchronize(h->stream));
-  int8_t *old_i = h->d_iraw, *old_w = h->d_waner;
   const int oldC = h->cap_chains;
   const size_t gn = (size_t)h->G * h->N;
   int rc;
+  // the chain state moves to the larger buffers; everything else starts afresh
+  DevBufs next;
   int8_t *ni, *nw;
-  if ((rc = dev_alloc(h, &ni, (size_t)C * gn, false))) return rc;
-  if ((rc = dev_alloc(h, &nw, (size_t)C * h->N, false))) return rc;
+  if ((rc = next.alloc(&ni, (size_t)C * gn)) || (rc = next.alloc(&nw, (size_t)C * h->N))) return rc;
   CU(cudaMemset(ni, 0, (size_t)C * gn));
   CU(cudaMemset(nw, 0, (size_t)C * h->N));
   if (oldC) {
-    CU(cudaMemcpy(ni, old_i, (size_t)oldC * gn, cudaMemcpyDeviceToDevice));
-    CU(cudaMemcpy(nw, old_w, (size_t)oldC * h->N, cudaMemcpyDeviceToDevice));
+    CU(cudaMemcpy(ni, h->d_iraw, (size_t)oldC * gn, cudaMemcpyDeviceToDevice));
+    CU(cudaMemcpy(nw, h->d_waner, (size_t)oldC * h->N, cudaMemcpyDeviceToDevice));
   }
-  for (void* p : {(void*)old_i, (void*)old_w, h->d_pack, (void*)h->d_theta, (void*)h->d_p, (void*)h->d_sums,
-                  (void*)h->d_out, (void*)h->d_ticket, (void*)h->d_stats, (void*)h->d_aux, (void*)h->d_traj, (void*)h->d_gen,
-                  (void*)h->d_queue})
-    if (p) cudaFree(p);
-  if (h->h_pin) cudaFreeHost(h->h_pin);
+  free_chains(h);
+  std::swap(h->chain_bufs.ptrs, next.ptrs);
   h->d_iraw = ni;
   h->d_waner = nw;
-  h->d_pack = nullptr;
-  h->pack_valid = 0;
-  {
-    char* pk = nullptr;
-    const size_t entry = with_mask(h, [](auto m) { return sizeof(PackedState<decltype(m)>); });
-    if ((rc = dev_alloc(h, &pk, (size_t)C * h->N * entry, false))) return rc;
-    h->d_pack = pk;
-  }
-  if ((rc = dev_alloc(h, &h->d_theta, (size_t)C * 17, false))) return rc;
-  if ((rc = dev_alloc(h, &h->d_p, (size_t)C * 2, false))) return rc;
-  if ((rc = dev_alloc(h, &h->d_sums, (size_t)C * kNSums, false))) return rc;
-  if ((rc = dev_alloc(h, &h->d_out, (size_t)C * 18, false))) return rc;
-  if ((rc = dev_alloc(h, &h->d_ticket, (size_t)C, false))) return rc;
-  if ((rc = dev_alloc(h, &h->d_aux, (size_t)C * kAuxDoubles, false))) return rc;
-  if ((rc = dev_alloc(h, &h->d_traj, (size_t)C * 34, false))) return rc;
-  if ((rc = dev_alloc(h, &h->d_gen, (size_t)C + 1, false))) return rc;
-  if ((rc = dev_alloc(h, &h->d_stats, (size_t)C * 2, false))) return rc;
-  if ((rc = dev_alloc(h, &h->d_queue, (size_t)C, false))) return rc;
+  DevBufs& b = h->chain_bufs;
+  char* pk = nullptr;
+  const size_t entry = with_mask(h, [](auto m) { return sizeof(PackedState<decltype(m)>); });
+  if ((rc = b.alloc(&pk, (size_t)C * h->N * entry))) return rc;
+  h->d_pack = pk;
+  if ((rc = b.alloc(&h->d_theta, (size_t)C * 17)) || (rc = b.alloc(&h->d_p, (size_t)C * 2)) ||
+      (rc = b.alloc(&h->d_sums, (size_t)C * kNSums)) || (rc = b.alloc(&h->d_out, (size_t)C * 18)) ||
+      (rc = b.alloc(&h->d_ticket, (size_t)C)) || (rc = b.alloc(&h->d_aux, (size_t)C * kAuxDoubles)) ||
+      (rc = b.alloc(&h->d_traj, (size_t)C * 34)) || (rc = b.alloc(&h->d_gen, (size_t)C + 1)) ||
+      (rc = b.alloc(&h->d_stats, (size_t)C * 2)) || (rc = b.alloc(&h->d_queue, (size_t)C)))
+    return rc;
   CU(cudaMemset(h->d_ticket, 0, (size_t)C * sizeof(unsigned)));
   CU(cudaMemset(h->d_gen, 0, ((size_t)C + 1) * sizeof(unsigned)));
   CU(cudaMallocHost((void**)&h->h_pin, (size_t)C * 40 * sizeof(double)));
-  h->h_pin_dev = nullptr;
   {
     void* dp = nullptr;
     if (cudaHostGetDevicePointer(&dp, h->h_pin, 0) == cudaSuccess) h->h_pin_dev = (double*)dp;
@@ -409,8 +437,10 @@ int ensure_chains(abd_handle* h, int C) {
 // `one_wave_rows`: tiles may grow to this many OD rows if that lets the whole grid run as ONE wave (12 500 individuals x
 // 4 chains -- an eighth of the 100k cohort -- is 1.25 waves of 2 200-row tiles: two waves, 18.4 us, against one wave of
 // 2 650-row tiles); 0 = the ordinary limit.  The caller falls back to 0 when such tiles do not fit in shared memory.
+// `cpc_fixed`: chains per CTA (0 = the planner's choice).
 constexpr int kTileRowsOneWave = 2750;
-void plan_grid(const abd_handle* h, int C, int ctas_per_sm, int* want_tiles, int* chains_per_cta, int one_wave_rows = 0) {
+void plan_grid(const abd_handle* h, int C, int ctas_per_sm, int cpc_fixed, int one_wave_rows, int* want_tiles,
+               int* chains_per_cta) {
   const double rows = (double)(h->R[0] + h->R[1]);
   const int target = h->tile_rows_override > 0 ? h->tile_rows_override : 2200;
   const int min_tiles = (h->N + kTileMaxInds - 1) / kTileMaxInds;
@@ -437,12 +467,12 @@ void plan_grid(const abd_handle* h, int C, int ctas_per_sm, int* want_tiles, int
   // chains looped over inside one CTA (the staged tile is reused): measured at 10k / 12.5k individuals, 32 chains run
   // 4 - 11 % faster with 2 per CTA than with 4 (twice the waves: shorter start-up and drain), 128 chains 5 % faster
   // with 4 than with 2, and 8 / 16 per CTA are 10 / 25 % slower than 4 (tools/tune.py sums)
-  int cpc = h->chains_per_cta_override > 0 ? h->chains_per_cta_override : (C >= 64 ? 4 : (C >= 32 ? 2 : 1));
+  int cpc = cpc_fixed > 0 ? cpc_fixed : (C >= 64 ? 4 : (C >= 32 ? 2 : 1));
   cpc = std::min(cpc, C);
   cpc = std::min(cpc, kMaxChainsPerCta);  // a CTA remembers at most this many chains it finished last (k_sums: s_pend)
   int tiles;
   const double waves1 = tiles_for(cpc, &tiles);
-  if (h->chains_per_cta_override == 0 && cpc == 1 && waves1 >= 3.0) {
+  if (cpc_fixed == 0 && cpc == 1 && waves1 >= 3.0) {
     // Few chains on a cohort of several waves: a wave of one-chain CTAs costs ~9.3 us whatever its tile size, a CTA
     // that loops over k chains ~1 + 8.3 k us per wave (measured, 4 chains: 25 000 individuals 28.3 us as 3 waves
     // against 21.2 as ONE wave of two-chain CTAs; 50 000 individuals 47.1 as 5 waves against 35.8 as one wave of
@@ -459,35 +489,63 @@ void plan_grid(const abd_handle* h, int C, int ctas_per_sm, int* want_tiles, int
   *chains_per_cta = cpc;
 }
 
+// One k_sums instantiation, as a type (its shared-memory setting is remembered per instantiation)
+template <typename M, typename XT, bool TRAJ, bool CP>
+struct SumsKernel {
+  using Mask = M;
+  static auto fn() { return k_sums<M, XT, TRAJ, CP>; }
+};
+
+// The one place that picks the k_sums instantiation for a launch: returns f(SumsKernel<...>{}) for the handle's mask
+// layout and dilution mode (fx), the compact cell layout or not, and trajectory mode or not.
+template <typename F>
+auto with_sums(const abd_handle* h, bool compact, bool traj, F&& f) {
+  return with_mask(h, [&](auto m) {
+    using M = decltype(m);
+    if (compact) return traj ? f(SumsKernel<M, uint8_t, true, true>{}) : f(SumsKernel<M, uint8_t, false, true>{});
+    if (h->fx) return traj ? f(SumsKernel<M, uint8_t, true, false>{}) : f(SumsKernel<M, uint8_t, false, false>{});
+    return traj ? f(SumsKernel<M, double, true, false>{}) : f(SumsKernel<M, double, false, false>{});
+  });
+}
+
 // The dynamic shared-memory limit of a kernel is a per-device function attribute shared by every
 // handle of the process: only ever raise it (a small cohort must not lower it under a large one).
-template <typename M, typename XT, bool TRAJ, bool CP>
-cudaError_t sums_smem_attr(int device, size_t smem) {
+template <typename K>
+cudaError_t sums_smem_attr(K, int device, size_t smem) {
   static size_t configured[64] = {};
   const int d = (device >= 0 && device < 64) ? device : 0;
   const size_t want = std::max<size_t>(smem, 48 * 1024);
   if (want <= configured[d]) return cudaSuccess;
-  cudaError_t e = cudaFuncSetAttribute(k_sums<M, XT, TRAJ, CP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)want);
+  cudaError_t e = cudaFuncSetAttribute(K::fn(), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)want);
   if (e != cudaSuccess) return e;
-  e = cudaFuncSetAttribute(k_sums<M, XT, TRAJ, CP>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
+  e = cudaFuncSetAttribute(K::fn(), cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
   if (e != cudaSuccess) return e;
   configured[d] = want;
   return cudaSuccess;
 }
 
-template <typename M, typename XT, bool CP>
-cudaError_t sums_occupancy(int device, size_t smem, int* occ) {
-  cudaError_t e = sums_smem_attr<M, XT, false, CP>(device, smem);
-  if (e != cudaSuccess) return e;
-  return cudaOccupancyMaxActiveBlocksPerMultiprocessor(occ, k_sums<M, XT, false, CP>, kSumsBlock, smem);
-}
 // resident CTAs per SM of the plain-evaluation kernel for this handle's mask width / dilution mode
-cudaError_t sums_occupancy_h(const abd_handle* h, bool compact, size_t smem, int* occ) {
-  return with_mask(h, [&](auto m) {
-    using M = decltype(m);
-    if (compact) return sums_occupancy<M, uint8_t, true>(h->device, smem, occ);
-    return h->fx ? sums_occupancy<M, uint8_t, false>(h->device, smem, occ) : sums_occupancy<M, double, false>(h->device, smem, occ);
+cudaError_t sums_occupancy(const abd_handle* h, bool compact, size_t smem, int* occ) {
+  return with_sums(h, compact, false, [&](auto k) {
+    cudaError_t e = sums_smem_attr(k, h->device, smem);
+    if (e != cudaSuccess) return e;
+    return cudaOccupancyMaxActiveBlocksPerMultiprocessor(occ, decltype(k)::fn(), kSumsBlock, smem);
   });
+}
+
+// A launch configuration that lets the kernel start while the previous one on the stream drains (programmatic
+// dependent launch); `attr` is the caller's storage for the one launch attribute
+cudaLaunchConfig_t pdl_config(dim3 grid, dim3 block, size_t smem, cudaStream_t st, cudaLaunchAttribute* attr) {
+  cudaLaunchConfig_t lc{};
+  lc.gridDim = grid;
+  lc.blockDim = block;
+  lc.dynamicSmemBytes = smem;
+  lc.stream = st;
+  attr->id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  attr->val.programmaticStreamSerializationAllowed = 1;
+  lc.attrs = attr;
+  lc.numAttrs = 1;
+  return lc;
 }
 
 // The packed copy of the resident chain state for a launch that reads (i_raw, waner): non-null only
@@ -495,7 +553,7 @@ cudaError_t sums_occupancy_h(const abd_handle* h, bool compact, size_t smem, int
 // launch on the same stream) unless the caller has just staged fresh host state for a single use.
 int resident_pack(abd_handle* h, int C, const int8_t* i_raw, const int8_t* waner, cudaStream_t st, void** out) {
   *out = nullptr;
-  if (!h->use_pack || i_raw != h->d_iraw || waner != h->d_waner || !h->d_pack) return ABD_OK;
+  if (i_raw != h->d_iraw || waner != h->d_waner || !h->d_pack) return ABD_OK;
   if (h->pack_valid < C) {
     if (!h->lazy_pack) return ABD_OK;
     dim3 grid((h->N + 127) / 128, C);
@@ -511,65 +569,17 @@ int resident_pack(abd_handle* h, int C, const int8_t* i_raw, const int8_t* waner
   return ABD_OK;
 }
 
-template <typename M, typename XT, bool CP>
-int launch_sums_t(abd_handle* h, const abd_handle::Tiling& tl, const SumsCfg& cfg, dim3 grid, const double* theta,
-                  int theta_is_q, const int8_t* i_raw, const int8_t* waner, const void* pack_v, double* sums,
-                  const FinalizeCfg& fin, const TrajCfg& traj, cudaStream_t st, const ThetaInline& thin) {
-  const PackedState<M>* pack = reinterpret_cast<const PackedState<M>*>(pack_v);
-  const size_t smem = CP ? tl.smem_cp : tl.smem;
-  if (std::getenv("ABD_B200_VERBOSE")) {
-    const int occ = CP ? tl.occ_cp : tl.occ;
-    std::fprintf(stderr, "[abd_b200] k_sums grid (%u, %u) dyn smem %zu B%s, occupancy %d CTAs/SM, caps rows %d/%d cells %d/%d\n",
-                 grid.x, grid.y, smem, CP ? " (compact cells)" : "", occ, tl.cap_n, tl.cap_s, tl.capk_n, tl.capk_s);
-  }
-  const int tj = traj.n_steps > 0 ? 1 : 0;
-  if (tj) CU((sums_smem_attr<M, XT, true, CP>(h->device, smem)));
-  else CU((sums_smem_attr<M, XT, false, CP>(h->device, smem)));
-  cudaLaunchConfig_t lc{};
-  lc.gridDim = grid;
-  lc.blockDim = dim3(kSumsBlock);
-  lc.dynamicSmemBytes = smem;
-  lc.stream = st;
-  cudaLaunchAttribute attr[1];
-  const TileDesc* tiles = reinterpret_cast<const TileDesc*>(tl.d_tiles);
-  const Priors* pri = h->d_priors;
-  if (tj) {
-    if (traj.n_steps > 1 && h->xch_active)
-      return fail(ABD_ERR_INVALID, "sharded leapfrog: one step per launch");
-    if (traj.n_steps > 1) {  // CTAs wait on one another: they must all be resident
-      int occ = 0;
-      CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_sums<M, XT, true, CP>, kSumsBlock, smem));
-      if ((long)grid.x * grid.y > (long)occ * h->n_sms)
-        return fail(ABD_ERR_INVALID, "abd_leapfrog_dev: the grid does not fit on the device at once");
-      attr[0].id = cudaLaunchAttributeCooperative;
-      attr[0].val.cooperative = 1;
-      lc.numAttrs = 1;
-    } else {  // a single step waits on nothing inside the grid: ordinary launch, overlapped like k_sums
-      attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-      attr[0].val.programmaticStreamSerializationAllowed = 1;
-      lc.numAttrs = h->use_pdl ? 1 : 0;
-    }
-    lc.attrs = attr;
-    CU(cudaLaunchKernelEx(&lc, k_sums<M, XT, true, CP>, h->dc, tiles, cfg, theta, theta_is_q, i_raw, waner, pack, h->d_partial,
-                          h->d_ticket, sums, fin, pri, h->d_aux, traj, h->xch_active ? h->xch : XchCfg{}, ThetaInline{}));
-  } else {
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    lc.attrs = attr;
-    lc.numAttrs = h->use_pdl ? 1 : 0;
-    CU(cudaLaunchKernelEx(&lc, k_sums<M, XT, false, CP>, h->dc, tiles, cfg, theta, theta_is_q, i_raw, waner, pack, h->d_partial,
-                          h->d_ticket, sums, fin, pri, h->d_aux, traj, h->xch_active ? h->xch : XchCfg{}, thin));
-  }
-  return ABD_OK;
-}
-
+// `sharded`: the fused launch that all-reduces the sums with the peers of the exchange (see abd_xch_connect)
 int launch_sums(abd_handle* h, int C, const double* theta, int theta_is_q, const int8_t* i_raw,
                 const int8_t* waner, double* sums, const FinalizeCfg& fin, cudaStream_t st,
-                const TrajCfg* traj_in = nullptr) {
+                const TrajCfg* traj_in = nullptr, bool sharded = false) {
   TrajCfg traj{};
   if (traj_in) traj = *traj_in;
   const ThetaInline thin = h->thin;  // consumed by this call whatever happens below
   h->thin.n = 0;
+  // a single leapfrog step waits on nothing inside the grid: the ordinary plan with one chain per CTA (the trajectory
+  // variant keeps a chain's position in shared memory), any number of waves
+  const int cpc_fixed = traj.n_steps == 1 ? 1 : h->chains_per_cta_override;
   // plan for the kernel's register-limited occupancy first; if the tiles that plan needs do not
   // fit that many CTAs per SM (shared memory), plan again for what actually fits
   int want, cpc, rc;
@@ -578,16 +588,7 @@ int launch_sums(abd_handle* h, int C, const double* theta, int theta_is_q, const
   for (int attempt = 0; attempt < 2 * ABD_SUMS_MINB; ++attempt) {
     const int occ = ABD_SUMS_MINB - attempt / 2;
     const int one_wave_rows = (attempt & 1) ? 0 : kTileRowsOneWave;  // first with the larger one-wave tiles, then without
-    if (traj.n_steps == 1) {
-      // a single leapfrog step waits on nothing inside the grid: the ordinary plan with one chain per CTA (the
-      // trajectory variant keeps a chain's position in shared memory), any number of waves
-      const int keep = h->chains_per_cta_override;
-      h->chains_per_cta_override = 1;
-      plan_grid(h, C, occ, &want, &cpc, one_wave_rows);
-      h->chains_per_cta_override = keep;
-    } else {
-      plan_grid(h, C, occ, &want, &cpc, one_wave_rows);
-    }
+    plan_grid(h, C, occ, cpc_fixed, one_wave_rows, &want, &cpc);
     if (traj.n_steps > 1 && cpc != 1) {  // persistent trajectory: re-plan with one chain per CTA, exactly one wave
       cpc = 1;
       want = std::max((h->N + kTileMaxInds - 1) / kTileMaxInds, (h->n_sms * occ) / C);
@@ -599,14 +600,14 @@ int launch_sums(abd_handle* h, int C, const double* theta, int theta_is_q, const
     // eighth of the 100k cohort -- then run as one wave: 18.5 -> 11.6 us per launch)
     if (tl->smem && !tl->occ) {
       int o = 0;
-      CU(sums_occupancy_h(h, false, tl->smem, &o));
+      CU(sums_occupancy(h, false, tl->smem, &o));
       tl->occ = std::max(o, 1);
     }
     compact = false;
     if (tl->smem && tl->occ >= occ && !(h->force_compact && tl->smem_cp)) break;
     if (tl->smem_cp && !tl->occ_cp) {
       int o = 0;
-      CU(sums_occupancy_h(h, true, tl->smem_cp, &o));
+      CU(sums_occupancy(h, true, tl->smem_cp, &o));
       tl->occ_cp = std::max(o, 1);
     }
     compact = tl->smem_cp != 0;
@@ -622,25 +623,36 @@ int launch_sums(abd_handle* h, int C, const double* theta, int theta_is_q, const
   const size_t need = (size_t)C * tl->ntiles * kNSums;
   if (need > h->cap_partial) {
     CU(cudaStreamSynchronize(st));
-    if (h->d_partial) cudaFree(h->d_partial);
-    h->d_partial = nullptr;
+    h->partial_buf.release();
     h->cap_partial = 0;
-    if ((rc = dev_alloc(h, &h->d_partial, need, false))) return rc;
+    if ((rc = h->partial_buf.alloc(&h->d_partial, need))) return rc;
     h->cap_partial = need;
   }
   SumsCfg cfg{tl->ntiles, tl->cap_n, tl->cap_s, tl->capr_n, tl->capr_s, tl->capk_n, tl->capk_s, cpc, C};
   dim3 grid(tl->ntiles, (C + cpc - 1) / cpc);
+  const size_t smem = compact ? tl->smem_cp : tl->smem;
   h->last_plan[0] = tl->ntiles, h->last_plan[1] = (int)grid.y, h->last_plan[2] = cpc;
-  h->last_plan[3] = (int)(compact ? tl->smem_cp : tl->smem), h->last_plan[4] = compact ? 1 : 0, h->last_plan[5] = tl_occ;
+  h->last_plan[3] = (int)smem, h->last_plan[4] = compact ? 1 : 0, h->last_plan[5] = tl_occ;
   void* pack = nullptr;
   if ((rc = resident_pack(h, C, i_raw, waner, st, &pack))) return rc;
-  rc = with_mask(h, [&](auto m) {
-    using M = decltype(m);
-#define ABD_LAUNCH_SUMS(XT_, CP_) \
-  launch_sums_t<M, XT_, CP_>(h, *tl, cfg, grid, theta, theta_is_q, i_raw, waner, pack, sums, fin, traj, st, thin)
-    if (compact) return ABD_LAUNCH_SUMS(uint8_t, true);
-    return h->fx ? ABD_LAUNCH_SUMS(uint8_t, false) : ABD_LAUNCH_SUMS(double, false);
-#undef ABD_LAUNCH_SUMS
+  const bool tj = traj.n_steps > 0;
+  rc = with_sums(h, compact, tj, [&](auto k) -> int {
+    using K = decltype(k);
+    CU(sums_smem_attr(k, h->device, smem));
+    cudaLaunchAttribute attr;
+    cudaLaunchConfig_t lc = pdl_config(grid, dim3(kSumsBlock), smem, st, &attr);
+    if (traj.n_steps > 1) {  // CTAs wait on one another: they must all be resident
+      int occ = 0;
+      CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, K::fn(), kSumsBlock, smem));
+      if ((long)grid.x * grid.y > (long)occ * h->n_sms)
+        return fail(ABD_ERR_INVALID, "abd_leapfrog_dev: the grid does not fit on the device at once");
+      attr.id = cudaLaunchAttributeCooperative;
+      attr.val.cooperative = 1;
+    }
+    CU(cudaLaunchKernelEx(&lc, K::fn(), h->dc, reinterpret_cast<const TileDesc*>(tl->d_tiles), cfg, theta, theta_is_q, i_raw,
+                          waner, reinterpret_cast<const PackedState<typename K::Mask>*>(pack), h->d_partial, h->d_ticket, sums,
+                          fin, h->d_priors, h->d_aux, traj, sharded ? h->xch : XchCfg{}, tj ? ThetaInline{} : thin));
+    return ABD_OK;
   });
   if (rc) return rc;
   CU(cudaGetLastError());
@@ -703,47 +715,28 @@ int set_device(const abd_handle* h) {
   return ABD_OK;
 }
 
-// copy optional host state into the resident buffers
-// Host -> device copy of a chain-state array.  A copy-engine transfer of ~1 MB from pinned memory
-// takes ~60 us on a B200 host (PCIe gen5, measured, whatever the stream count); when the source is
-// pinned (page-locked, hence mapped into the device's address space under UVA) and 16-byte aligned,
-// the SMs pull it themselves with 16-byte loads -- every byte of the transfer is in flight at once
-// and the copy runs at the link's bandwidth.  Pageable sources take cudaMemcpyAsync.
-int copy_state_h2d(abd_handle* h, void* dst, const void* src, size_t bytes) {
-  if (bytes >= (4u << 10) && h->use_pull && (reinterpret_cast<uintptr_t>(src) & 15u) == 0) {
+// Copy of a chain-state array between the host and the device (`dir`).  A copy-engine transfer of ~1 MB from pinned
+// memory takes ~60 us on a B200 host (PCIe gen5, measured, whatever the stream count); when the host side is pinned
+// (page-locked, hence mapped into the device's address space under UVA) and 16-byte aligned, the SMs move it
+// themselves with 16-byte loads and stores -- every byte of the transfer is in flight at once and the copy runs at the
+// link's bandwidth (device -> host: posted PCIe writes).  Pageable host memory takes cudaMemcpyAsync.
+int copy_state(abd_handle* h, void* dst, const void* src, size_t bytes, cudaMemcpyKind dir) {
+  const bool h2d = dir == cudaMemcpyHostToDevice;
+  const void* host = h2d ? src : dst;
+  if (bytes >= (4u << 10) && (reinterpret_cast<uintptr_t>(host) & 15u) == 0) {
     cudaPointerAttributes at{};
-    if (cudaPointerGetAttributes(&at, src) == cudaSuccess && at.type == cudaMemoryTypeHost && at.devicePointer) {
+    if (cudaPointerGetAttributes(&at, host) == cudaSuccess && at.type == cudaMemoryTypeHost && at.devicePointer) {
       const size_t n16 = bytes / 16, rem = bytes - n16 * 16;
       const int grid = (int)std::min<size_t>((size_t)h->n_sms * 4, (n16 + 255) / 256);
-      k_pull<<<grid, 256, 0, h->stream>>>(reinterpret_cast<const uint4*>(at.devicePointer), reinterpret_cast<uint4*>(dst), n16,
-                                          rem);
+      k_pull<<<grid, 256, 0, h->stream>>>(reinterpret_cast<const uint4*>(h2d ? at.devicePointer : src),
+                                          reinterpret_cast<uint4*>(h2d ? dst : at.devicePointer), n16, rem);
       CU(cudaGetLastError());
       h->launches++;
       return ABD_OK;
     }
     cudaGetLastError();  // not a CUDA-known pointer: clear the sticky-free error and copy the ordinary way
   }
-  CU(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyHostToDevice, h->stream));
-  return ABD_OK;
-}
-
-// Device -> host copy of a chain-state array: pinned, 16-byte aligned destinations are written by
-// the SMs (posted PCIe writes), anything else by the copy engine.
-int copy_state_d2h(abd_handle* h, void* dst, const void* src, size_t bytes) {
-  if (bytes >= (4u << 10) && h->use_pull && (reinterpret_cast<uintptr_t>(dst) & 15u) == 0) {
-    cudaPointerAttributes at{};
-    if (cudaPointerGetAttributes(&at, dst) == cudaSuccess && at.type == cudaMemoryTypeHost && at.devicePointer) {
-      const size_t n16 = bytes / 16, rem = bytes - n16 * 16;
-      const int grid = (int)std::min<size_t>((size_t)h->n_sms * 4, (n16 + 255) / 256);
-      k_pull<<<grid, 256, 0, h->stream>>>(reinterpret_cast<const uint4*>(src), reinterpret_cast<uint4*>(at.devicePointer), n16,
-                                          rem);
-      CU(cudaGetLastError());
-      h->launches++;
-      return ABD_OK;
-    }
-    cudaGetLastError();
-  }
-  CU(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, h->stream));
+  CU(cudaMemcpyAsync(dst, src, bytes, dir, h->stream));
   return ABD_OK;
 }
 
@@ -754,64 +747,53 @@ int stage_state(abd_handle* h, int C, const int8_t* i_raw, const int8_t* waner) 
   // packed copy goes stale; a call on the resident state (NULL pointers) rebuilds it on first use
   h->lazy_pack = !(i_raw || waner);
   if (i_raw || waner) h->pack_valid = 0;
-  if (i_raw && (rc = copy_state_h2d(h, h->d_iraw, i_raw, (size_t)C * gn))) return rc;
-  if (waner && (rc = copy_state_h2d(h, h->d_waner, waner, (size_t)C * h->N))) return rc;
+  if (i_raw && (rc = copy_state(h, h->d_iraw, i_raw, (size_t)C * gn, cudaMemcpyHostToDevice))) return rc;
+  if (waner && (rc = copy_state(h, h->d_waner, waner, (size_t)C * h->N, cudaMemcpyHostToDevice))) return rc;
   return ABD_OK;
 }
 
-// A handle with its device facts, stream and environment switches (everything that does not depend on the cohort)
-int new_handle(abd_handle** out, int device, int G, int N, int mask_bits) {
+// A handle for the cohort `d` describes: its device facts, stream and priors, and every field the description fixes.
+// The cohort arrays follow (built by abd_create, read by abd_create_from_cache).
+int new_handle(abd_handle** out, int device, const CohortDesc& d) {
   abd_handle* h = new abd_handle();
   h->device = device;
-  if (const char* e = std::getenv("ABD_B200_NO_PDL")) h->use_pdl = !(e[0] == '1');
-  if (const char* e = std::getenv("ABD_B200_NO_PULL")) h->use_pull = !(e[0] == '1');
-  if (const char* e = std::getenv("ABD_B200_NO_INLINE")) h->use_inline = !(e[0] == '1');
-  if (const char* e = std::getenv("ABD_B200_NO_POLL")) h->use_poll = !(e[0] == '1');
-  if (const char* e = std::getenv("ABD_B200_NO_PACK")) h->use_pack = !(e[0] == '1');
   if (const char* e = std::getenv("ABD_B200_COMPACT_CELLS")) h->force_compact = (e[0] == '1');  // tests: compact cells wherever they exist
   {
     int v = 0;
     if (cudaDeviceGetAttribute(&v, cudaDevAttrMultiProcessorCount, device) == cudaSuccess && v > 0) h->n_sms = v;
     if (cudaDeviceGetAttribute(&v, cudaDevAttrMaxSharedMemoryPerBlockOptin, device) == cudaSuccess) h->smem_optin = (size_t)v;
   }
-  h->G = G;
-  h->N = N;
-  h->mask_bits = mask_bits;
-  if (cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking) != cudaSuccess) {
+  const CacheHeader& hd = d.hd;
+  h->desc = d;
+  h->G = h->dc.G = hd.G;
+  h->N = h->dc.N = hd.N;
+  h->mask_bits = 32 << hd.wide;
+  h->R[0] = hd.R[0], h->R[1] = hd.R[1];
+  h->tot = Totals{hd.tot[0], hd.tot[1], hd.tot[2], hd.tot[3]};
+  h->dc.ind_offset = hd.ind_offset;
+  h->dc.chain_offset = 0;
+  h->dc.ch.n = hd.n_chunks;
+  for (int k = 0; k < 3; ++k) h->dc.ch.mask[k] = hd.chunk_mask[k], h->dc.ch.mask_hi[k] = d.mask_hi[k];
+  h->fx = hd.fx != 0;
+  h->dc.n_xlev = hd.n_xlev;
+  int rc = ABD_OK;
+  double* d_lv = nullptr;
+  if (cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking) != cudaSuccess) rc = fail(ABD_ERR_CUDA, "cudaStreamCreate failed");
+  if (!rc) rc = upload(h, &d_lv, std::vector<double>(hd.xlev, hd.xlev + kMaxXLevels));
+  if (!rc) rc = upload(h, &h->d_priors, std::vector<Priors>{default_priors(hd.G)});
+  if (rc) {
     abd_destroy(h);
-    return fail(ABD_ERR_CUDA, "cudaStreamCreate failed");
+    return rc;
   }
+  h->dc.xlev = d_lv;
   *out = h;
   return ABD_OK;
 }
 
-// what every handle needs after its cohort arrays are on the device
-int finish_handle(abd_handle* h) {
-  int rc;
-  Priors pr = default_priors(h->G);
-  if ((rc = dev_alloc(h, &h->d_priors, 1))) return rc;
-  CU(cudaMemcpy(h->d_priors, &pr, sizeof(pr), cudaMemcpyHostToDevice));
-  return ABD_OK;
-}
-
-// ---- preprocessed-cohort cache file (SURVEY 8f-4: TiterData -> device upload format) -----------------
+// ---- preprocessed-cohort cache file ---------------------------------------------------------------------
 // Everything abd_create derives from the cohort (bit masks, CSR row / cell tables sorted by individual and
-// gap, packed row -> cell / dilution words, the Gibbs work order) as one binary file: a header, then the
-// arrays in a fixed order, each padded to 16 bytes.  Loading it is reading + uploading.
-struct CacheHeader {
-  char magic[8];           // "ABDB200\0"
-  int32_t version, G, N, n_chunks;
-  uint64_t chunk_mask[3];
-  int32_t wide, fx, n_xlev, has_pcr;   // wide: mask layout, 0 = 32, 1 = 64, 2 = 128 bits
-  int64_t R[2], K[2];      // OD rows / (individual, gap) cells per antigen (N, S)
-  double tot[4];
-  uint32_t ind_offset, pad;
-  double xlev[kMaxXLevels];
-};
-// Version 2: 32- and 64-bit masks.  Version 3 (128-bit masks): the same header, then the chunk masks' high words
-// (gaps 64..127) before the arrays.
-constexpr int kCacheVersion = 2, kCacheVersionWide = 3;
-
+// gap, packed row -> cell / dilution words, the Gibbs work order) as one binary file: the header (CacheHeader), then
+// the arrays in a fixed order, each padded to 16 bytes.  Loading it is reading + uploading.
 struct CacheIo {
   FILE* f = nullptr;
   bool writing = false, ok = true;
@@ -845,7 +827,8 @@ int cache_array(abd_handle* h, CacheIo& io, T** dptr, size_t n, std::vector<T>* 
 }
 
 // the cohort arrays of a handle, in file order (shared by save and load)
-int cache_body(abd_handle* h, CacheIo& io, const CacheHeader& hd) {
+int cache_body(abd_handle* h, CacheIo& io) {
+  const CacheHeader& hd = h->desc.hd;
   int rc;
   const size_t N = (size_t)hd.N;
   rc = with_mask(h, [&](auto m) {
@@ -882,7 +865,6 @@ int cache_body(abd_handle* h, CacheIo& io, const CacheHeader& hd) {
     }
     h->dc.rp[a] = rp, h->dc.x[a] = x, h->dc.od[a] = od, h->dc.meta[a] = meta, h->dc.rowcell[a] = rowcell;
     h->dc.cmeta[a] = cmeta, h->dc.rcx[a] = hd.fx ? rcx : nullptr;
-    h->R[a] = hd.R[a];
   }
   if ((rc = cache_array(h, io, &h->d_order, N))) return rc;
   return io.ok ? ABD_OK : fail(ABD_ERR_INVALID, "cache file I/O error");
@@ -914,6 +896,56 @@ bool wait_slots(const double* ho, size_t n) {
   return true;
 }
 
+// the first C x k doubles of `v` into the pinned staging buffer and on to d_theta
+int stage_params(abd_handle* h, int C, const double* v, int k) {
+  std::memcpy(h->h_pin, v, (size_t)C * k * sizeof(double));
+  CU(cudaMemcpyAsync(h->d_theta, h->h_pin, (size_t)C * k * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+  return ABD_OK;
+}
+
+// A host-pointer evaluation on the resident state: k = 13 parameters per chain (log-likelihood and its gradient) or 17
+// (joint logp and its gradient).  The finishing warps write the C values and C x k gradients straight into the pinned
+// staging buffer (posted PCIe writes cost the kernel nothing), behind the parameters; the host watches those slots
+// fill when there are few enough, else synchronises the stream.  Where the device cannot address the pinned buffer,
+// the results take a device -> host copy.  `counts`: also read back the Bernoulli counts of every chain.
+int eval_to_host(abd_handle* h, int C, const double* params, int k, double* out_val, double* out_grad, int64_t* counts) {
+  int rc;
+  if (C <= kInlineChains) {  // by value, inside the launch (no host -> device copy)
+    h->thin.n = C * k;
+    std::memcpy(h->thin.v, params, (size_t)C * k * sizeof(double));
+  } else if ((rc = stage_params(h, C, params, k))) {
+    return rc;
+  }
+  double* ho = h->h_pin + (size_t)C * 17;
+  double* dout = h->h_pin_dev ? h->h_pin_dev + (size_t)C * 17 : h->d_out;
+  const FinalizeCfg fin{k == 17 ? 2 : 1, h->tot, dout, dout + C};
+  const size_t nres = (size_t)C * (1 + k);
+  const bool poll = h->h_pin_dev && !counts && nres <= kMaxPolledSlots;
+  if (poll) unset_slots(ho, nres);
+  if ((rc = launch_sums(h, C, h->d_theta, k == 17, h->d_iraw, h->d_waner, h->d_sums, fin, h->stream))) return rc;
+  if (!h->h_pin_dev) CU(cudaMemcpyAsync(ho, h->d_out, nres * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+  // (the sums go where the parameters were staged: the launch has read those)
+  if (counts)
+    CU(cudaMemcpyAsync(h->h_pin, h->d_sums, (size_t)C * kNSums * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+  if (!(poll && wait_slots(ho, nres))) CU(cudaStreamSynchronize(h->stream));
+  std::memcpy(out_val, ho, (size_t)C * sizeof(double));
+  if (out_grad) std::memcpy(out_grad, ho + C, (size_t)C * k * sizeof(double));
+  if (counts)
+    for (int c = 0; c < C; ++c) {
+      counts[2 * c] = (int64_t)h->h_pin[(size_t)c * kNSums + S_KI];
+      counts[2 * c + 1] = (int64_t)h->h_pin[(size_t)c * kNSums + S_KW];
+    }
+  return ABD_OK;
+}
+
+// Fused sharded launches need the exchange allocated and connected, with room for C chains
+int check_xch(const abd_handle* h, int C, const char* fn) {
+  if (!h->xch_local || !h->xch.buf[h->xch.world - 1] || !h->xch.buf[0])
+    return fail(ABD_ERR_INVALID, std::string(fn) + ": call abd_xch_alloc and abd_xch_connect first");
+  if (C > h->xch.cmax) return fail(ABD_ERR_INVALID, "more chains than abd_xch_alloc reserved");
+  return ABD_OK;
+}
+
 #define PROLOGUE(h, C)                                         \
   if (!(h)) return fail(ABD_ERR_INVALID, "NULL handle");       \
   {                                                            \
@@ -936,10 +968,12 @@ int abd_create(abd_handle** out, const abd_cohort* co, int device) {
   const int G = co->n_gaps, N = co->n_inds;
   if (G < 1 || G > ABD_MAX_GAPS) return fail(ABD_ERR_INVALID, "n_gaps must be in [1, 127]");
   if (N < 1 || N >= (1 << 26)) return fail(ABD_ERR_INVALID, "n_inds must be in [1, 2^26)");
+  CohortDesc d{};
+  CacheHeader& hd = d.hd;
   // ABD_B200_MASK_BITS=128 (tests, measurements): the 128-bit layout whatever G
   const char* mb = std::getenv("ABD_B200_MASK_BITS");
-  const int mask_bits = (mb && std::strcmp(mb, "128") == 0) ? 128 : mask_bits_for(G);
-  if (mask_bits == 128 && N >= (1 << 25))
+  hd.wide = (mb && std::strcmp(mb, "128") == 0) ? 2 : wide_for(G);
+  if (hd.wide == 2 && N >= (1 << 25))
     return fail(ABD_ERR_INVALID, "n_inds must be < 2^25 with more than 63 gaps (128-bit masks)");
   if (!co->vacs) return fail(ABD_ERR_INVALID, "vacs is NULL");
   // check_splits, abd.py:604-622
@@ -953,56 +987,21 @@ int abd_create(abd_handle** out, const abd_cohort* co, int device) {
   if (co->n_splits == 2 && co->splits[0] > co->splits[1])
     return fail(ABD_ERR_INVALID, "splits must be in ascending order");
 
-  int ndev = 0;
-  CU(cudaGetDeviceCount(&ndev));
-  if (device < 0 || device >= ndev) return fail(ABD_ERR_CUDA, "no such CUDA device");
-  CU(cudaSetDevice(device));
-
-  abd_handle* h = nullptr;
-  {
-    int rc0 = new_handle(&h, device, G, N, mask_bits);
-    if (rc0) return rc0;
-  }
-  auto bail = [&](int rc) {
-    abd_destroy(h);
-    return rc;
-  };
-
-  // bit masks per individual
-  std::vector<u128> pcr((size_t)N, 0), vac((size_t)N, 0);
-  for (int t = 0; t < G; ++t)
-    for (int n = 0; n < N; ++n) {
-      if (co->pcrpos && co->pcrpos[(size_t)t * N + n]) pcr[n] |= (u128)1 << t;
-      if (co->vacs[(size_t)t * N + n]) vac[n] |= (u128)1 << t;
-    }
-  int rc = with_mask(h, [&](auto m) {
-    using M = decltype(m);
-    std::vector<M> pm(pcr.begin(), pcr.end()), vm(vac.begin(), vac.end());
-    M *dp, *dv;
-    int r;
-    if ((r = upload(h, &dp, pm)) || (r = upload(h, &dv, vm))) return r;
-    h->dc.pcr = dp;
-    h->dc.vac = dv;
-    return ABD_OK;
-  });
-  if (rc) return bail(rc);
-  h->dc.G = G;
-  h->dc.N = N;
-  h->dc.ind_offset = (unsigned)co->ind_offset;
-  h->dc.chain_offset = 0;
+  std::memcpy(hd.magic, "ABDB200", 8);
+  hd.version = hd.wide == 2 ? kCacheVersionWide : kCacheVersion;
+  hd.G = G, hd.N = N;
   // time chunks, abd.py:865-882
-  h->dc.ch.n = co->n_splits + 1;
+  hd.n_chunks = co->n_splits + 1;
   {
     int edges[4] = {0, 0, 0, 0};
     for (int k = 0; k < co->n_splits; ++k) edges[k + 1] = co->splits[k];
     edges[co->n_splits + 1] = G;
-    for (int k = 0; k < 3; ++k) h->dc.ch.mask[k] = h->dc.ch.mask_hi[k] = 0;
     for (int k = 0; k <= co->n_splits; ++k)
-      for (int t = edges[k]; t < edges[k + 1]; ++t) (t < 64 ? h->dc.ch.mask[k] : h->dc.ch.mask_hi[k]) |= 1ull << (t & 63);
+      for (int t = edges[k]; t < edges[k + 1]; ++t) (t < 64 ? hd.chunk_mask[k] : d.mask_hi[k]) |= 1ull << (t & 63);
   }
   // distinct dilutions over both antigens: <= 32 of them (and no NaN) enables the factored mode
   {
-    std::vector<double>& lv = h->x_levels;
+    std::vector<double> lv;
     bool ok = std::getenv("ABD_B200_NO_FACTORED") == nullptr;
     for (int a = 0; a < 2 && ok; ++a) {
       const double* xa = a ? co->x_s : co->x_n;
@@ -1020,17 +1019,55 @@ int abd_create(abd_handle** out, const abd_cohort* co, int device) {
       }
     }
     // a row packs its cell index in 27 bits
-    h->fx = ok && (co->n_rows_n < ((int64_t)1 << 27)) && (co->n_rows_s < ((int64_t)1 << 27));
-    if (!h->fx) lv.clear();
-    std::vector<double> padded(lv);
-    padded.resize(kMaxXLevels, 0.0);
-    double* d_lv;
-    if ((rc = upload(h, &d_lv, padded))) return bail(rc);
-    h->dc.xlev = d_lv;
-    h->dc.n_xlev = h->fx ? (int)lv.size() : 0;
+    hd.fx = ok && (co->n_rows_n < ((int64_t)1 << 27)) && (co->n_rows_s < ((int64_t)1 << 27));
+    if (hd.fx) {
+      hd.n_xlev = (int)lv.size();
+      std::copy(lv.begin(), lv.end(), hd.xlev);
+    }
   }
+  hd.has_pcr = co->pcrpos != nullptr;
+  hd.R[0] = co->n_rows_n, hd.R[1] = co->n_rows_s;
+  const double tn = co->total_inds > 0 ? (double)co->total_inds : (double)N;
+  hd.tot[0] = co->total_rows_n > 0 ? (double)co->total_rows_n : (double)co->n_rows_n;
+  hd.tot[1] = co->total_rows_s > 0 ? (double)co->total_rows_s : (double)co->n_rows_s;
+  hd.tot[2] = tn * G;
+  hd.tot[3] = tn;
+  hd.ind_offset = (uint32_t)co->ind_offset;
+
+  int ndev = 0;
+  CU(cudaGetDeviceCount(&ndev));
+  if (device < 0 || device >= ndev) return fail(ABD_ERR_CUDA, "no such CUDA device");
+  CU(cudaSetDevice(device));
+
+  abd_handle* h = nullptr;
+  int rc = new_handle(&h, device, d);
+  if (rc) return rc;
+  auto bail = [&](int r) {
+    abd_destroy(h);
+    return r;
+  };
+
+  // bit masks per individual
+  std::vector<u128> pcr((size_t)N, 0), vac((size_t)N, 0);
+  for (int t = 0; t < G; ++t)
+    for (int n = 0; n < N; ++n) {
+      if (co->pcrpos && co->pcrpos[(size_t)t * N + n]) pcr[n] |= (u128)1 << t;
+      if (co->vacs[(size_t)t * N + n]) vac[n] |= (u128)1 << t;
+    }
+  rc = with_mask(h, [&](auto m) {
+    using M = decltype(m);
+    std::vector<M> pm(pcr.begin(), pcr.end()), vm(vac.begin(), vac.end());
+    M *dp, *dv;
+    int r;
+    if ((r = upload(h, &dp, pm)) || (r = upload(h, &dv, vm))) return r;
+    h->dc.pcr = dp;
+    h->dc.vac = dv;
+    return ABD_OK;
+  });
+  if (rc) return bail(rc);
   if ((rc = build_rows(h, 0, co->n_rows_n, co->x_n, co->od_n, co->gap_n, co->ind_n))) return bail(rc);
   if ((rc = build_rows(h, 1, co->n_rows_s, co->x_s, co->od_s, co->gap_s, co->ind_s))) return bail(rc);
+  for (int a = 0; a < 2; ++a) h->desc.hd.K[a] = h->h_cp[a][N];
 
   {
     std::vector<int> order((size_t)N);
@@ -1041,14 +1078,6 @@ int abd_create(abd_handle** out, const abd_cohort* co, int device) {
     std::stable_sort(order.begin(), order.end(), [&](int a, int b) { return nrows(a) > nrows(b); });
     if ((rc = upload(h, &h->d_order, order))) return bail(rc);
   }
-  const double tn = co->total_inds > 0 ? (double)co->total_inds : (double)N;
-  h->tot.rows_n = co->total_rows_n > 0 ? (double)co->total_rows_n : (double)co->n_rows_n;
-  h->tot.rows_s = co->total_rows_s > 0 ? (double)co->total_rows_s : (double)co->n_rows_s;
-  h->tot.bits_i = tn * G;
-  h->tot.bits_w = tn;
-
-  h->has_pcr = co->pcrpos != nullptr;
-  if ((rc = finish_handle(h))) return bail(rc);
   *out = h;
   return ABD_OK;
 }
@@ -1058,23 +1087,13 @@ int abd_save_cache(abd_handle* h, const char* path) {
   int rc = set_device(h);
   if (rc) return rc;
   CU(cudaStreamSynchronize(h->stream));
-  CacheHeader hd{};
-  std::memcpy(hd.magic, "ABDB200", 8);
-  const bool v3 = h->mask_bits == 128;
-  hd.version = v3 ? kCacheVersionWide : kCacheVersion, hd.G = h->G, hd.N = h->N, hd.n_chunks = h->dc.ch.n;
-  for (int k = 0; k < 3; ++k) hd.chunk_mask[k] = h->dc.ch.mask[k];
-  hd.wide = h->mask_bits == 128 ? 2 : (h->mask_bits == 64 ? 1 : 0), hd.fx = h->fx, hd.n_xlev = h->dc.n_xlev, hd.has_pcr = h->has_pcr;
-  for (int a = 0; a < 2; ++a) hd.R[a] = h->R[a], hd.K[a] = h->h_cp[a].empty() ? 0 : h->h_cp[a].back();
-  hd.tot[0] = h->tot.rows_n, hd.tot[1] = h->tot.rows_s, hd.tot[2] = h->tot.bits_i, hd.tot[3] = h->tot.bits_w;
-  hd.ind_offset = h->dc.ind_offset;
-  for (size_t k = 0; k < h->x_levels.size() && k < (size_t)kMaxXLevels; ++k) hd.xlev[k] = h->x_levels[k];
   CacheIo io;
   io.writing = true;
   io.f = std::fopen(path, "wb");
   if (!io.f) return fail(ABD_ERR_INVALID, std::string("cannot write ") + path);
-  io.raw(&hd, sizeof(hd));
-  if (v3) io.raw(h->dc.ch.mask_hi, sizeof(h->dc.ch.mask_hi));
-  if ((rc = cache_body(h, io, hd))) return rc;
+  io.raw(&h->desc.hd, sizeof(h->desc.hd));
+  if (h->desc.hd.version == kCacheVersionWide) io.raw(h->desc.mask_hi, sizeof(h->desc.mask_hi));
+  if ((rc = cache_body(h, io))) return rc;
   return io.ok ? ABD_OK : fail(ABD_ERR_INVALID, "cache file I/O error");
 }
 
@@ -1084,16 +1103,15 @@ int abd_create_from_cache(abd_handle** out, const char* path, int device) {
   CacheIo io;
   io.f = std::fopen(path, "rb");
   if (!io.f) return fail(ABD_ERR_INVALID, std::string("cannot read ") + path);
-  CacheHeader hd{};
+  CohortDesc d{};
+  CacheHeader& hd = d.hd;
   io.raw(&hd, sizeof(hd));
   if (!io.ok || std::memcmp(hd.magic, "ABDB200", 8) != 0) return fail(ABD_ERR_INVALID, "not an abd_b200 cache file");
   if (hd.version != kCacheVersion && hd.version != kCacheVersionWide)
     return fail(ABD_ERR_INVALID, "cache file of another version: rebuild it");
   const bool v3 = hd.version == kCacheVersionWide;
-  const int mask_bits = v3 ? 128 : (hd.wide ? 64 : 32);
-  uint64_t mask_hi[3] = {0, 0, 0};
-  if (v3) io.raw(mask_hi, sizeof(mask_hi));
-  if (!io.ok || hd.G < 1 || hd.G > ABD_MAX_GAPS || hd.N < 1 || hd.N >= (mask_bits == 128 ? (1 << 25) : (1 << 26)) ||
+  if (v3) io.raw(d.mask_hi, sizeof(d.mask_hi));
+  if (!io.ok || hd.G < 1 || hd.G > ABD_MAX_GAPS || hd.N < 1 || hd.N >= (v3 ? (1 << 25) : (1 << 26)) ||
       hd.n_chunks < 1 || hd.n_chunks > 3 || hd.wide != (v3 ? 2 : (hd.G > 31 ? 1 : 0)) || (!v3 && hd.G > 63) ||
       hd.R[0] < 0 || hd.R[1] < 0 || hd.K[0] < 0 || hd.K[1] < 0 || hd.n_xlev < 0 || hd.n_xlev > kMaxXLevels)
     return fail(ABD_ERR_INVALID, "corrupt cache header");
@@ -1102,26 +1120,12 @@ int abd_create_from_cache(abd_handle** out, const char* path, int device) {
   if (device < 0 || device >= ndev) return fail(ABD_ERR_CUDA, "no such CUDA device");
   CU(cudaSetDevice(device));
   abd_handle* h = nullptr;
-  int rc = new_handle(&h, device, hd.G, hd.N, mask_bits);
+  int rc = new_handle(&h, device, d);
   if (rc) return rc;
-  auto bail = [&](int r) {
+  if ((rc = cache_body(h, io))) {
     abd_destroy(h);
-    return r;
-  };
-  h->dc.G = hd.G, h->dc.N = hd.N, h->dc.ind_offset = hd.ind_offset, h->dc.chain_offset = 0;
-  h->dc.ch.n = hd.n_chunks;
-  for (int k = 0; k < 3; ++k) h->dc.ch.mask[k] = hd.chunk_mask[k], h->dc.ch.mask_hi[k] = mask_hi[k];
-  h->fx = hd.fx != 0, h->has_pcr = hd.has_pcr != 0;
-  h->x_levels.assign(hd.xlev, hd.xlev + hd.n_xlev);
-  {
-    std::vector<double> padded(hd.xlev, hd.xlev + kMaxXLevels);
-    double* d_lv;
-    if ((rc = upload(h, &d_lv, padded))) return bail(rc);
-    h->dc.xlev = d_lv, h->dc.n_xlev = hd.n_xlev;
+    return rc;
   }
-  h->tot.rows_n = hd.tot[0], h->tot.rows_s = hd.tot[1], h->tot.bits_i = hd.tot[2], h->tot.bits_w = hd.tot[3];
-  if ((rc = cache_body(h, io, hd))) return bail(rc);
-  if ((rc = finish_handle(h))) return bail(rc);
   *out = h;
   return ABD_OK;
 }
@@ -1135,7 +1139,7 @@ int abd_cohort_info(const abd_handle* h, int32_t* n_splits, int32_t* splits, int
       const uint64_t lo = h->dc.ch.mask[k + 1], hi = h->dc.ch.mask_hi[k + 1];
       splits[k] = lo ? __builtin_ctzll(lo) : (hi ? 64 + __builtin_ctzll(hi) : h->G);
     }
-  if (has_pcrpos) *has_pcrpos = h->has_pcr ? 1 : 0;
+  if (has_pcrpos) *has_pcrpos = h->desc.hd.has_pcr ? 1 : 0;
   return ABD_OK;
 }
 
@@ -1145,13 +1149,9 @@ int abd_destroy(abd_handle* h) {
   if (h->stream) cudaStreamSynchronize(h->stream);
   for (void* p : h->xch_peer)
     if (p) cudaIpcCloseMemHandle(p);
-  if (h->xch_local) cudaFree(h->xch_local);
-  for (void* p : h->owned) cudaFree(p);
-  for (void* p : {(void*)h->d_iraw, (void*)h->d_waner, h->d_pack, (void*)h->d_theta, (void*)h->d_p, (void*)h->d_sums,
-                  (void*)h->d_out, (void*)h->d_ticket, (void*)h->d_stats, (void*)h->d_partial, (void*)h->d_aux, (void*)h->d_traj,
-                  (void*)h->d_gen, (void*)h->d_queue})
-    if (p) cudaFree(p);
-  if (h->h_pin) cudaFreeHost(h->h_pin);
+  h->owned.release();
+  free_chains(h);
+  h->partial_buf.release();
   if (h->stream) cudaStreamDestroy(h->stream);
   delete h;
   return ABD_OK;
@@ -1223,8 +1223,8 @@ int abd_download_state(abd_handle* h, int C, int8_t* i_raw, int8_t* waner) {
   PROLOGUE(h, C);
   const size_t gn = (size_t)h->G * h->N;
   int rc;
-  if (i_raw && (rc = copy_state_d2h(h, i_raw, h->d_iraw, (size_t)C * gn))) return rc;
-  if (waner && (rc = copy_state_d2h(h, waner, h->d_waner, (size_t)C * h->N))) return rc;
+  if (i_raw && (rc = copy_state(h, i_raw, h->d_iraw, (size_t)C * gn, cudaMemcpyDeviceToHost))) return rc;
+  if (waner && (rc = copy_state(h, waner, h->d_waner, (size_t)C * h->N, cudaMemcpyDeviceToHost))) return rc;
   CU(cudaStreamSynchronize(h->stream));
   return ABD_OK;
 }
@@ -1242,42 +1242,7 @@ int abd_loglik_grad(abd_handle* h, int C, const double* theta13, const int8_t* i
   if (!theta13 || !out_loglik) return fail(ABD_ERR_INVALID, "NULL argument");
   int rc = stage_state(h, C, i_raw, waner);
   if (rc) return rc;
-  if (C <= kInlineChains && h->use_inline) {  // by value, inside the launch (no host -> device copy)
-    h->thin.n = C * 13;
-    std::memcpy(h->thin.v, theta13, (size_t)C * 13 * sizeof(double));
-  } else {
-    std::memcpy(h->h_pin, theta13, (size_t)C * 13 * sizeof(double));
-    CU(cudaMemcpyAsync(h->d_theta, h->h_pin, (size_t)C * 13 * sizeof(double), cudaMemcpyHostToDevice, h->stream));
-  }
-  double* hp = h->h_pin;
-  if (!out_counts && out_grad && h->h_pin_dev && h->use_pull && h->use_poll && (size_t)C * 14 <= kMaxPolledSlots) {
-    // the per-leapfrog call of the PyTensor Op (resident state, no counts): results land in pinned memory and are
-    // watched for, as in abd_logp_dlogp
-    double* ho = hp + (size_t)C * 17;
-    double* dout = h->h_pin_dev + (size_t)C * 17;
-    FinalizeCfg finp{1, h->tot, dout, dout + C};
-    unset_slots(ho, (size_t)C * 14);
-    if ((rc = launch_sums(h, C, h->d_theta, 0, h->d_iraw, h->d_waner, h->d_sums, finp, h->stream))) return rc;
-    if (!wait_slots(ho, (size_t)C * 14)) CU(cudaStreamSynchronize(h->stream));
-    std::memcpy(out_loglik, ho, (size_t)C * sizeof(double));
-    std::memcpy(out_grad, ho + C, (size_t)C * 13 * sizeof(double));
-    return ABD_OK;
-  }
-  FinalizeCfg fin{1, h->tot, h->d_out, h->d_out + C};
-  if ((rc = launch_sums(h, C, h->d_theta, 0, h->d_iraw, h->d_waner, h->d_sums, fin, h->stream))) return rc;
-  CU(cudaMemcpyAsync(hp, h->d_out, (size_t)C * 14 * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
-  if (out_counts)
-    CU(cudaMemcpyAsync(hp + (size_t)C * 14, h->d_sums, (size_t)C * kNSums * sizeof(double),
-                       cudaMemcpyDeviceToHost, h->stream));
-  CU(cudaStreamSynchronize(h->stream));
-  std::memcpy(out_loglik, hp, (size_t)C * sizeof(double));
-  if (out_grad) std::memcpy(out_grad, hp + C, (size_t)C * 13 * sizeof(double));
-  if (out_counts)
-    for (int c = 0; c < C; ++c) {
-      out_counts[2 * c] = (int64_t)hp[(size_t)C * 14 + (size_t)c * kNSums + S_KI];
-      out_counts[2 * c + 1] = (int64_t)hp[(size_t)C * 14 + (size_t)c * kNSums + S_KW];
-    }
-  return ABD_OK;
+  return eval_to_host(h, C, theta13, 13, out_loglik, out_grad, out_counts);
 }
 
 int abd_logp_dlogp(abd_handle* h, int C, const double* q17, const int8_t* i_raw, const int8_t* waner,
@@ -1286,53 +1251,20 @@ int abd_logp_dlogp(abd_handle* h, int C, const double* q17, const int8_t* i_raw,
   if (!q17 || !out_logp) return fail(ABD_ERR_INVALID, "NULL argument");
   int rc = stage_state(h, C, i_raw, waner);
   if (rc) return rc;
-  // (Letting the kernel read the 17 scalars and write its results in place in the pinned staging
-  // buffer over PCIe was measured: 81 us per call instead of 41 -- every CTA pays sysmem latency for
-  // its parameter loads.  Small copy-engine transfers on both sides of the launch it is.)
-  // The RESULTS, however, are written by the finishing warps straight into the pinned staging
-  // buffer (posted PCIe writes cost the kernel nothing): no device -> host copy after the launch.
-  double* ho = h->h_pin + (size_t)C * 17;
-  if (C <= kInlineChains && h->use_inline) {  // by value, inside the launch (no host -> device copy)
-    h->thin.n = C * 17;
-    std::memcpy(h->thin.v, q17, (size_t)C * 17 * sizeof(double));
-  } else {
-    std::memcpy(h->h_pin, q17, (size_t)C * 17 * sizeof(double));
-    CU(cudaMemcpyAsync(h->d_theta, h->h_pin, (size_t)C * 17 * sizeof(double), cudaMemcpyHostToDevice, h->stream));
-  }
-  if (h->h_pin_dev && h->use_pull) {
-    double* dout = h->h_pin_dev + (size_t)C * 17;
-    FinalizeCfg fin{2, h->tot, dout, dout + C};
-    const size_t nres = (size_t)C * 18;
-    const bool poll = h->use_poll && nres <= kMaxPolledSlots;
-    if (poll) unset_slots(ho, nres);
-    if ((rc = launch_sums(h, C, h->d_theta, 1, h->d_iraw, h->d_waner, h->d_sums, fin, h->stream))) return rc;
-    if (poll && wait_slots(ho, nres)) {
-      std::memcpy(out_logp, ho, (size_t)C * sizeof(double));
-      if (out_dlogp) std::memcpy(out_dlogp, ho + C, (size_t)C * 17 * sizeof(double));
-      return ABD_OK;
-    }
-  } else {
-    FinalizeCfg fin{2, h->tot, h->d_out, h->d_out + C};
-    if ((rc = launch_sums(h, C, h->d_theta, 1, h->d_iraw, h->d_waner, h->d_sums, fin, h->stream))) return rc;
-    CU(cudaMemcpyAsync(ho, h->d_out, (size_t)C * 18 * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
-  }
-  CU(cudaStreamSynchronize(h->stream));
-  std::memcpy(out_logp, ho, (size_t)C * sizeof(double));
-  if (out_dlogp) std::memcpy(out_dlogp, ho + C, (size_t)C * 17 * sizeof(double));
-  return ABD_OK;
+  // (Letting the kernel read the 17 scalars in place in the pinned staging buffer over PCIe was measured: 81 us per
+  // call instead of 41 -- every CTA pays sysmem latency for its parameter loads.)
+  return eval_to_host(h, C, q17, 17, out_logp, out_dlogp, nullptr);
 }
 
 static int stage_gibbs_params(abd_handle* h, int C, const double* theta13, const double* p, const double* pw) {
   double* hp = h->h_pin;
-  std::memcpy(hp, theta13, (size_t)C * 13 * sizeof(double));
   for (int c = 0; c < C; ++c) {
     hp[(size_t)C * 13 + c] = p[c];
     hp[(size_t)C * 14 + c] = pw[c];
   }
-  CU(cudaMemcpyAsync(h->d_theta, hp, (size_t)C * 13 * sizeof(double), cudaMemcpyHostToDevice, h->stream));
   CU(cudaMemcpyAsync(h->d_p, hp + (size_t)C * 13, (size_t)C * 2 * sizeof(double), cudaMemcpyHostToDevice,
                      h->stream));
-  return ABD_OK;
+  return stage_params(h, C, theta13, 13);
 }
 
 int abd_cond_logodds(abd_handle* h, int C, const double* theta13, const double* p, const double* p_w,
@@ -1343,23 +1275,14 @@ int abd_cond_logodds(abd_handle* h, int C, const double* theta13, const double* 
   if (rc) return rc;
   if ((rc = stage_gibbs_params(h, C, theta13, p, p_w))) return rc;
   const size_t gn = (size_t)h->G * h->N;
-  double *d_oi = nullptr, *d_ow = nullptr;
-  if ((rc = dev_alloc(h, &d_oi, (size_t)C * gn, false))) return rc;
-  if ((rc = dev_alloc(h, &d_ow, (size_t)C * h->N, false))) {
-    cudaFree(d_oi);
-    return rc;
-  }
+  DevBufs tmp;
+  double *d_oi, *d_ow;
+  if ((rc = tmp.alloc(&d_oi, (size_t)C * gn)) || (rc = tmp.alloc(&d_ow, (size_t)C * h->N))) return rc;
   GibbsCfg cfg{0, 0, -1, 1.0, d_oi, d_ow, nullptr};
-  rc = launch_gibbs(h, C, h->d_theta, 0, h->d_p, h->d_p + C, h->d_iraw, h->d_waner, cfg, h->stream);
-  cudaError_t e1 = cudaMemcpyAsync(out_i, d_oi, (size_t)C * gn * sizeof(double), cudaMemcpyDeviceToHost, h->stream);
-  cudaError_t e2 = cudaMemcpyAsync(out_w, d_ow, (size_t)C * h->N * sizeof(double), cudaMemcpyDeviceToHost, h->stream);
-  cudaError_t e3 = cudaStreamSynchronize(h->stream);
-  cudaFree(d_oi);
-  cudaFree(d_ow);
-  if (rc) return rc;
-  CU(e1);
-  CU(e2);
-  CU(e3);
+  if ((rc = launch_gibbs(h, C, h->d_theta, 0, h->d_p, h->d_p + C, h->d_iraw, h->d_waner, cfg, h->stream))) return rc;
+  CU(cudaMemcpyAsync(out_i, d_oi, (size_t)C * gn * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+  CU(cudaMemcpyAsync(out_w, d_ow, (size_t)C * h->N * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+  CU(cudaStreamSynchronize(h->stream));
   return ABD_OK;
 }
 
@@ -1379,8 +1302,8 @@ int abd_gibbs_sweep(abd_handle* h, int C, const double* theta13, const double* p
   if ((rc = launch_gibbs(h, C, h->d_theta, 0, h->d_p, h->d_p + C, h->d_iraw, h->d_waner, cfg, h->stream)))
     return rc;
   const size_t gn = (size_t)h->G * h->N;
-  if (i_raw && (rc = copy_state_d2h(h, i_raw, h->d_iraw, (size_t)C * gn))) return rc;
-  if (waner && (rc = copy_state_d2h(h, waner, h->d_waner, (size_t)C * h->N))) return rc;
+  if (i_raw && (rc = copy_state(h, i_raw, h->d_iraw, (size_t)C * gn, cudaMemcpyDeviceToHost))) return rc;
+  if (waner && (rc = copy_state(h, waner, h->d_waner, (size_t)C * h->N, cudaMemcpyDeviceToHost))) return rc;
   if (out_stats)
     CU(cudaMemcpyAsync(h->h_pin, h->d_stats, (size_t)C * 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost,
                        h->stream));
@@ -1395,37 +1318,19 @@ int abd_deterministics(abd_handle* h, int C, const double* theta13, const int8_t
   if (!theta13) return fail(ABD_ERR_INVALID, "NULL argument");
   int rc = stage_state(h, C, i_raw, waner);
   if (rc) return rc;
-  std::memcpy(h->h_pin, theta13, (size_t)C * 13 * sizeof(double));
-  CU(cudaMemcpyAsync(h->d_theta, h->h_pin, (size_t)C * 13 * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+  if ((rc = stage_params(h, C, theta13, 13))) return rc;
   const size_t gn = (size_t)h->G * h->N * C;
+  DevBufs tmp;
   int8_t* d_i = nullptr;
   double *d_n = nullptr, *d_s = nullptr;
-  auto cleanup = [&]() {
-    if (d_i) cudaFree(d_i);
-    if (d_n) cudaFree(d_n);
-    if (d_s) cudaFree(d_s);
-  };
-  if (out_i && (rc = dev_alloc(h, &d_i, gn, false))) return rc;
-  if (out_mu_n && (rc = dev_alloc(h, &d_n, gn, false))) {
-    cleanup();
+  if ((out_i && (rc = tmp.alloc(&d_i, gn))) || (out_mu_n && (rc = tmp.alloc(&d_n, gn))) ||
+      (out_mu_s && (rc = tmp.alloc(&d_s, gn))))
     return rc;
-  }
-  if (out_mu_s && (rc = dev_alloc(h, &d_s, gn, false))) {
-    cleanup();
-    return rc;
-  }
-  rc = abd_deterministics_dev(h, C, h->d_theta, h->d_iraw, h->d_waner, d_i, d_n, d_s, h->stream);
-  cudaError_t e = cudaSuccess;
-  if (!rc && out_i) e = cudaMemcpyAsync(out_i, d_i, gn, cudaMemcpyDeviceToHost, h->stream);
-  if (!rc && e == cudaSuccess && out_mu_n)
-    e = cudaMemcpyAsync(out_mu_n, d_n, gn * sizeof(double), cudaMemcpyDeviceToHost, h->stream);
-  if (!rc && e == cudaSuccess && out_mu_s)
-    e = cudaMemcpyAsync(out_mu_s, d_s, gn * sizeof(double), cudaMemcpyDeviceToHost, h->stream);
-  cudaError_t e2 = cudaStreamSynchronize(h->stream);
-  cleanup();
-  if (rc) return rc;
-  CU(e);
-  CU(e2);
+  if ((rc = abd_deterministics_dev(h, C, h->d_theta, h->d_iraw, h->d_waner, d_i, d_n, d_s, h->stream))) return rc;
+  if (out_i) CU(cudaMemcpyAsync(out_i, d_i, gn, cudaMemcpyDeviceToHost, h->stream));
+  if (out_mu_n) CU(cudaMemcpyAsync(out_mu_n, d_n, gn * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+  if (out_mu_s) CU(cudaMemcpyAsync(out_mu_s, d_s, gn * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+  CU(cudaStreamSynchronize(h->stream));
   return ABD_OK;
 }
 
@@ -1435,25 +1340,15 @@ int abd_loglik_rows(abd_handle* h, int C, const double* theta13, const int8_t* i
   if (!theta13) return fail(ABD_ERR_INVALID, "NULL argument");
   int rc = stage_state(h, C, i_raw, waner);
   if (rc) return rc;
-  std::memcpy(h->h_pin, theta13, (size_t)C * 13 * sizeof(double));
-  CU(cudaMemcpyAsync(h->d_theta, h->h_pin, (size_t)C * 13 * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+  if ((rc = stage_params(h, C, theta13, 13))) return rc;
+  DevBufs tmp;
   double *d_s = nullptr, *d_n = nullptr;
-  if (out_s && (rc = dev_alloc(h, &d_s, (size_t)C * h->R[1], false))) return rc;
-  if (out_n && (rc = dev_alloc(h, &d_n, (size_t)C * h->R[0], false))) {
-    if (d_s) cudaFree(d_s);
+  if ((out_s && (rc = tmp.alloc(&d_s, (size_t)C * h->R[1]))) || (out_n && (rc = tmp.alloc(&d_n, (size_t)C * h->R[0]))))
     return rc;
-  }
-  rc = abd_loglik_rows_dev(h, C, h->d_theta, h->d_iraw, h->d_waner, d_s, d_n, h->stream);
-  cudaError_t e = cudaSuccess;
-  if (!rc && out_s) e = cudaMemcpyAsync(out_s, d_s, (size_t)C * h->R[1] * sizeof(double), cudaMemcpyDeviceToHost, h->stream);
-  if (!rc && e == cudaSuccess && out_n)
-    e = cudaMemcpyAsync(out_n, d_n, (size_t)C * h->R[0] * sizeof(double), cudaMemcpyDeviceToHost, h->stream);
-  cudaError_t e2 = cudaStreamSynchronize(h->stream);
-  if (d_s) cudaFree(d_s);
-  if (d_n) cudaFree(d_n);
-  if (rc) return rc;
-  CU(e);
-  CU(e2);
+  if ((rc = abd_loglik_rows_dev(h, C, h->d_theta, h->d_iraw, h->d_waner, d_s, d_n, h->stream))) return rc;
+  if (out_s) CU(cudaMemcpyAsync(out_s, d_s, (size_t)C * h->R[1] * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+  if (out_n) CU(cudaMemcpyAsync(out_n, d_n, (size_t)C * h->R[0] * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+  CU(cudaStreamSynchronize(h->stream));
   return ABD_OK;
 }
 
@@ -1643,22 +1538,11 @@ int abd_nuts_leaf_dev(abd_handle* h, int C, int max_depth, int depth, int leaf, 
     return fail(ABD_ERR_INVALID, "NULL argument");
   if (max_depth < 1 || max_depth > kNutsMaxDepth || depth < 0 || depth >= max_depth || leaf < 0 || leaf >= (1 << depth))
     return fail(ABD_ERR_INVALID, "bad depth / leaf");
-  {
-    cudaLaunchConfig_t lc{};
-    lc.gridDim = dim3((C + 3) / 4);
-    lc.blockDim = dim3(128);
-    lc.stream = (cudaStream_t)stream;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    lc.attrs = attr;
-    lc.numAttrs = h->use_pdl ? 1 : 0;
-    const NutsLeafArgs a{state, NutsLayout{max_depth}, depth, leaf, max_depth, eps, seed, iter, h->dc.chain_offset, eps_signed,
-                         any_active};
-    const double* lpw_c = lpw;
-    const double* im_c = inv_mass;
-    CU(cudaLaunchKernelEx(&lc, k_nuts_leaf, C, a, qw, pw, gw, lpw_c, im_c));
-  }
+  cudaLaunchAttribute attr;
+  const cudaLaunchConfig_t lc = pdl_config(dim3((C + 3) / 4), dim3(128), 0, (cudaStream_t)stream, &attr);
+  const NutsLeafArgs a{state, NutsLayout{max_depth}, depth, leaf, max_depth, eps, seed, iter, h->dc.chain_offset, eps_signed,
+                       any_active};
+  CU(cudaLaunchKernelEx(&lc, k_nuts_leaf, C, a, qw, pw, gw, lpw, inv_mass));
   CU(cudaGetLastError());
   h->launches++;
   return ABD_OK;
@@ -1675,18 +1559,15 @@ int abd_nuts_extend_dev(abd_handle* h, int C, int max_depth, int depth, double* 
     return fail(ABD_ERR_INVALID, "NULL argument");
   if (max_depth < 1 || max_depth > kNutsMaxDepth) return fail(ABD_ERR_INVALID, "max_depth must be in [1, 10]");
   const bool sharded = h->xch_local != nullptr;
-  if (sharded && (!h->xch.buf[h->xch.world - 1] || !h->xch.buf[0] || C > h->xch.cmax))
-    return fail(ABD_ERR_INVALID, "abd_nuts_extend_dev on a sharded handle: connect the exchange first (and reserve enough chains)");
+  int rc;
+  if (sharded && (rc = check_xch(h, C, "abd_nuts_extend_dev"))) return rc;
   for (int n = 0; n < (1 << depth); ++n) {
     // the leaf's leapfrog step and its tree bookkeeping in ONE launch (the finishing warp of each chain does both)
     TrajCfg traj{1, qw, pw, gw, lpw, eps_signed, inv_mass, h->d_traj, h->d_gen, h->d_gen + C,
                  NutsLeafArgs{state, NutsLayout{max_depth}, depth, n, max_depth, eps, seed, iter, h->dc.chain_offset, eps_signed,
                               any_active}};
     FinalizeCfg fin{2, h->tot, nullptr, nullptr};
-    h->xch_active = sharded;
-    const int rc = launch_sums(h, C, qw, 1, i_raw, waner, nullptr, fin, (cudaStream_t)stream, &traj);
-    h->xch_active = false;
-    if (rc) return rc;
+    if ((rc = launch_sums(h, C, qw, 1, i_raw, waner, nullptr, fin, (cudaStream_t)stream, &traj, sharded))) return rc;
   }
   return ABD_OK;
 }
@@ -1714,13 +1595,15 @@ int abd_xch_alloc(abd_handle* h, int world, int rank, int max_chains, void* out_
   if (rc) return rc;
   if (h->xch_local) return fail(ABD_ERR_INVALID, "abd_xch_alloc: already allocated");
   const size_t bytes = (size_t)2 * world * max_chains * 32 * sizeof(unsigned long long);
-  CU(cudaMalloc(&h->xch_local, bytes));
+  char* local;
+  if ((rc = h->owned.alloc(&local, bytes))) return rc;
+  h->xch_local = local;
   CU(cudaMemset(h->xch_local, 0, bytes));
   unsigned* seq;
-  if ((rc = dev_alloc(h, &seq, (size_t)max_chains + 1))) return rc;
+  if ((rc = h->owned.alloc(&seq, (size_t)max_chains + 1))) return rc;
   CU(cudaMemset(seq, 0, ((size_t)max_chains + 1) * sizeof(unsigned)));
   unsigned long long* stat;
-  if ((rc = dev_alloc(h, &stat, (size_t)kMaxPeers + 1))) return rc;
+  if ((rc = h->owned.alloc(&stat, (size_t)kMaxPeers + 1))) return rc;
   CU(cudaMemset(stat, 0, ((size_t)kMaxPeers + 1) * sizeof(unsigned long long)));
   h->xch = XchCfg{};
   h->xch.world = world;
@@ -1760,14 +1643,9 @@ int abd_logp_dlogp_sharded_dev(abd_handle* h, int C, const double* q17, const in
   PROLOGUE(h, C);
   h->lazy_pack = true;
   if (!q17 || !i_raw || !waner || !out_logp) return fail(ABD_ERR_INVALID, "NULL argument");
-  if (!h->xch_local || !h->xch.buf[h->xch.world - 1] || !h->xch.buf[0])
-    return fail(ABD_ERR_INVALID, "abd_logp_dlogp_sharded_dev: call abd_xch_alloc and abd_xch_connect first");
-  if (C > h->xch.cmax) return fail(ABD_ERR_INVALID, "more chains than abd_xch_alloc reserved");
+  if (int rc = check_xch(h, C, "abd_logp_dlogp_sharded_dev")) return rc;
   FinalizeCfg fin{2, h->tot, out_logp, out_dlogp};
-  h->xch_active = true;
-  const int rc = launch_sums(h, C, q17, 1, i_raw, waner, h->d_sums, fin, (cudaStream_t)stream);
-  h->xch_active = false;
-  return rc;
+  return launch_sums(h, C, q17, 1, i_raw, waner, h->d_sums, fin, (cudaStream_t)stream, nullptr, true);
 }
 
 int abd_leapfrog_sharded_dev(abd_handle* h, int C, double* q17, double* p17, double* grad17, double* logp, const double* eps,
@@ -1775,15 +1653,10 @@ int abd_leapfrog_sharded_dev(abd_handle* h, int C, double* q17, double* p17, dou
   PROLOGUE(h, C);
   h->lazy_pack = true;
   if (!q17 || !p17 || !grad17 || !logp || !eps || !inv_mass || !i_raw || !waner) return fail(ABD_ERR_INVALID, "NULL argument");
-  if (!h->xch_local || !h->xch.buf[h->xch.world - 1] || !h->xch.buf[0])
-    return fail(ABD_ERR_INVALID, "abd_leapfrog_sharded_dev: call abd_xch_alloc and abd_xch_connect first");
-  if (C > h->xch.cmax) return fail(ABD_ERR_INVALID, "more chains than abd_xch_alloc reserved");
+  if (int rc = check_xch(h, C, "abd_leapfrog_sharded_dev")) return rc;
   TrajCfg traj{1, q17, p17, grad17, logp, eps, inv_mass, h->d_traj, h->d_gen, h->d_gen + C, NutsLeafArgs{}};
   FinalizeCfg fin{2, h->tot, nullptr, nullptr};
-  h->xch_active = true;
-  const int rc = launch_sums(h, C, q17, 1, i_raw, waner, nullptr, fin, (cudaStream_t)stream, &traj);
-  h->xch_active = false;
-  return rc;
+  return launch_sums(h, C, q17, 1, i_raw, waner, nullptr, fin, (cudaStream_t)stream, &traj, true);
 }
 
 int abd_xch_stats(abd_handle* h, uint64_t* out, int reset) {
@@ -1808,22 +1681,16 @@ int abd_xch_status(abd_handle* h) {
 int abd_debug_fast_math(int device, int64_t n, const double* z, double* out_exp, double* out_rcp) {
   if (n < 0 || !z || !out_exp || !out_rcp) return fail(ABD_ERR_INVALID, "bad argument");
   CU(cudaSetDevice(device));
-  double *dz = nullptr, *de = nullptr, *dr = nullptr;
-  const size_t bytes = (size_t)std::max<int64_t>(n, 1) * sizeof(double);
-  CU(cudaMalloc((void**)&dz, bytes));
-  CU(cudaMalloc((void**)&de, bytes));
-  CU(cudaMalloc((void**)&dr, bytes));
-  cudaError_t e = cudaMemcpy(dz, z, (size_t)n * sizeof(double), cudaMemcpyHostToDevice);
-  if (e == cudaSuccess) {
-    k_debug_fast_math<<<296, 256>>>(n, dz, de, dr);
-    e = cudaGetLastError();
-  }
-  if (e == cudaSuccess) e = cudaMemcpy(out_exp, de, (size_t)n * sizeof(double), cudaMemcpyDeviceToHost);
-  if (e == cudaSuccess) e = cudaMemcpy(out_rcp, dr, (size_t)n * sizeof(double), cudaMemcpyDeviceToHost);
-  cudaFree(dz);
-  cudaFree(de);
-  cudaFree(dr);
-  CU(e);
+  DevBufs tmp;
+  double *dz, *de, *dr;
+  const size_t n1 = (size_t)std::max<int64_t>(n, 1);
+  int rc;
+  if ((rc = tmp.alloc(&dz, n1)) || (rc = tmp.alloc(&de, n1)) || (rc = tmp.alloc(&dr, n1))) return rc;
+  CU(cudaMemcpy(dz, z, (size_t)n * sizeof(double), cudaMemcpyHostToDevice));
+  k_debug_fast_math<<<296, 256>>>(n, dz, de, dr);
+  CU(cudaGetLastError());
+  CU(cudaMemcpy(out_exp, de, (size_t)n * sizeof(double), cudaMemcpyDeviceToHost));
+  CU(cudaMemcpy(out_rcp, dr, (size_t)n * sizeof(double), cudaMemcpyDeviceToHost));
   return ABD_OK;
 }
 

@@ -159,7 +159,7 @@ int abd_logp_dlogp(abd_handle* h, int n_chains, const double* q17, const int8_t*
  * straight into pinned host memory and the library watches them arrive instead of waiting for the end
  * of the stream -- for <= 64 chains, falling back to cudaStreamSynchronize after 150 us; the handle's
  * stream may still be draining the launch's last CTAs, which later calls on the handle are ordered
- * behind.  ABD_B200_NO_POLL=1 restores the stream synchronisation.)                                   */
+ * behind.)                                                                                           */
 
 /* Conditional log-odds of every binary variable given all others (test hook; what "Gibbs
  * parity" means, SURVEY.md section 8a):  out_i[c][t][n] = logp(i_raw[t,n]=1 | rest) -

@@ -57,6 +57,6 @@ lib.abd_debug_spans(buf.ctypes.data_as(C.c_void_p), 0)
 s = buf[:n].astype(np.int64)
 span = (s[:, 1] - s[:, 0]) / 1e3
 gap = (s[1:, 0] - s[:-1, 1]) / 1e3
-print(f"C={C_} PDL={'off' if os.environ.get('ABD_B200_NO_PDL') == '1' else 'on'}: graph of {n} launches {e0.elapsed_time(e1) * 1e3 / n:.2f} us/launch; "
+print(f"C={C_}: graph of {n} launches {e0.elapsed_time(e1) * 1e3 / n:.2f} us/launch; "
       f"kernel span median {np.median(span):.2f} (min {span.min():.2f}, max {span.max():.2f}); gap start-after-end median {np.median(gap):.2f} "
       f"(min {gap.min():.2f}, max {gap.max():.2f})")
