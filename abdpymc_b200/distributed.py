@@ -21,8 +21,12 @@ from __future__ import annotations
 import os
 
 import numpy as np
+import torch
+import torch.distributed as dist
 
 from .cohort import CohortArrays, shard_bounds
+from .engine import AbdEngine
+from .sampler import DeviceTarget
 
 N_SUMS = 16
 
@@ -35,8 +39,6 @@ def dist_env():
 def init_process_group(backend=None, device=None):
     """Initialise torch.distributed from the torchrun environment; no-op for a single process.
     NCCL when a CUDA device is given, gloo otherwise (CPU tests)."""
-    import torch.distributed as dist
-
     rank, world, _ = dist_env()
     if world == 1 or dist.is_initialized():
         return dist if world > 1 else None
@@ -69,17 +71,9 @@ def shard_cohort(cohort: CohortArrays, rank: int, world: int):
 def allreduce_sums(sums, group=None):
     """Sum the per-shard raw sums (C x 16 doubles, every entry additive over individuals) over
     all ranks, in place.  ``sums``: torch tensor on the device the process group runs on."""
-    import torch.distributed as dist
-
     if dist.is_available() and dist.is_initialized() and dist.get_world_size(group) > 1:
         dist.all_reduce(sums, op=dist.ReduceOp.SUM, group=group)
     return sums
-
-
-def _nuts_mixin():
-    from .sampler import DeviceNutsMixin
-
-    return DeviceNutsMixin
 
 
 class ShardedEngine:
@@ -95,10 +89,6 @@ class ShardedEngine:
         (``abd_logp_dlogp_sharded_dev``: every rank's finishing CTA stores its sums into all peers'
         exchange buffers and waits for theirs) -- one launch per evaluation, no NCCL call.  Needs
         an initialised process group once, to exchange the CUDA IPC handles."""
-        import torch
-
-        from .engine import AbdEngine
-
         env_rank, env_world, _ = dist_env()
         self.rank = env_rank if rank is None else rank
         self.world = env_world if world is None else world
@@ -111,8 +101,6 @@ class ShardedEngine:
         self._bufs = {}
         self.fused = bool(fused) and self.world > 1
         if self.fused:
-            import torch.distributed as dist
-
             mine = self.engine.xch_alloc(self.world, self.rank, max_chains)
             handles = [None] * self.world
             dist.all_gather_object(handles, mine, group=group)
@@ -120,8 +108,6 @@ class ShardedEngine:
             dist.barrier(group=group)  # every rank has mapped every buffer before the first launch
 
     def _buffers(self, C):
-        import torch
-
         if C not in self._bufs:
             self._bufs[C] = (
                 torch.zeros(C, N_SUMS, dtype=torch.float64, device=self.device),
@@ -140,8 +126,6 @@ class ShardedEngine:
         """``q17``: torch (C, 17) float64 tensor on this rank's device (identical on all ranks).
         Uses the resident chain state.  Returns (logp (C,), dlogp (C, 17)) device tensors (``out`` /
         ``outg`` when given, otherwise buffers reused by the next call)."""
-        import torch
-
         C = q17.shape[0] if n_chains is None else n_chains
         sums, out_, outg_ = self._buffers(C)
         out = out_ if out is None else out
@@ -156,26 +140,6 @@ class ShardedEngine:
         self.engine.finalize_logp_dev(C, q17.data_ptr(), sums.data_ptr(), out.data_ptr(), outg.data_ptr(), st)
         return out, outg
 
-    def gibbs_sweep(self, q17, seed, sweep, mode=0, transit_p=0.8):
-        """Sweep this rank's individuals of every chain in place (no collective: theta is the
-        same on every rank, updates are local; RNG streams are keyed by GLOBAL individual)."""
-        import torch
-
-        C = q17.shape[0]
-        st = torch.cuda.current_stream(self.device).cuda_stream
-        d_i, d_w = self.engine.state_dev(C)
-        self.engine.gibbs_sweep_dev(C, q17.data_ptr(), 1, None, None, d_i, d_w, seed, sweep, mode=mode,
-                                    transit_p=transit_p, stream=st)
-
-    def leapfrog_step(self, C, q, p, grad, logp, eps, inv_mass):
-        """One leapfrog step in place (device tensors), the exchange fused into the launch (fused engines only)."""
-        import torch
-
-        st = torch.cuda.current_stream(self.device).cuda_stream
-        d_i, d_w = self.engine.state_dev(C)
-        self.engine.leapfrog_sharded_dev(C, q.data_ptr(), p.data_ptr(), grad.data_ptr(), logp.data_ptr(), eps.data_ptr(),
-                                         inv_mass.data_ptr(), d_i, d_w, st)
-
     def exchange_wait_us(self, reset=True):
         """Mean time (us) the finishing CTA of an evaluation spent waiting for its slowest peer's contribution
         -- launch skew between the ranks plus NVLink latency -- since the last reset (fused engines only)."""
@@ -186,7 +150,7 @@ class ShardedEngine:
         self.engine.close()
 
 
-class ShardedTarget(_nuts_mixin()):
+class ShardedTarget(DeviceTarget):
     """The posterior of an INDIVIDUAL-SHARDED cohort as a sampler target (same interface as
     ``sampler.AbdTarget``): every rank holds a contiguous block of individuals and the matching slice of
     every chain's binary state; the 17 scalars, their momenta, step sizes and the metric are replicated.
@@ -199,92 +163,30 @@ class ShardedTarget(_nuts_mixin()):
       (seed; iteration, chain) -- the same seed on every rank gives the same momenta and decisions.
     * Gibbs sweep: local, no communication (individuals are conditionally independent given the
       scalars; streams keyed by GLOBAL individual, so the draws do not depend on the sharding).
-    What abd.py:922 runs as NUTS + BinaryGibbsMetropolis on one CPU core per chain."""
+    What abd.py:922 runs as NUTS + BinaryGibbsMetropolis on one CPU core per chain.  Its draws of the (G, N)
+    Deterministics are not gathered over the ranks, so it has no ``deterministics`` / ``loglik_rows``."""
 
     def __init__(self, sharded: ShardedEngine, n_chains, i_raw, waner, seed=0, gibbs_mode=0, transit_p=0.8):
-        import torch
-
-        self.sh, self.engine, self.C = sharded, sharded.engine, n_chains
-        self.device = sharded.device
+        super().__init__(sharded.engine, n_chains, sharded.device, seed, gibbs_mode, transit_p)
+        self.sh, self.device_loop = sharded, sharded.fused
         sharded.upload_state(i_raw, waner)          # (C, G, N_total) / (C, N_total): this rank keeps its block
-        self.seed, self.gibbs_mode, self.transit_p = seed, gibbs_mode, transit_p
-        self.dim = 17
-        self.out = torch.zeros(n_chains, dtype=torch.float64, device=self.device)
-        self.outg = torch.zeros(n_chains, 17, dtype=torch.float64, device=self.device)
-        if sharded.fused:  # the device-resident transitions of sampler._sample_fused (HMC and No-U-Turn)
-            self.hmc_begin, self.hmc_end = self._hmc_begin, self._hmc_end
-            self.nuts_extend_in_library = True   # abd_nuts_extend_dev exchanges inside its leapfrog launches
-        else:              # host-driven loop: hide the device tree methods
-            self.nuts_begin = None
-
-    def _stream(self):
-        import torch
-
-        return torch.cuda.current_stream(self.device).cuda_stream
-
-    @property
-    def d_i(self):
-        return self.engine.state_dev(self.C)[0]
-
-    @property
-    def d_w(self):
-        return self.engine.state_dev(self.C)[1]
-
-    def logp_dlogp(self, q):
-        lp, g = self.sh.logp_dlogp(q.contiguous(), self.C)
-        return lp.clone(), g.clone()
 
     def logp_dlogp_into(self, q, logp, grad):
         self.sh.logp_dlogp(q, self.C, out=logp, outg=grad)
 
+    def leapfrog_inplace(self, q, p, grad, logp, eps, inv_mass, n_steps):
+        """One launch per step, the exchange fused into it (fused engines only)."""
+        for _ in range(n_steps):
+            self.engine.leapfrog_sharded_dev(self.C, q.data_ptr(), p.data_ptr(), grad.data_ptr(), logp.data_ptr(), eps.data_ptr(),
+                                             inv_mass.data_ptr(), self.d_i, self.d_w, self._stream())
+
     def check_status(self):
-        self.engine.leapfrog_status(self.C)
+        super().check_status()
         if self.sh.fused:
             self.engine.xch_status()
 
-    def leapfrog_inplace(self, q, p, grad, logp, eps, inv_mass, n_steps):
-        for _ in range(n_steps):
-            self.sh.leapfrog_step(self.C, q, p, grad, logp, eps, inv_mass)
-
-    def _hmc_begin(self, q, grad, logp, linv_t, it, qw, pw, gw, h0):
-        self.engine.hmc_begin_dev(self.C, q.data_ptr(), grad.data_ptr(), logp.data_ptr(), linv_t.data_ptr(), self.seed, it,
-                                  qw.data_ptr(), pw.data_ptr(), gw.data_ptr(), h0.data_ptr(), self._stream())
-
-    def _hmc_end(self, q, grad, logp, qw, pw, gw, lpw, inv_mass, h0, it, acc, da, eps, adapt, target_accept):
-        self.engine.hmc_end_dev(self.C, q.data_ptr(), grad.data_ptr(), logp.data_ptr(), qw.data_ptr(), pw.data_ptr(),
-                                gw.data_ptr(), lpw.data_ptr(), inv_mass.data_ptr(), h0.data_ptr(), self.seed, it,
-                                acc.data_ptr(), da.data_ptr(), eps.data_ptr(), adapt, target_accept, self._stream())
-
-    def gibbs(self, q, sweep):
-        self.sh.gibbs_sweep(q.contiguous(), self.seed, sweep, mode=self.gibbs_mode, transit_p=self.transit_p)
-
-    def fits_persistent(self):
-        return self.sh.fused
-
-    def accumulate_deterministics(self, q, sums):
-        """Running totals of i, ab_n_mu, ab_s_mu over this rank's individuals: (G, N_local) device tensors."""
-        import torch
-
-        G, N = self.engine.G, self.engine.N
-        for name in ("i", "ab_n_mu", "ab_s_mu"):
-            if name not in sums:
-                sums[name] = torch.zeros(G, N, dtype=torch.float64, device=self.device)
-        q = q.contiguous()
-        d_i, d_w = self.engine.state_dev(self.C)
-        self.engine.deterministics_accum_dev(self.C, q.data_ptr(), 1, d_i, d_w, sums["i"].data_ptr(),
-                                             sums["ab_n_mu"].data_ptr(), sums["ab_s_mu"].data_ptr(), self._stream())
-
-    def state(self):
-        """This rank's block of the binary state: (i_raw (C, G, N_local), waner (C, N_local))."""
-        import torch
-
-        torch.cuda.synchronize(self.device)
-        return self.engine.download_state(self.C)
-
     def gather_individuals(self, local, axis=-1):
         """Concatenate per-rank blocks of individuals (NumPy arrays) along ``axis`` on every rank."""
-        import torch.distributed as dist
-
         parts = [None] * self.sh.world
         dist.all_gather_object(parts, np.ascontiguousarray(local), group=self.sh.group)
         return np.concatenate(parts, axis=axis)

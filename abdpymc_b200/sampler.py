@@ -13,11 +13,13 @@ e.g. ab_n_init against ab_n_perm), jittered trajectory length, step size by dual
 (Nesterov; Hoffman & Gelman 2014, the scheme PyMC's NUTS uses) and Stan-style windowed covariance
 adaptation pooled over the chains of the batch.  It is *not* NUTS: trajectory length is fixed up to
 jitter, which keeps all chains of a batch in lockstep (one kernel launch per leapfrog for all
-chains).  The binary block is updated by ``abd_gibbs_sweep`` (Metropolised flips with
-BinaryGibbsMetropolis semantics by default).
+chains).  ``SamplerConfig(kernel="nuts")`` runs batched No-U-Turn trees instead.  The binary block is
+updated by ``abd_gibbs_sweep`` (Metropolised flips with BinaryGibbsMetropolis semantics by default).
 
-The sampler is generic over a ``target`` (see ``AbdTarget``), so its host logic is tested on
-CPU against a Gaussian with known moments (tests/test_sampler.py).
+``sample`` is one loop (warm-up windows, recording, result) over one of two transitions: ``_DeviceLoop``
+for targets with the device-resident loop (``DeviceTarget``: ``AbdTarget``, ``distributed.ShardedTarget``),
+``_HostLoop`` (torch ops) for any target with ``logp_dlogp``.  So the host logic is tested on CPU against
+Gaussians with known moments (tests/test_host_logic.py).
 """
 
 from __future__ import annotations
@@ -25,6 +27,7 @@ from __future__ import annotations
 import time
 from collections import deque
 from dataclasses import dataclass, field
+from functools import cached_property
 
 import numpy as np
 import torch
@@ -32,58 +35,18 @@ import torch
 from .engine import Q17_RV, Q_OF_THETA, backward
 
 
-class DeviceNutsMixin:
-    """The No-U-Turn tree on the device (abd_nuts_*_dev) for a target with ``engine``, ``C``, ``seed``, ``device``
-    and ``_stream()``: one tree launch per leaf besides the leapfrog launch."""
+class DeviceTarget:
+    """A sampler target whose chain state (i_raw, waner) is resident on the GPU of ``engine``, for C chains: the
+    device-resident transitions (abd_hmc_*_dev, abd_nuts_*_dev), the Gibbs sweep and the streaming Deterministic means.
+    Subclasses add ``logp_dlogp_into`` and ``leapfrog_inplace``.  ``device_loop``: ``sample`` may run the loop that keeps
+    every transition on the device."""
 
-    def nuts_scratch(self, max_depth):
-        f64 = dict(dtype=torch.float64, device=self.device)
-        return (torch.zeros(self.C, self.engine.nuts_state_doubles(max_depth), **f64), torch.zeros(self.C, **f64),
-                torch.zeros(max_depth + 1, dtype=torch.int32, device=self.device))
+    device_loop = True
+    dim = 17
 
-    def nuts_begin(self, D, q, grad, logp, linv_t, eps, it, state, qw, pw, gw, eps_signed, any_active):
-        self.engine.nuts_begin_dev(self.C, D, q.data_ptr(), grad.data_ptr(), logp.data_ptr(), linv_t.data_ptr(), eps.data_ptr(),
-                                   self.seed, it, state.data_ptr(), qw.data_ptr(), pw.data_ptr(), gw.data_ptr(),
-                                   eps_signed.data_ptr(), any_active.data_ptr(), self._stream())
-
-    def nuts_leaf(self, D, j, n, qw, pw, gw, lpw, inv_mass, eps, it, state, eps_signed, any_active):
-        self.engine.nuts_leaf_dev(self.C, D, j, n, qw.data_ptr(), pw.data_ptr(), gw.data_ptr(), lpw.data_ptr(), inv_mass.data_ptr(),
-                                  eps.data_ptr(), self.seed, it, state.data_ptr(), eps_signed.data_ptr(), any_active.data_ptr(),
-                                  self._stream())
-
-    def nuts_extend(self, D, j, qw, pw, gw, lpw, inv_mass, eps, it, state, eps_signed, any_active):
-        """All 2^j leaves of one doubling (leapfrog + tree launch each) in one library call; targets whose leapfrog is
-        not ``abd_leapfrog_dev`` on their own engine (sharded cohorts) loop over ``leapfrog_inplace`` / ``nuts_leaf``."""
-        if getattr(self, "nuts_extend_in_library", False):
-            self.engine.nuts_extend_dev(self.C, D, j, qw.data_ptr(), pw.data_ptr(), gw.data_ptr(), lpw.data_ptr(), inv_mass.data_ptr(),
-                                        eps.data_ptr(), self.seed, it, state.data_ptr(), eps_signed.data_ptr(), any_active.data_ptr(),
-                                        self.d_i, self.d_w, self._stream())
-            return
-        for n in range(1 << j):
-            self.leapfrog_inplace(qw, pw, gw, lpw, eps_signed, inv_mass, 1)
-            self.nuts_leaf(D, j, n, qw, pw, gw, lpw, inv_mass, eps, it, state, eps_signed, any_active)
-
-    def nuts_end(self, D, q, grad, logp, state, acc, depth, div, da, eps, adapt, target_accept):
-        self.engine.nuts_end_dev(self.C, D, q.data_ptr(), grad.data_ptr(), logp.data_ptr(), state.data_ptr(), acc.data_ptr(),
-                                 depth.data_ptr(), div.data_ptr(), da.data_ptr(), eps.data_ptr(), adapt, target_accept,
-                                 self._stream())
-
-
-
-class AbdTarget(DeviceNutsMixin):
-    """The antibody-dynamics posterior on one GPU: joint logp + gradient over q17 for C chains
-    with the chain state (i_raw, waner) resident on the device, and the Gibbs sweep over it."""
-
-    nuts_extend_in_library = True
-
-    def __init__(self, engine, n_chains, i_raw, waner, seed=0, gibbs_mode=0, transit_p=0.8):
-        self.engine, self.C = engine, n_chains
-        self.device = torch.device("cuda", engine.device)
-        engine.upload_state(i_raw, waner)
-        self.out = torch.zeros(n_chains, dtype=torch.float64, device=self.device)
-        self.outg = torch.zeros(n_chains, 17, dtype=torch.float64, device=self.device)
+    def __init__(self, engine, n_chains, device, seed, gibbs_mode, transit_p):
+        self.engine, self.C, self.device = engine, n_chains, device
         self.seed, self.gibbs_mode, self.transit_p = seed, gibbs_mode, transit_p
-        self.dim = 17
 
     # the resident state's addresses are asked for on every use: the library reallocates the buffers when a
     # call with more chains than ever before arrives, and cached pointers would dangle silently
@@ -99,28 +62,10 @@ class AbdTarget(DeviceNutsMixin):
         return torch.cuda.current_stream(self.device).cuda_stream
 
     def logp_dlogp(self, q):
-        q = q.contiguous()
-        self.engine.logp_dlogp_dev(self.C, q.data_ptr(), self.d_i, self.d_w, self.out.data_ptr(), self.outg.data_ptr(),
-                                   self._stream())
-        return self.out.clone(), self.outg.clone()
-
-    def leapfrog(self, q, p, grad, eps, inv_mass, n_steps):
-        """n_steps leapfrog steps for all chains in one persistent launch (abd_leapfrog_dev).
-        Returns (q, p, logp, grad) at the end point; inputs are not modified."""
-        q, p, grad = q.clone().contiguous(), p.clone().contiguous(), grad.clone().contiguous()
-        eps, inv_mass = eps.contiguous(), inv_mass.contiguous()
-        lp = torch.empty(self.C, dtype=torch.float64, device=self.device)
-        self.engine.leapfrog_dev(self.C, n_steps, q.data_ptr(), p.data_ptr(), grad.data_ptr(), lp.data_ptr(),
-                                 eps.data_ptr(), inv_mass.data_ptr(), self.d_i, self.d_w, self._stream())
-        return q, p, lp, grad
-
-    # ---- fused transition (device-resident; no host synchronisation per iteration) -------------
-    def logp_dlogp_into(self, q, logp, grad):
-        self.engine.logp_dlogp_dev(self.C, q.data_ptr(), self.d_i, self.d_w, logp.data_ptr(), grad.data_ptr(), self._stream())
-
-    def leapfrog_inplace(self, q, p, grad, logp, eps, inv_mass, n_steps):
-        self.engine.leapfrog_dev(self.C, n_steps, q.data_ptr(), p.data_ptr(), grad.data_ptr(), logp.data_ptr(),
-                                 eps.data_ptr(), inv_mass.data_ptr(), self.d_i, self.d_w, self._stream())
+        logp = torch.empty(self.C, dtype=torch.float64, device=self.device)
+        grad = torch.empty(self.C, self.dim, dtype=torch.float64, device=self.device)
+        self.logp_dlogp_into(q.contiguous(), logp, grad)
+        return logp, grad
 
     def hmc_begin(self, q, grad, logp, linv_t, it, qw, pw, gw, h0):
         self.engine.hmc_begin_dev(self.C, q.data_ptr(), grad.data_ptr(), logp.data_ptr(), linv_t.data_ptr(), self.seed, it,
@@ -131,55 +76,33 @@ class AbdTarget(DeviceNutsMixin):
                                 gw.data_ptr(), lpw.data_ptr(), inv_mass.data_ptr(), h0.data_ptr(), self.seed, it,
                                 acc.data_ptr(), da.data_ptr(), eps.data_ptr(), adapt, target_accept, self._stream())
 
+    def nuts_scratch(self, max_depth):
+        f64 = dict(dtype=torch.float64, device=self.device)
+        return (torch.zeros(self.C, self.engine.nuts_state_doubles(max_depth), **f64), torch.zeros(self.C, **f64),
+                torch.zeros(max_depth + 1, dtype=torch.int32, device=self.device))
+
+    def nuts_begin(self, D, q, grad, logp, linv_t, eps, it, state, qw, pw, gw, eps_signed, any_active):
+        self.engine.nuts_begin_dev(self.C, D, q.data_ptr(), grad.data_ptr(), logp.data_ptr(), linv_t.data_ptr(), eps.data_ptr(),
+                                   self.seed, it, state.data_ptr(), qw.data_ptr(), pw.data_ptr(), gw.data_ptr(),
+                                   eps_signed.data_ptr(), any_active.data_ptr(), self._stream())
+
+    def nuts_extend(self, D, j, qw, pw, gw, lpw, inv_mass, eps, it, state, eps_signed, any_active):
+        """All 2^j leaves of one doubling (one leapfrog launch each, which also updates the trees) in one library call."""
+        self.engine.nuts_extend_dev(self.C, D, j, qw.data_ptr(), pw.data_ptr(), gw.data_ptr(), lpw.data_ptr(), inv_mass.data_ptr(),
+                                    eps.data_ptr(), self.seed, it, state.data_ptr(), eps_signed.data_ptr(), any_active.data_ptr(),
+                                    self.d_i, self.d_w, self._stream())
+
+    def nuts_end(self, D, q, grad, logp, state, acc, depth, div, da, eps, adapt, target_accept):
+        self.engine.nuts_end_dev(self.C, D, q.data_ptr(), grad.data_ptr(), logp.data_ptr(), state.data_ptr(), acc.data_ptr(),
+                                 depth.data_ptr(), div.data_ptr(), da.data_ptr(), eps.data_ptr(), adapt, target_accept,
+                                 self._stream())
+
     def gibbs(self, q, sweep):
+        """Sweep the binaries of every chain in place (on a sharded cohort: this rank's individuals, no collective --
+        RNG streams are keyed by global individual)."""
         q = q.contiguous()
         self.engine.gibbs_sweep_dev(self.C, q.data_ptr(), 1, None, None, self.d_i, self.d_w, self.seed, sweep,
                                     mode=self.gibbs_mode, transit_p=self.transit_p, stream=self._stream())
-
-    def check_status(self):
-        self.engine.leapfrog_status(self.C)
-
-    def fits_persistent(self):
-        """Whether a whole trajectory fits one resident grid (abd_leapfrog_dev): try one step."""
-        z = torch.zeros(self.C, 17, dtype=torch.float64, device=self.device)
-        one = torch.full((self.C,), 1e-9, dtype=torch.float64, device=self.device)
-        eye = torch.eye(17, dtype=torch.float64, device=self.device)
-        try:
-            self.leapfrog_inplace(z.clone(), z.clone(), z.clone(), one.clone(), one, eye, 1)
-            torch.cuda.synchronize(self.device)
-            return True
-        except Exception:
-            return False
-
-    def deterministics(self, q):
-        """(i, ab_n_mu, ab_s_mu) of the current state, device tensors (C, G, N).  No host round
-        trip: the back-transform of q runs on the device, the output buffers are reused."""
-        G, N, C = self.engine.G, self.engine.N, self.C
-        if not hasattr(self, "_det"):
-            kinds = torch.tensor([{None: 0, "log": 1, "logodds": 2}[Q17_RV[j][1]] for j in Q_OF_THETA], device=self.device)
-            self._det = (kinds, torch.tensor(Q_OF_THETA, device=self.device),
-                         torch.empty(C, G, N, dtype=torch.int8, device=self.device),
-                         torch.empty(C, G, N, dtype=torch.float64, device=self.device),
-                         torch.empty(C, G, N, dtype=torch.float64, device=self.device))
-        kinds, idx, oi, mn, ms = self._det
-        y = q.index_select(1, idx)
-        th = torch.where(kinds == 1, torch.exp(y), torch.where(kinds == 2, torch.sigmoid(y), y)).contiguous()
-        self.engine.deterministics_dev(C, th.data_ptr(), self.d_i, self.d_w, oi.data_ptr(), mn.data_ptr(), ms.data_ptr(),
-                                       self._stream())
-        return oi, mn, ms
-
-    def loglik_rows(self, q):
-        """Pointwise log-likelihood of the current state: (it_s_lik (C, R_s), it_n_lik (C, R_n)) device tensors."""
-        C, e = self.C, self.engine
-        if not hasattr(self, "_llr"):
-            self._llr = (torch.empty(C, e.R_s, dtype=torch.float64, device=self.device),
-                         torch.empty(C, e.R_n, dtype=torch.float64, device=self.device))
-        kinds = torch.tensor([{None: 0, "log": 1, "logodds": 2}[Q17_RV[j][1]] for j in Q_OF_THETA], device=self.device)
-        y = q.index_select(1, torch.tensor(Q_OF_THETA, device=self.device))
-        th = torch.where(kinds == 1, torch.exp(y), torch.where(kinds == 2, torch.sigmoid(y), y)).contiguous()
-        ls, ln = self._llr
-        e.loglik_rows_dev(C, th.data_ptr(), self.d_i, self.d_w, ls.data_ptr(), ln.data_ptr(), self._stream())
-        return ls, ln
 
     def accumulate_deterministics(self, q, sums):
         """Streaming posterior summaries: adds this state's i, ab_n_mu, ab_s_mu, summed over the chains,
@@ -194,8 +117,63 @@ class AbdTarget(DeviceNutsMixin):
                                              sums["ab_n_mu"].data_ptr(), sums["ab_s_mu"].data_ptr(), self._stream())
 
     def state(self):
+        """The binary state (i_raw (C, G, N), waner (C, N)); on a sharded cohort this rank's block of individuals."""
         torch.cuda.synchronize(self.device)
         return self.engine.download_state(self.C)
+
+    def check_status(self):
+        self.engine.leapfrog_status(self.C)
+
+
+class AbdTarget(DeviceTarget):
+    """The antibody-dynamics posterior on one GPU: joint logp + gradient over q17 for C chains
+    with the chain state (i_raw, waner) resident on the device, and the Gibbs sweep over it."""
+
+    def __init__(self, engine, n_chains, i_raw, waner, seed=0, gibbs_mode=0, transit_p=0.8):
+        super().__init__(engine, n_chains, torch.device("cuda", engine.device), seed, gibbs_mode, transit_p)
+        engine.upload_state(i_raw, waner)
+
+    def logp_dlogp_into(self, q, logp, grad):
+        self.engine.logp_dlogp_dev(self.C, q.data_ptr(), self.d_i, self.d_w, logp.data_ptr(), grad.data_ptr(), self._stream())
+
+    def leapfrog_inplace(self, q, p, grad, logp, eps, inv_mass, n_steps):
+        self.engine.leapfrog_dev(self.C, n_steps, q.data_ptr(), p.data_ptr(), grad.data_ptr(), logp.data_ptr(),
+                                 eps.data_ptr(), inv_mass.data_ptr(), self.d_i, self.d_w, self._stream())
+
+    @cached_property
+    def _theta_of_q(self):   # per component of theta13: its back-transform (0 none, 1 exp, 2 sigmoid) and its column of q
+        kinds = torch.tensor([{None: 0, "log": 1, "logodds": 2}[Q17_RV[j][1]] for j in Q_OF_THETA], device=self.device)
+        return kinds, torch.tensor(Q_OF_THETA, device=self.device)
+
+    def _theta13(self, q):
+        kinds, idx = self._theta_of_q
+        y = q.index_select(1, idx)
+        return torch.where(kinds == 1, torch.exp(y), torch.where(kinds == 2, torch.sigmoid(y), y)).contiguous()
+
+    def deterministics(self, q):
+        """(i, ab_n_mu, ab_s_mu) of the current state, device tensors (C, G, N).  No host round
+        trip: the back-transform of q runs on the device, the output buffers are reused."""
+        G, N, C = self.engine.G, self.engine.N, self.C
+        if not hasattr(self, "_det"):
+            self._det = (torch.empty(C, G, N, dtype=torch.int8, device=self.device),
+                         torch.empty(C, G, N, dtype=torch.float64, device=self.device),
+                         torch.empty(C, G, N, dtype=torch.float64, device=self.device))
+        oi, mn, ms = self._det
+        th = self._theta13(q)
+        self.engine.deterministics_dev(C, th.data_ptr(), self.d_i, self.d_w, oi.data_ptr(), mn.data_ptr(), ms.data_ptr(),
+                                       self._stream())
+        return oi, mn, ms
+
+    def loglik_rows(self, q):
+        """Pointwise log-likelihood of the current state: (it_s_lik (C, R_s), it_n_lik (C, R_n)) device tensors."""
+        C, e = self.C, self.engine
+        if not hasattr(self, "_llr"):
+            self._llr = (torch.empty(C, e.R_s, dtype=torch.float64, device=self.device),
+                         torch.empty(C, e.R_n, dtype=torch.float64, device=self.device))
+        ls, ln = self._llr
+        th = self._theta13(q)
+        e.loglik_rows_dev(C, th.data_ptr(), self.d_i, self.d_w, ls.data_ptr(), ln.data_ptr(), self._stream())
+        return ls, ln
 
 
 @dataclass
@@ -210,10 +188,12 @@ class SamplerConfig:
     record_deterministics_every: int = 0   # 0 = never; k = accumulate means every k-th draw
     thinned_deterministics: int = 0        # keep this many evenly spaced draws of i / ab_n_mu / ab_s_mu per chain (the
                                            # consumers use <= 250: survival.py:109-114, timelines.py:289-301); 0 = none
-    persistent_trajectories: bool = True   # leapfrog integration inside the library (abd_leapfrog_dev) when it fits
-    single_step_launches: bool = True      # ... as one launch per step rather than one persistent launch per trajectory
+    persistent_trajectories: bool = True   # run the whole transition on the device when the target can (``device_loop``);
+                                           # False: torch ops driven from the host on any target
+    single_step_launches: bool = True      # device HMC: one abd_leapfrog_dev launch per step rather than one persistent
+                                           # launch per trajectory
     seed: int = 0
-    kernel: str = "hmc"                    # "hmc": jittered fixed-length trajectories (the fused device loop when it fits);
+    kernel: str = "hmc"                    # "hmc": jittered fixed-length trajectories;
                                            # "nuts": batched multinomial No-U-Turn trajectories (what pm.sample runs for
                                            # the 17 scalars, abd.py:922), chains doubling in lockstep; tree bookkeeping on
                                            # the device when the target offers it (abd_nuts_*_dev), else torch ops
@@ -235,7 +215,7 @@ class SamplerResult:
     means: dict = field(default_factory=dict)   # posterior means of i, ab_n_mu, ab_s_mu (G, N)
     thinned: dict = field(default_factory=dict)  # i (int8), ab_n_mu, ab_s_mu (float32): (chains, kept draws, G, N); "draw" = their indexes
     stats: dict = field(default_factory=dict)   # NUTS: tree_depth, diverging (chains, draws); what PyMC puts in sample_stats
-    wall_tune_s: float = 0.0           # device-resident drivers: the part of wall_s spent in the tuning iterations ...
+    wall_tune_s: float = 0.0           # the part of wall_s spent in the tuning iterations ...
     n_grad_evals_tune: int = 0         # ... and the gradient evaluations they took
 
     def posterior(self):
@@ -325,130 +305,6 @@ class _Thinned:
         if self.with_ll:
             out["it_s_lik"], out["it_n_lik"] = self.ls.permute(1, 0, 2).cpu().numpy(), self.ln.permute(1, 0, 2).cpu().numpy()
         return out
-
-
-def _sample_fused(target, q0, cfg, progress, nuts=False):
-    """The same iteration as ``sample`` with the whole transition on the device: abd_hmc_begin_dev,
-    abd_leapfrog_dev (one launch per step, or one persistent launch), abd_hmc_end_dev,
-    abd_gibbs_sweep_dev, abd_logp_dlogp_dev, no host synchronisation; the host only picks the trajectory length and,
-    at the end of a warm-up window, re-estimates the metric."""
-    dev = q0.device
-    C, D = q0.shape
-    f64 = dict(dtype=torch.float64, device=dev)
-    rng = np.random.default_rng(cfg.seed)
-    q = q0.clone().to(torch.float64).contiguous()
-    logp, grad = torch.empty(C, **f64), torch.empty(C, D, **f64)
-    target.logp_dlogp_into(q, logp, grad)
-    inv_mass = torch.eye(D, **f64)
-    linv_t = torch.eye(D, **f64)        # (chol^T)^-1 with inv_mass = chol chol^T
-    eps = torch.full((C,), cfg.init_step, **f64)
-    da = torch.zeros(C, 4, **f64)       # mu, hbar, log_avg, t
-    da[:, 0] = torch.log(10.0 * eps)
-    qw, pw, gw = torch.empty(C, D, **f64), torch.empty(C, D, **f64), torch.empty(C, D, **f64)
-    lpw, h0, acc = torch.empty(C, **f64), torch.empty(C, **f64), torch.empty(C, **f64)
-    ends = _windows(cfg.tune)
-    win_start = 75 if cfg.tune >= 150 else 0
-    win_draws = []
-    total = cfg.tune + cfg.draws
-    out_q = torch.empty(cfg.draws, C, D, **f64)
-    out_lp, out_acc = torch.empty(cfg.draws, C, **f64), torch.empty(cfg.draws, C, **f64)
-    means, n_means, n_grad = {}, 0, 0
-    thin = _Thinned(target, cfg)
-    if nuts:
-        TD = int(min(max(cfg.max_treedepth, 1), 10))   # maximum tree depth
-        nstate, eps_signed, any_active = target.nuts_scratch(TD)
-        depth_d, div_d = torch.zeros(C, **f64), torch.zeros(C, **f64)
-        out_depth, out_div = torch.zeros(cfg.draws, C, **f64), torch.zeros(cfg.draws, C, **f64)
-        recent_depths = deque(maxlen=32)
-    t0 = time.perf_counter()
-    wall_tune, n_grad_tune = 0.0, 0
-    for it in range(total):
-        if nuts:
-            # the chains double in lockstep: depth j adds 2^j leaves (one leapfrog launch + one tree launch each);
-            # one word is read back per depth: does any chain still want to double?
-            target.nuts_begin(TD, q, grad, logp, linv_t, eps, it, nstate, qw, pw, gw, eps_signed, any_active)
-            # Depths below `check_from` are built without asking (a read-back costs as much as two leaves): the shallowest
-            # tree of the last 32 iterations, never below cfg.nuts_check_from_depth.  Building a depth no chain wanted
-            # changes nothing (its leaves are masked on the device), it only costs their launches.
-            check_from = max(cfg.nuts_check_from_depth, min(recent_depths)) if cfg.nuts_adaptive_checks and recent_depths \
-                else cfg.nuts_check_from_depth
-            flags = None
-            for j in range(TD):
-                target.nuts_extend(TD, j, qw, pw, gw, lpw, inv_mass, eps, it, nstate, eps_signed, any_active)
-                n_grad += 1 << j
-                if j + 1 < TD and j + 1 >= check_from:
-                    flags = any_active.tolist()       # [k]: did any chain want depth k?  (one read-back, all depths)
-                    if flags[j + 1] == 0:
-                        break
-            # lockstep depth of this tree: the first depth nobody wanted
-            recent_depths.append(TD if flags is None else next((k for k in range(1, TD + 1) if flags[k] == 0), TD))
-            target.nuts_end(TD, q, grad, logp, nstate, acc, depth_d, div_d, da, eps, it < cfg.tune, cfg.target_accept)
-            L = 0
-        else:
-            L = max(1, int(round(cfg.n_leapfrog * (cfg.jitter[0] + (cfg.jitter[1] - cfg.jitter[0]) * rng.random()))))
-            target.hmc_begin(q, grad, logp, linv_t, it, qw, pw, gw, h0)
-            if cfg.single_step_launches:   # L overlapped launches: 14.7 us per step (one persistent launch: 16.8)
-                for _ in range(L):
-                    target.leapfrog_inplace(qw, pw, gw, lpw, eps, inv_mass, 1)
-            else:
-                target.leapfrog_inplace(qw, pw, gw, lpw, eps, inv_mass, L)
-            target.hmc_end(q, grad, logp, qw, pw, gw, lpw, inv_mass, h0, it, acc, da, eps, it < cfg.tune, cfg.target_accept)
-        target.gibbs(q, it)
-        target.logp_dlogp_into(q, logp, grad)
-        n_grad += L + 1
-        if it < cfg.tune:
-            if ends and win_start <= it:
-                win_draws.append(q.clone())
-            if ends and it + 1 == ends[0]:
-                # 17 x 17 linear algebra on the host (a handful of times per run; the first cuSOLVER
-                # call alone would cost more than all of them)
-                x = torch.stack(win_draws).reshape(-1, D).cpu().numpy()
-                n = x.shape[0]
-                cov = np.cov(x.T)
-                im = (n / (n + 5.0)) * cov + 1e-3 * (5.0 / (n + 5.0)) * np.eye(D)  # Stan's shrinkage keeps it positive definite
-                chol = np.linalg.cholesky(im)
-                inv_mass = torch.from_numpy(np.ascontiguousarray(im)).to(dev)
-                linv_t = torch.from_numpy(np.ascontiguousarray(np.linalg.inv(chol.T))).to(dev)
-                win_draws, win_start = [], ends.pop(0)
-                # restart step-size adaptation under the new metric from the averaged step
-                eps = torch.exp(da[:, 2]).contiguous()
-                da.zero_()
-                da[:, 0] = torch.log(10.0 * eps)
-            if it + 1 == cfg.tune:
-                eps = torch.where(da[:, 3] > 0, torch.exp(da[:, 2]), eps).contiguous()
-                torch.cuda.synchronize(dev)     # once per run: the draws are timed on their own as well
-                wall_tune, n_grad_tune = time.perf_counter() - t0, n_grad
-        else:
-            k = it - cfg.tune
-            out_q[k].copy_(q)
-            out_lp[k].copy_(logp)
-            out_acc[k].copy_(acc)
-            if nuts:
-                out_depth[k].copy_(depth_d)
-                out_div[k].copy_(div_d)
-            thin.record(target, k, q)
-            every = cfg.record_deterministics_every
-            if every and k % every == 0:
-                if hasattr(target, "accumulate_deterministics"):
-                    target.accumulate_deterministics(q, means)   # sums over chains; divided once at the end
-                    n_means += C
-                elif hasattr(target, "deterministics"):
-                    oi, mn, ms = target.deterministics(q)
-                    for name, v in (("i", oi.to(torch.float64)), ("ab_n_mu", mn), ("ab_s_mu", ms)):
-                        means[name] = v.sum(dim=0) if name not in means else means[name] + v.sum(dim=0)
-                    n_means += C
-        if progress and (it + 1) % progress == 0:
-            print(f"  iter {it + 1}/{total}  step {eps.mean().item():.4f}  accept {acc.mean().item():.2f}", flush=True)
-    torch.cuda.synchronize(dev)
-    target.check_status()
-    wall = time.perf_counter() - t0
-    stats = {"tree_depth": out_depth.T.cpu().numpy().astype(np.int64), "diverging": out_div.T.cpu().numpy() != 0} if nuts else {}
-    return SamplerResult(
-        q=out_q.permute(1, 0, 2).cpu().numpy(), logp=out_lp.T.cpu().numpy(), accept=out_acc.T.cpu().numpy(),
-        step_size=eps.cpu().numpy(), inv_mass=inv_mass.cpu().numpy(), wall_s=wall, n_grad_evals=n_grad,
-        means={k: (v / n_means).cpu().numpy() for k, v in means.items()}, thinned=thin.result(), stats=stats,
-        wall_tune_s=wall_tune, n_grad_evals_tune=n_grad_tune,
-    )
 
 
 def _nuts_transition(target, q, logp, grad, eps, inv_mass, chol, gen, max_depth):
@@ -546,118 +402,226 @@ def _nuts_transition(target, q, logp, grad, eps, inv_mass, chol, gen, max_depth)
     return q_prop, lp_prop, g_prop, sum_acc / torch.clamp(n_acc, min=1.0), depth, diverged, n_leaves
 
 
+class _HostLoop:
+    """The transition as torch ops driven from the host, for any target with ``logp_dlogp(q) -> (logp, grad)``: momenta,
+    trajectory jitter and accept decisions from one torch.Generator, step size by ``_DualAveraging``, the metric by
+    torch.linalg."""
+
+    def __init__(self, target, q0, cfg):
+        dev, (C, D) = q0.device, q0.shape
+        self.target, self.cfg, self.nuts = target, cfg, cfg.kernel == "nuts"
+        self.gen = torch.Generator(device=dev)
+        self.gen.manual_seed(cfg.seed)
+        self.q = q0.clone().to(torch.float64)
+        self.logp, self.grad = target.logp_dlogp(self.q)
+        self.inv_mass = torch.eye(D, dtype=torch.float64, device=dev)   # Sigma = M^-1 (dense)
+        self.chol = torch.eye(D, dtype=torch.float64, device=dev)       # Sigma = chol chol^T
+        self.eps = torch.full((C,), cfg.init_step, dtype=torch.float64, device=dev)
+        self.da = _DualAveraging(self.eps, cfg.target_accept, dev)
+
+    def transition(self, it):
+        """Moves q given the binaries; returns the number of gradient evaluations."""
+        cfg, q, logp, grad, eps, inv_mass, gen = self.cfg, self.q, self.logp, self.grad, self.eps, self.inv_mass, self.gen
+        if self.nuts:   # ---- NUTS over q given the binaries (abd.py:922 runs PyMC's) ----
+            q, logp, grad, self.acc, self.depth, self.div, n_grad = _nuts_transition(self.target, q, logp, grad, eps, inv_mass,
+                                                                                     self.chol, gen, cfg.max_treedepth)
+        else:           # ---- HMC over q given the binaries ----
+            C, D = q.shape
+            # p ~ N(0, M) with M = Sigma^-1:  p = chol^-T z
+            z = torch.randn(C, D, dtype=torch.float64, device=q.device, generator=gen)
+            p = torch.linalg.solve_triangular(self.chol.T, z.T, upper=True).T
+            h0 = -logp + 0.5 * (z * z).sum(dim=1)
+            jitter = cfg.jitter[0] + (cfg.jitter[1] - cfg.jitter[0]) * torch.rand((), device=q.device, generator=gen).item()
+            n_grad = L = max(1, int(round(cfg.n_leapfrog * jitter)))
+            qn, pn, gn, lpn = q, p, grad, logp
+            e = eps[:, None]
+            for _ in range(L):
+                pn = pn + 0.5 * e * gn
+                qn = qn + e * (pn @ inv_mass)
+                lpn, gn = self.target.logp_dlogp(qn)
+                pn = pn + 0.5 * e * gn
+            h1 = -lpn + 0.5 * ((pn @ inv_mass) * pn).sum(dim=1)
+            dh = h0 - h1
+            dh = torch.where(torch.isfinite(dh), dh, torch.full_like(dh, -float("inf")))
+            self.acc = torch.exp(torch.clamp(dh, max=0.0))
+            take = torch.rand(C, dtype=torch.float64, device=q.device, generator=gen) < self.acc
+            q, grad, logp = torch.where(take[:, None], qn, q), torch.where(take[:, None], gn, grad), torch.where(take, lpn, logp)
+        self.q, self.logp, self.grad = q, logp, grad
+        if it < cfg.tune:
+            self.eps = self.da.update(self.acc)
+        return n_grad
+
+    def refresh(self):
+        self.logp, self.grad = self.target.logp_dlogp(self.q)
+
+    def set_metric(self, x):
+        n, D = x.shape
+        cov = torch.cov(x.T)
+        self.inv_mass = (n / (n + 5.0)) * cov + 1e-3 * (5.0 / (n + 5.0)) * torch.eye(D, dtype=cov.dtype, device=x.device)
+        self.chol = torch.linalg.cholesky(self.inv_mass)  # Stan's shrinkage keeps it positive definite
+        self.eps = self.da.final()  # restart step-size adaptation under the new metric
+        self.da = _DualAveraging(self.eps, self.cfg.target_accept, x.device)
+
+    def end_tuning(self):
+        if self.da.t:
+            self.eps = self.da.final()
+
+
+class _DeviceLoop:
+    """The transition on the device, no host synchronisation: abd_hmc_begin_dev, abd_leapfrog_dev (one launch per step, or
+    one persistent launch per trajectory), abd_hmc_end_dev -- or abd_nuts_begin_dev, one abd_nuts_extend_dev per tree
+    depth, abd_nuts_end_dev -- with the momenta, accept decisions and dual averaging in the kernels.  The host only picks
+    the trajectory length and, at the end of a warm-up window, computes the metric."""
+
+    def __init__(self, target, q0, cfg):
+        dev, (C, D) = q0.device, q0.shape
+        f64 = dict(dtype=torch.float64, device=dev)
+        self.target, self.cfg, self.nuts = target, cfg, cfg.kernel == "nuts"
+        self.rng = np.random.default_rng(cfg.seed)
+        self.q = q0.clone().to(torch.float64).contiguous()
+        self.logp, self.grad = torch.empty(C, **f64), torch.empty(C, D, **f64)
+        target.logp_dlogp_into(self.q, self.logp, self.grad)
+        self.inv_mass = torch.eye(D, **f64)
+        self.linv_t = torch.eye(D, **f64)        # (chol^T)^-1 with inv_mass = chol chol^T
+        self.eps = torch.full((C,), cfg.init_step, **f64)
+        self.da = torch.zeros(C, 4, **f64)       # mu, hbar, log_avg, t
+        self.da[:, 0] = torch.log(10.0 * self.eps)
+        self.qw, self.pw, self.gw = torch.empty(C, D, **f64), torch.empty(C, D, **f64), torch.empty(C, D, **f64)
+        self.lpw, self.h0, self.acc = torch.empty(C, **f64), torch.empty(C, **f64), torch.empty(C, **f64)
+        if self.nuts:
+            self.TD = int(min(max(cfg.max_treedepth, 1), 10))   # maximum tree depth
+            self.tree, self.eps_signed, self.any_active = target.nuts_scratch(self.TD)
+            self.depth, self.div = torch.zeros(C, **f64), torch.zeros(C, **f64)
+            self.recent_depths = deque(maxlen=32)
+
+    def transition(self, it):
+        """Moves q given the binaries; returns the number of gradient evaluations."""
+        tgt, cfg, adapt = self.target, self.cfg, it < self.cfg.tune
+        q, grad, logp, eps, qw, pw, gw, lpw = self.q, self.grad, self.logp, self.eps, self.qw, self.pw, self.gw, self.lpw
+        if not self.nuts:
+            L = max(1, int(round(cfg.n_leapfrog * (cfg.jitter[0] + (cfg.jitter[1] - cfg.jitter[0]) * self.rng.random()))))
+            tgt.hmc_begin(q, grad, logp, self.linv_t, it, qw, pw, gw, self.h0)
+            if cfg.single_step_launches:   # L overlapped launches: 14.7 us per step (one persistent launch: 16.8)
+                for _ in range(L):
+                    tgt.leapfrog_inplace(qw, pw, gw, lpw, eps, self.inv_mass, 1)
+            else:
+                tgt.leapfrog_inplace(qw, pw, gw, lpw, eps, self.inv_mass, L)
+            tgt.hmc_end(q, grad, logp, qw, pw, gw, lpw, self.inv_mass, self.h0, it, self.acc, self.da, eps, adapt,
+                        cfg.target_accept)
+            return L
+        # the chains double in lockstep: depth j adds 2^j leaves (one leapfrog launch each, which also updates the trees);
+        # one word is read back per depth: does any chain still want to double?
+        TD, tree, eps_signed, any_active = self.TD, self.tree, self.eps_signed, self.any_active
+        tgt.nuts_begin(TD, q, grad, logp, self.linv_t, eps, it, tree, qw, pw, gw, eps_signed, any_active)
+        # Depths below `check_from` are built without asking (a read-back costs as much as two leaves): the shallowest
+        # tree of the last 32 iterations, never below cfg.nuts_check_from_depth.  Building a depth no chain wanted
+        # changes nothing (its leaves are masked on the device), it only costs their launches.
+        recent = self.recent_depths
+        check_from = max(cfg.nuts_check_from_depth, min(recent)) if cfg.nuts_adaptive_checks and recent \
+            else cfg.nuts_check_from_depth
+        flags, n_grad = None, 0
+        for j in range(TD):
+            tgt.nuts_extend(TD, j, qw, pw, gw, lpw, self.inv_mass, eps, it, tree, eps_signed, any_active)
+            n_grad += 1 << j
+            if j + 1 < TD and j + 1 >= check_from:
+                flags = any_active.tolist()       # [k]: did any chain want depth k?  (one read-back, all depths)
+                if flags[j + 1] == 0:
+                    break
+        # lockstep depth of this tree: the first depth nobody wanted
+        recent.append(TD if flags is None else next((k for k in range(1, TD + 1) if flags[k] == 0), TD))
+        tgt.nuts_end(TD, q, grad, logp, tree, self.acc, self.depth, self.div, self.da, eps, adapt, cfg.target_accept)
+        return n_grad
+
+    def refresh(self):
+        self.target.logp_dlogp_into(self.q, self.logp, self.grad)
+
+    def set_metric(self, x):
+        # 17 x 17 linear algebra on the host (a handful of times per run; the first cuSOLVER
+        # call alone would cost more than all of them)
+        x = x.cpu().numpy()
+        n, D = x.shape
+        cov = np.cov(x.T)
+        im = (n / (n + 5.0)) * cov + 1e-3 * (5.0 / (n + 5.0)) * np.eye(D)  # Stan's shrinkage keeps it positive definite
+        chol = np.linalg.cholesky(im)
+        dev = self.q.device
+        self.inv_mass = torch.from_numpy(np.ascontiguousarray(im)).to(dev)
+        self.linv_t = torch.from_numpy(np.ascontiguousarray(np.linalg.inv(chol.T))).to(dev)
+        # restart step-size adaptation under the new metric from the averaged step
+        self.eps = torch.exp(self.da[:, 2]).contiguous()
+        self.da.zero_()
+        self.da[:, 0] = torch.log(10.0 * self.eps)
+
+    def end_tuning(self):
+        self.eps = torch.where(self.da[:, 3] > 0, torch.exp(self.da[:, 2]), self.eps).contiguous()
+
+
 def sample(target, q0, cfg: SamplerConfig = SamplerConfig(), progress=None) -> SamplerResult:
-    """Run tune + draws iterations of [HMC on q | binaries] then [Gibbs on binaries | q]."""
-    if cfg.kernel == "hmc" and cfg.persistent_trajectories and hasattr(target, "hmc_begin") and target.fits_persistent():
-        return _sample_fused(target, q0, cfg, progress)
-    if (cfg.kernel == "nuts" and cfg.persistent_trajectories and getattr(target, "nuts_begin", None) is not None
-            and target.fits_persistent()):
-        return _sample_fused(target, q0, cfg, progress, nuts=True)
+    """Run tune + draws iterations of [HMC or NUTS on q | binaries] then [Gibbs on binaries | q].  The transitions run on
+    the device when the target has the device-resident loop (``device_loop``) and ``cfg.persistent_trajectories`` is set,
+    otherwise as torch ops driven from the host."""
+    if cfg.kernel not in ("hmc", "nuts"):
+        raise ValueError(f"unknown kernel {cfg.kernel!r}: 'hmc' or 'nuts'")
+    on_device = cfg.persistent_trajectories and getattr(target, "device_loop", False)
+    run = (_DeviceLoop if on_device else _HostLoop)(target, q0, cfg)
     dev = q0.device
     C, D = q0.shape
-    gen = torch.Generator(device=dev)
-    gen.manual_seed(cfg.seed)
-    q = q0.clone().to(torch.float64)
-    logp, grad = target.logp_dlogp(q)
-    inv_mass = torch.eye(D, dtype=torch.float64, device=dev)   # Sigma = M^-1 (dense)
-    chol = torch.eye(D, dtype=torch.float64, device=dev)       # Sigma = chol chol^T
-    eps = torch.full((C,), cfg.init_step, dtype=torch.float64, device=dev)
-    da = _DualAveraging(eps, cfg.target_accept, dev)
+    f64 = dict(dtype=torch.float64, device=dev)
+
+    def sync():
+        if dev.type == "cuda":
+            torch.cuda.synchronize(dev)
+
     ends = _windows(cfg.tune)
     win_start = 75 if cfg.tune >= 150 else 0
     win_draws = []
     total = cfg.tune + cfg.draws
-    out_q = torch.empty(cfg.draws, C, D, dtype=torch.float64, device=dev)
-    out_lp = torch.empty(cfg.draws, C, dtype=torch.float64, device=dev)
-    out_acc = torch.empty(cfg.draws, C, dtype=torch.float64, device=dev)
-    out_depth = torch.zeros(cfg.draws, C, dtype=torch.long, device=dev)
-    out_div = torch.zeros(cfg.draws, C, dtype=torch.bool, device=dev)
+    out_q = torch.empty(cfg.draws, C, D, **f64)
+    out_lp, out_acc = torch.empty(cfg.draws, C, **f64), torch.empty(cfg.draws, C, **f64)
+    out_depth, out_div = torch.zeros(cfg.draws, C, **f64), torch.zeros(cfg.draws, C, **f64)   # NUTS tree statistics
     means, n_means, n_grad = {}, 0, 0
     thin = _Thinned(target, cfg)
     has_gibbs = hasattr(target, "gibbs")
-    use_traj = hasattr(target, "leapfrog") and cfg.persistent_trajectories
     t0 = time.perf_counter()
+    wall_tune, n_grad_tune = 0.0, 0
     for it in range(total):
-        if cfg.kernel == "nuts":
-            # ---- NUTS over q given the binaries (abd.py:922 runs PyMC's) ------------------------
-            q, logp, grad, acc_p, tree_depth, tree_div, n_leaf = _nuts_transition(target, q, logp, grad, eps, inv_mass, chol, gen,
-                                                                                  cfg.max_treedepth)
-            n_grad += n_leaf
-        else:
-            # ---- HMC over q given the binaries ---------------------------------------------
-            # p ~ N(0, M) with M = Sigma^-1:  p = chol^-T z
-            z = torch.randn(C, D, dtype=torch.float64, device=dev, generator=gen)
-            p = torch.linalg.solve_triangular(chol.T, z.T, upper=True).T
-            h0 = -logp + 0.5 * (z * z).sum(dim=1)
-            jitter = cfg.jitter[0] + (cfg.jitter[1] - cfg.jitter[0]) * torch.rand((), device=dev, generator=gen).item()
-            L = max(1, int(round(cfg.n_leapfrog * jitter)))
-            if use_traj:
-                try:
-                    qn, pn, lpn, gn = target.leapfrog(q, p, grad, eps, inv_mass, L)
-                except Exception:  # too many chains for one resident grid: per-step launches
-                    use_traj = False
-            if not use_traj:
-                qn, pn, gn, lpn = q, p, grad, logp
-                e = eps[:, None]
-                for _ in range(L):
-                    pn = pn + 0.5 * e * gn
-                    qn = qn + e * (pn @ inv_mass)
-                    lpn, gn = target.logp_dlogp(qn)
-                    pn = pn + 0.5 * e * gn
-            n_grad += L
-            h1 = -lpn + 0.5 * ((pn @ inv_mass) * pn).sum(dim=1)
-            dh = h0 - h1
-            dh = torch.where(torch.isfinite(dh), dh, torch.full_like(dh, -float("inf")))
-            acc_p = torch.exp(torch.clamp(dh, max=0.0))
-            take = torch.rand(C, dtype=torch.float64, device=dev, generator=gen) < acc_p
-            q = torch.where(take[:, None], qn, q)
-            grad = torch.where(take[:, None], gn, grad)
-            logp = torch.where(take, lpn, logp)
-        # ---- Gibbs over the binaries given q (then logp / grad at the new state) -------------
-        if has_gibbs:
-            target.gibbs(q, it)
-            logp, grad = target.logp_dlogp(q)
+        n_grad += run.transition(it)
+        if has_gibbs:   # Gibbs over the binaries given q, then logp / grad at the new state
+            target.gibbs(run.q, it)
+            run.refresh()
             n_grad += 1
-        # ---- adaptation / recording -----------------------------------------------------------
         if it < cfg.tune:
-            eps = da.update(acc_p)
             if ends and win_start <= it:
-                win_draws.append(q.clone())
+                win_draws.append(run.q.clone())
             if ends and it + 1 == ends[0]:
-                x = torch.stack(win_draws).reshape(-1, D)
-                n = x.shape[0]
-                cov = torch.cov(x.T)
-                inv_mass = (n / (n + 5.0)) * cov + 1e-3 * (5.0 / (n + 5.0)) * torch.eye(D, dtype=cov.dtype, device=dev)
-                chol = torch.linalg.cholesky(inv_mass)  # Stan's shrinkage keeps it positive definite
+                run.set_metric(torch.stack(win_draws).reshape(-1, D))
                 win_draws, win_start = [], ends.pop(0)
-                eps = da.final()  # restart step-size adaptation under the new metric
-                da = _DualAveraging(eps, cfg.target_accept, dev)
-            if it + 1 == cfg.tune and da.t:
-                eps = da.final()
+            if it + 1 == cfg.tune:
+                run.end_tuning()
+                sync()     # once per run: the draws are timed on their own as well
+                wall_tune, n_grad_tune = time.perf_counter() - t0, n_grad
         else:
             k = it - cfg.tune
-            out_q[k], out_lp[k], out_acc[k] = q, logp, acc_p
-            if cfg.kernel == "nuts":
-                out_depth[k], out_div[k] = tree_depth, tree_div
-            thin.record(target, k, q)
+            out_q[k].copy_(run.q)
+            out_lp[k].copy_(run.logp)
+            out_acc[k].copy_(run.acc)
+            if run.nuts:
+                out_depth[k].copy_(run.depth)
+                out_div[k].copy_(run.div)
+            thin.record(target, k, run.q)
             every = cfg.record_deterministics_every
-            if every and k % every == 0:
-                if hasattr(target, "accumulate_deterministics"):
-                    target.accumulate_deterministics(q, means)   # sums over chains; divided once at the end
-                    n_means += C
-                elif hasattr(target, "deterministics"):
-                    oi, mn, ms = target.deterministics(q)
-                    for name, v in (("i", oi.to(torch.float64)), ("ab_n_mu", mn), ("ab_s_mu", ms)):
-                        means[name] = v.sum(dim=0) if name not in means else means[name] + v.sum(dim=0)
-                    n_means += C
+            if every and k % every == 0 and hasattr(target, "accumulate_deterministics"):
+                target.accumulate_deterministics(run.q, means)   # sums over chains; divided once at the end
+                n_means += C
         if progress and (it + 1) % progress == 0:
-            print(f"  iter {it + 1}/{total}  step {eps.mean().item():.4f}  accept {acc_p.mean().item():.2f}", flush=True)
-    if dev.type == "cuda":
-        torch.cuda.synchronize(dev)
+            print(f"  iter {it + 1}/{total}  step {run.eps.mean().item():.4f}  accept {run.acc.mean().item():.2f}", flush=True)
+    sync()
+    if on_device:
+        target.check_status()
     wall = time.perf_counter() - t0
-    stats = {"tree_depth": out_depth.T.cpu().numpy(), "diverging": out_div.T.cpu().numpy()} if cfg.kernel == "nuts" else {}
+    stats = {"tree_depth": out_depth.T.cpu().numpy().astype(np.int64), "diverging": out_div.T.cpu().numpy() != 0} if run.nuts else {}
     return SamplerResult(
         q=out_q.permute(1, 0, 2).cpu().numpy(), logp=out_lp.T.cpu().numpy(), accept=out_acc.T.cpu().numpy(),
-        step_size=eps.cpu().numpy(), inv_mass=inv_mass.cpu().numpy(), wall_s=wall, n_grad_evals=n_grad,
+        step_size=run.eps.cpu().numpy(), inv_mass=run.inv_mass.cpu().numpy(), wall_s=wall, n_grad_evals=n_grad,
         means={k: (v / n_means).cpu().numpy() for k, v in means.items()}, thinned=thin.result(), stats=stats,
+        wall_tune_s=wall_tune, n_grad_evals_tune=n_grad_tune,
     )
