@@ -76,6 +76,7 @@ SIGNATURES = {
                                       C.c_uint64, C.c_uint64, C.c_int, C.c_double, C.c_void_p, C.c_void_p]),
     "abd_deterministics_dev": (C.c_int, [H, C.c_int] + [C.c_void_p] * 7),
     "abd_deterministics_accum_dev": (C.c_int, [H, C.c_int, C.c_void_p, C.c_int] + [C.c_void_p] * 6),
+    "abd_infection_probs_accum_dev": (C.c_int, [H, C.c_int] + [C.c_void_p] * 6),
     "abd_leapfrog_dev": (C.c_int, [H, C.c_int, C.c_int] + [C.c_void_p] * 9),
     "abd_leapfrog_status": (C.c_int, [H, C.c_int]),
     "abd_hmc_begin_dev": (C.c_int, [H, C.c_int] + [C.c_void_p] * 4 + [C.c_uint64, C.c_uint64] + [C.c_void_p] * 5),

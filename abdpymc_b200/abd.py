@@ -349,13 +349,44 @@ def pointwise_log_likelihood(engine, posterior, batch=64):
     return {"it_s_lik": ls.reshape(n_c, n_d, -1), "it_n_lik": ln.reshape(n_c, n_d, -1)}
 
 
+def infection_probabilities(engine, posterior, batch=64):
+    """Rao-Blackwellised posterior infection and waner probabilities from posterior draws of the 17 scalars,
+    ``i_raw`` (chain, draw, gap, ind) and ``ab_s_waner`` (chain, draw, ind): {"i_rb": (gap, ind), "ab_s_waner_rb": (ind,)},
+    the average over the draws of the exact conditional probability of each constrained infection given the rest of the
+    draw's state, and of ab_s_waner = 1 given the draw's scalars and i_raw.  They estimate the same quantities as the
+    mean of the Deterministic ``i`` and of ``ab_s_waner`` over the draws, with smaller Monte-Carlo error.
+    ``posterior``: mapping name -> array (an InferenceData's posterior group works)."""
+    import torch
+
+    x = np.stack([np.asarray(posterior[n], dtype=np.float64) for n, _ in Q17_RV], axis=-1)      # (chain, draw, 17)
+    i_raw, w = np.asarray(posterior["i_raw"]), np.asarray(posterior["ab_s_waner"])
+    q = forward(x.reshape(-1, 17))
+    flat_i = i_raw.reshape((-1,) + i_raw.shape[2:])
+    flat_w = w.reshape((-1,) + w.shape[2:])
+    n = len(q)
+    dev = torch.device("cuda", engine.device)
+    sum_i = torch.zeros(engine.G, engine.N, dtype=torch.float64, device=dev)
+    sum_w = torch.zeros(engine.N, dtype=torch.float64, device=dev)
+    st = torch.cuda.current_stream(dev).cuda_stream
+    for k in range(0, n, batch):
+        b = min(batch, n - k)
+        qd = torch.from_numpy(np.ascontiguousarray(q[k:k + b])).to(dev)
+        i8 = torch.from_numpy(np.ascontiguousarray(flat_i[k:k + b] != 0, dtype=np.int8)).to(dev)
+        w8 = torch.from_numpy(np.ascontiguousarray(flat_w[k:k + b] != 0, dtype=np.int8)).to(dev)
+        engine.infection_probs_accum_dev(b, qd.data_ptr(), i8.data_ptr(), w8.data_ptr(), sum_i.data_ptr(), sum_w.data_ptr(), st)
+    torch.cuda.synchronize(dev)
+    return {"i_rb": (sum_i / n).cpu().numpy(), "ab_s_waner_rb": (sum_w / n).cpu().numpy()}
+
+
 # ------------------------------------------------------------------------------------------
 # abdpymc-infer
 # ------------------------------------------------------------------------------------------
 def infer_builtin(cohort, splits, ignore_pcrpos, tune, draws, chains=4, device=0, seed=0, progress=None, gibbs_mode=0,
-                  thinned=0, kernel="hmc", shard=None, rank=0, world=1, engine=None):
+                  thinned=0, kernel="hmc", shard=None, rank=0, world=1, engine=None, rao_blackwell=False):
     """tune + draws iterations of the built-in HMC + GPU-Gibbs sampler.  Returns (result,
     {name: array (chain, draw, ...)}, last binary state) with the reference's posterior variable names.
+    ``rao_blackwell``: ``result.means`` also holds the Rao-Blackwellised infection and waner probabilities
+    ``i_rb`` (G, N) and ``ab_s_waner_rb`` (N,) (``SamplerConfig.rao_blackwell``).
 
     ``shard`` (one process per GPU, ``torch.distributed`` initialised, ``world`` ranks):
       "individuals": the cohort is split into contiguous blocks of individuals, one per rank; the 17 scalars
@@ -377,7 +408,7 @@ def infer_builtin(cohort, splits, ignore_pcrpos, tune, draws, chains=4, device=0
     x0 = np.array([1.0 / G, 2, 1, 10 / 11, -2, 2, 10 / 11, 0.5, 1, 1, -2, -1, 2, 1, -1, 2, 1], dtype=np.float64)
     q0 = forward(x0)[None, :] + rng.uniform(-1, 1, size=(chains, 17))
     cfg = SamplerConfig(tune=tune, draws=draws, seed=seed, record_deterministics_every=1, thinned_deterministics=thinned,
-                        kernel=kernel)
+                        kernel=kernel, rao_blackwell=rao_blackwell)
     if world > 1 and shard == "individuals":
         from .distributed import ShardedEngine, ShardedTarget
 
@@ -447,6 +478,12 @@ def _write_builtin(args, data, res, post, last):
                         extra["observed_data"] = {"it_s_lik": data.rows(1)[1], "it_n_lik": data.rows(0)[1]}
             idata = az.from_dict(posterior=posterior, sample_stats=sample_stats, dims=dims,
                                  coords={"gap": np.arange(data.n_gaps), "ind": np.arange(data.n_inds)}, **extra)
+            if "i_rb" in res.means:   # no (chain, draw) axes: a Dataset, so that ArviZ does not prepend them
+                import xarray as xr
+
+                idata.add_groups(rao_blackwell=xr.Dataset(
+                    {"i_rb": (GAP_IND, res.means["i_rb"]), "ab_s_waner_rb": ("ind", res.means["ab_s_waner_rb"])},
+                    coords={"gap": np.arange(data.n_gaps), "ind": np.arange(data.n_inds)}))
             az.to_netcdf(idata, out)
             print(f"PyMC not installed: sampled with the built-in HMC+Gibbs driver in {res.wall_s:.1f} s; wrote {out}",
                   file=sys.stderr)
@@ -504,7 +541,8 @@ def _builtin_worker(rank, args, devices, port):
     res, post, last = infer_builtin(data, splits, args.ignore_pcrpos, args.tune, args.draws, chains=args.chains,
                                     device=devices[rank], progress=max(1, (args.tune + args.draws) // 10),
                                     gibbs_mode=args.gibbs_mode, thinned=args.thinned, kernel=args.kernel,
-                                    shard=args.shard if world > 1 else None, rank=rank, world=world, engine=engine)
+                                    shard=args.shard if world > 1 else None, rank=rank, world=world, engine=engine,
+                                    rao_blackwell=args.rao_blackwell)
     if rank == 0:
         _write_builtin(args, data, res, post, last)
     if world > 1:
@@ -546,6 +584,10 @@ def main(argv=None):
     parser.add_argument("--gibbs_mode", type=int, default=0, choices=[0, 1, 2],
                         help="(extension) update rule of the indicator sweep: 0 BinaryGibbsMetropolis semantics, "
                              "1 single-site exact conditionals, 2 per-chunk block draw (include/abd_b200.h)")
+    parser.add_argument("--rao_blackwell", action="store_true",
+                        help="(extension, PyMC-free driver) also write the Rao-Blackwellised posterior infection and waner "
+                             "probabilities (mean_i_rb (gap, ind), mean_ab_s_waner_rb (ind)): the same quantities as the "
+                             "mean of i and of ab_s_waner, with smaller Monte-Carlo error")
     args = parser.parse_args(argv)
     if args.cores not in (None, 1):
         print(f"abdpymc-infer: --cores {args.cores} ignored -- the chains of a run are batched on the GPU(s) of this process "

@@ -16,6 +16,7 @@
 //   k_sums.cuh              k_sums (joint logp + gradient sums, fused finaliser, persistent trajectory
 //                           mode, fused peer all-reduce), k_finalize
 //   k_gibbs.cuh             k_gibbs (Gibbs sweep, conditional log-odds); k_gibbs_blk.cuh: the per-chunk block draw
+//   k_infprob.cuh           k_infprob_accum (Rao-Blackwellised posterior infection and waner probabilities)
 //   k_nuts.cuh              the No-U-Turn tree (k_nuts_begin / k_nuts_leaf / k_nuts_end; nuts_leaf_chain is also called by
 //                           the finishing warp of k_sums' single-step leapfrog launches)
 //   k_misc.cuh              k_hmc_begin / k_hmc_end, k_determ, k_determ_accum, k_loglik_rows, k_pack, k_pull, k_debug_fast_math
@@ -61,6 +62,7 @@ int fail(int code, const std::string& msg) {
 #include "k_sums.cuh"
 #include "k_gibbs.cuh"
 #include "k_gibbs_blk.cuh"
+#include "k_infprob.cuh"
 #include "k_misc.cuh"
 
 
@@ -1458,6 +1460,25 @@ int abd_deterministics_accum_dev(abd_handle* h, int C, const double* theta, int 
   const cudaStream_t st = (cudaStream_t)stream;
   with_mask(h, [&](auto m) {
     k_determ_accum<decltype(m)><<<grid, 128, 0, st>>>(h->dc, C, theta, theta_is_q17, i_raw, waner, sum_i, sum_mu_n, sum_mu_s);
+  });
+  CU(cudaGetLastError());
+  h->launches++;
+  return ABD_OK;
+}
+
+int abd_infection_probs_accum_dev(abd_handle* h, int C, const double* q17, const int8_t* i_raw, const int8_t* waner,
+                                  double* sum_i, double* sum_w, void* stream) {
+  PROLOGUE(h, C);
+  if (!q17 || !i_raw || !waner || !sum_i || !sum_w) return fail(ABD_ERR_INVALID, "NULL argument");
+  const cudaStream_t st = (cudaStream_t)stream;
+  void* pack = nullptr;
+  int rc = resident_pack(h, C, i_raw, waner, st, &pack);
+  if (rc) return rc;
+  const int grid = (h->N + kGibbsWarps - 1) / kGibbsWarps;
+  with_mask(h, [&](auto m) {
+    using M = decltype(m);
+    k_infprob_accum<M><<<grid, kGibbsWarps * 32, 0, st>>>(h->dc, h->d_order, C, q17, i_raw, waner,
+                                                          (const PackedState<M>*)pack, sum_i, sum_w);
   });
   CU(cudaGetLastError());
   h->launches++;

@@ -74,9 +74,10 @@ __device__ __forceinline__ double gibbs_row_tv(double x, double od, int t, bool 
 // One chain's parameters into a warp's shared-memory slot (all 32 lanes call it):
 //   s_th[0..12] theta13, [13], [14] -1/(2 sigma^2) of N / S, [15], [16] logit p / p_waner,
 //   [17], [18] sigmoid of those, [19], [20], [21] log p, log(1 - p), p; s_pw[0] = rho_n^k, s_pw[1] = rho_s^k.
+template <typename M = uint32_t>
 __device__ __forceinline__ void gibbs_load_chain(const double* __restrict__ theta, int theta_is_q,
                                                  const double* __restrict__ p_arr, const double* __restrict__ pw_arr,
-                                                 int c, int G, int lane, double* s_th, double (*s_pw)[kGapTab<uint32_t>]) {
+                                                 int c, int G, int lane, double* s_th, double (*s_pw)[kGapTab<M>]) {
   __syncwarp();
   fill_pow_warp(load_param(theta, theta_is_q, c, N_RHO), G, lane, s_pw[0], nullptr);
   fill_pow_warp(load_param(theta, theta_is_q, c, S_RHO), G, lane, s_pw[1], nullptr);

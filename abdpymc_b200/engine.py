@@ -424,3 +424,9 @@ class AbdEngine:
         """Adds the sum over chains of i, ab_n_mu, ab_s_mu (G, N) to the running totals (device pointers)."""
         check(self._lib.abd_deterministics_accum_dev(self._h, C_, theta, int(theta_is_q17), i_raw, waner, sum_i, sum_mu_n,
                                                      sum_mu_s, stream))
+
+    def infection_probs_accum_dev(self, C_, q17, i_raw, waner, sum_i, sum_w, stream=0):
+        """Adds, summed over the chains, the Rao-Blackwellised infection probabilities (G, N) to ``sum_i`` and the waner
+        probabilities (N,) to ``sum_w`` (device pointers): the exact conditional probability of each constrained
+        infection given the rest of the state, and of ab_s_waner = 1 given theta and i_raw."""
+        check(self._lib.abd_infection_probs_accum_dev(self._h, C_, q17, i_raw, waner, sum_i, sum_w, stream))

@@ -116,6 +116,18 @@ class DeviceTarget:
         self.engine.deterministics_accum_dev(self.C, q.data_ptr(), 1, self.d_i, self.d_w, sums["i"].data_ptr(),
                                              sums["ab_n_mu"].data_ptr(), sums["ab_s_mu"].data_ptr(), self._stream())
 
+    def accumulate_infection_probs(self, q, sums):
+        """Rao-Blackwellised posterior probabilities: adds this state's exact conditional infection probabilities
+        ``sums["i_rb"]`` (G, N) and waner probabilities ``sums["ab_s_waner_rb"]`` (N,), summed over the chains, in one
+        launch (float64 device tensors, created on first use).  Reads the state only; the chain is not touched."""
+        G, N = self.engine.G, self.engine.N
+        if "i_rb" not in sums:
+            sums["i_rb"] = torch.zeros(G, N, dtype=torch.float64, device=self.device)
+            sums["ab_s_waner_rb"] = torch.zeros(N, dtype=torch.float64, device=self.device)
+        q = q.contiguous()
+        self.engine.infection_probs_accum_dev(self.C, q.data_ptr(), self.d_i, self.d_w, sums["i_rb"].data_ptr(),
+                                              sums["ab_s_waner_rb"].data_ptr(), self._stream())
+
     def state(self):
         """The binary state (i_raw (C, G, N), waner (C, N)); on a sharded cohort this rank's block of individuals."""
         torch.cuda.synchronize(self.device)
@@ -186,6 +198,8 @@ class SamplerConfig:
     target_accept: float = 0.8
     init_step: float = 0.05
     record_deterministics_every: int = 0   # 0 = never; k = accumulate means every k-th draw
+    rao_blackwell: bool = False            # at the same draws, also average the exact conditional infection / waner
+                                           # probabilities: means["i_rb"] (G, N), means["ab_s_waner_rb"] (N,)
     thinned_deterministics: int = 0        # keep this many evenly spaced draws of i / ab_n_mu / ab_s_mu per chain (the
                                            # consumers use <= 250: survival.py:109-114, timelines.py:289-301); 0 = none
     persistent_trajectories: bool = True   # run the whole transition on the device when the target can (``device_loop``);
@@ -212,7 +226,8 @@ class SamplerResult:
     inv_mass: np.ndarray               # (dim, dim) adapted covariance (inverse mass matrix)
     wall_s: float
     n_grad_evals: int
-    means: dict = field(default_factory=dict)   # posterior means of i, ab_n_mu, ab_s_mu (G, N)
+    means: dict = field(default_factory=dict)   # posterior means of i, ab_n_mu, ab_s_mu (G, N); with rao_blackwell
+                                                # also i_rb (G, N) and ab_s_waner_rb (N,)
     thinned: dict = field(default_factory=dict)  # i (int8), ab_n_mu, ab_s_mu (float32): (chains, kept draws, G, N); "draw" = their indexes
     stats: dict = field(default_factory=dict)   # NUTS: tree_depth, diverging (chains, draws); what PyMC puts in sample_stats
     wall_tune_s: float = 0.0           # the part of wall_s spent in the tuning iterations ...
@@ -611,6 +626,8 @@ def sample(target, q0, cfg: SamplerConfig = SamplerConfig(), progress=None) -> S
             every = cfg.record_deterministics_every
             if every and k % every == 0 and hasattr(target, "accumulate_deterministics"):
                 target.accumulate_deterministics(run.q, means)   # sums over chains; divided once at the end
+                if cfg.rao_blackwell:
+                    target.accumulate_infection_probs(run.q, means)
                 n_means += C
         if progress and (it + 1) % progress == 0:
             print(f"  iter {it + 1}/{total}  step {run.eps.mean().item():.4f}  accept {run.acc.mean().item():.2f}", flush=True)

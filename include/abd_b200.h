@@ -233,6 +233,18 @@ int abd_deterministics_dev(abd_handle* h, int n_chains, const double* theta13,
 int abd_deterministics_accum_dev(abd_handle* h, int n_chains, const double* theta, int theta_is_q17,
                                  const int8_t* i_raw, const int8_t* waner, double* sum_i,
                                  double* sum_mu_n, double* sum_mu_s, void* stream);
+/* Rao-Blackwellised posterior infection and waner probabilities (serves the posterior means of i and
+ * ab_s_waner that survival.py:68-69 and timelines.py:274,305-309 read; i is abd.py:649 / 667).  For
+ * the state (q17, i_raw, waner) of each of the C chains, ADD to sum_i (G, N) the exact conditional
+ * probability of each constrained infection i[t, n] given the state outside its block (the time chunk
+ * holding gap t, or raw bit t alone without splits), and to sum_w (N) that of ab_s_waner[n] = 1 given
+ * theta and i_raw; the chains are summed in order first, so the totals are bitwise reproducible.
+ * Divided by chains x recorded draws these estimate the same posterior means as the average of the
+ * 0/1 draws of i and ab_s_waner, with smaller Monte-Carlo error (DESIGN.md section 4,
+ * k_infprob_accum).  Reads the state only (the resident buffers, or any device int8 arrays); draws no random numbers.  On a
+ * sharded cohort each rank adds its own block of individuals; there is no collective.           */
+int abd_infection_probs_accum_dev(abd_handle* h, int n_chains, const double* q17, const int8_t* i_raw,
+                                  const int8_t* waner, double* sum_i, double* sum_w, void* stream);
 /* n_steps leapfrog steps of Hamiltonian dynamics over q17 for C chains with the binary state
  * fixed, in ONE persistent launch (what a NUTS / HMC trajectory of pm.sample, abd.py:922, costs
  * n_steps calls of logp_dlogp_function for).  Per step: p += eps/2 grad; q += eps inv_mass p;
