@@ -664,52 +664,36 @@ int launch_sums(abd_handle* h, int C, const double* theta, int theta_is_q, const
 
 int launch_gibbs(abd_handle* h, int C, const double* theta, int theta_is_q, const double* p,
                  const double* pw, int8_t* i_raw, int8_t* waner, const GibbsCfg& cfg, cudaStream_t st) {
-  if (cfg.mode == ABD_GIBBS_BLOCKED) {
-    if (h->mask_bits > 32 || h->dc.ch.n < 2) {
-      // no "first raw 1 of the chunk" structure (one chunk) or more options than lanes (masks wider than 32 bits):
-      // single-site exact conditionals instead
-      GibbsCfg c2 = cfg;
-      c2.mode = ABD_GIBBS_HEATBATH;
-      return launch_gibbs(h, C, theta, theta_is_q, p, pw, i_raw, waner, c2, st);
-    }
-    if (!h->gibbs_blk_ctas) {
+  const bool blk = cfg.mode == ABD_GIBBS_BLOCKED;
+  if (blk && (h->mask_bits > 32 || h->dc.ch.n < 2)) {
+    // no "first raw 1 of the chunk" structure (one chunk) or more options than lanes (masks wider than 32 bits):
+    // single-site exact conditionals instead
+    GibbsCfg c2 = cfg;
+    c2.mode = ABD_GIBBS_HEATBATH;
+    return launch_gibbs(h, C, theta, theta_is_q, p, pw, i_raw, waner, c2, st);
+  }
+  return with_mask(h, [&](auto m) -> int {
+    using M = decltype(m);
+    auto kernel = k_gibbs<M>;
+    if constexpr (std::is_same_v<M, uint32_t>)
+      if (blk) kernel = k_gibbs_blk;
+    int& ctas = blk ? h->gibbs_blk_ctas : h->gibbs_ctas;  // one persistent wave
+    if (!ctas) {
       int occ = 0;
-      CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_gibbs_blk, kGibbsWarps * 32, 0));
-      h->gibbs_blk_ctas = h->n_sms * std::max(occ, 1);
+      CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kernel, kGibbsWarps * 32, 0));
+      ctas = h->n_sms * std::max(occ, 1);
     }
     const long items = (long)C * h->N;
-    const int grid = (int)std::min<long>(h->gibbs_blk_ctas, (items + kGibbsWarps - 1) / kGibbsWarps);
+    const int grid = (int)std::min<long>(ctas, (items + kGibbsWarps - 1) / kGibbsWarps);
     CU(cudaMemsetAsync(h->d_queue, 0, (size_t)C * sizeof(unsigned), st));
     void* pack = nullptr;
-    int rcp = resident_pack(h, C, i_raw, waner, st, &pack);
-    if (rcp) return rcp;
-    k_gibbs_blk<<<grid, kGibbsWarps * 32, 0, st>>>(h->dc, h->d_order, C, theta, theta_is_q, p, pw, i_raw, waner,
-                                                   (PackedState<uint32_t>*)pack, h->d_queue, cfg);
+    if (int rc = resident_pack(h, C, i_raw, waner, st, &pack)) return rc;
+    kernel<<<grid, kGibbsWarps * 32, 0, st>>>(h->dc, h->d_order, C, theta, theta_is_q, p, pw, i_raw, waner,
+                                              (PackedState<M>*)pack, h->d_queue, cfg);
     CU(cudaGetLastError());
     h->launches++;
     return ABD_OK;
-  }
-  if (!h->gibbs_ctas) {
-    int occ = 0;
-    CU(with_mask(h, [&](auto m) {
-      return cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_gibbs<decltype(m)>, kGibbsWarps * 32, 0);
-    }));
-    h->gibbs_ctas = h->n_sms * std::max(occ, 1);
-  }
-  const long items = (long)C * h->N;
-  const int grid = (int)std::min<long>(h->gibbs_ctas, (items + kGibbsWarps - 1) / kGibbsWarps);
-  CU(cudaMemsetAsync(h->d_queue, 0, (size_t)C * sizeof(unsigned), st));
-  void* pack = nullptr;
-  int rcp = resident_pack(h, C, i_raw, waner, st, &pack);
-  if (rcp) return rcp;
-  with_mask(h, [&](auto m) {
-    using M = decltype(m);
-    k_gibbs<M><<<grid, kGibbsWarps * 32, 0, st>>>(h->dc, h->d_order, C, theta, theta_is_q, p, pw, i_raw, waner,
-                                                   (PackedState<M>*)pack, h->d_queue, cfg);
   });
-  CU(cudaGetLastError());
-  h->launches++;
-  return ABD_OK;
 }
 
 int set_device(const abd_handle* h) {

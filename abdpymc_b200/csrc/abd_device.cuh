@@ -123,16 +123,6 @@ __device__ __forceinline__ M constrain(M raw, M pcr, const Chunks& ch) {
   return out;
 }
 
-__device__ __forceinline__ double ipow(double r, int k) {
-  double acc = 1.0, b = r;
-  while (k) {
-    if (k & 1) acc *= b;
-    b *= b;
-    k >>= 1;
-  }
-  return acc;
-}
-
 // N antigen at gap t: P = 1[any infection <= t], T = sum_{s in inf, s<=t} rho^(t-s),
 // dT = dT/drho.  pwd[k] = {rho^k, k rho^(k-1)} (one 16-byte shared-memory load per event).
 template <typename M>
@@ -174,41 +164,6 @@ __device__ __forceinline__ void traj_s(M inf, M vac, int w, int t, const double2
   } else {
     U = (double)(popc(e) + popc(v));
   }
-}
-
-// value-only versions for the Gibbs kernel
-template <typename M>
-__device__ __forceinline__ double mu_n_at(M inf, int t, const double* pw, double init, double perm,
-                                          double temp) {
-  M e = inf & low_mask<M>(t);
-  double T = 0.0;
-  const double P = e ? perm : 0.0;
-  while (e) {
-    T += pw[t - ctz(e)];
-    e &= e - 1;
-  }
-  return init + P + temp * T;
-}
-template <typename M>
-__device__ __forceinline__ double mu_s_at(M inf, M vac, int w, int t, const double* pw, double init,
-                                          double perm) {
-  const M lm = low_mask<M>(t);
-  M e = inf & lm, v = vac & lm;
-  const double P = (e | v) ? perm : 0.0;
-  double U = 0.0;
-  if (w) {
-    while (e) {
-      U += pw[t - ctz(e)];
-      e &= e - 1;
-    }
-    while (v) {
-      U += pw[t - ctz(v)];
-      v &= v - 1;
-    }
-  } else {
-    U = (double)(popc(e) + popc(v));
-  }
-  return init + P + U;
 }
 
 // ---- fast fp64 exp / reciprocal for the OD-row hot loop -------------------------------------

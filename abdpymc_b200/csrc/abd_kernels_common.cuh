@@ -70,9 +70,15 @@ __device__ __forceinline__ M top_bit() { return (M)1 << (sizeof(M) * 8 - 1); }
 //   inf = constrain(raw, pcr, chunks), the constrained infections (abd.py:640-667)
 // so that an evaluation reads 8 (16) bytes per individual and chain instead of G + 1 strided bytes
 // and does not repeat the integer prologue: the binary state only changes once per Gibbs sweep.
+// Kernels go through the accessors below, never through the bits of rw.
 template <typename M>
 struct __align__(2 * sizeof(M)) PackedState {
   M rw, inf;
+  PackedState() = default;
+  __device__ __forceinline__ PackedState(M raw, int w, M inf_) : rw(raw | (w ? top_bit<M>() : (M)0)), inf(inf_) {}
+  __device__ __forceinline__ M raw() const { return rw & ~top_bit<M>(); }
+  __device__ __forceinline__ M waner_bit() const { return rw & top_bit<M>(); }  // ab_s_waner in the top bit, else 0
+  __device__ __forceinline__ int waner() const { return waner_bit() != 0; }
 };
 
 // One thread's i_raw column (gaps 0..G-1, stride N) as a bit mask.  Unpredicated loads along an address chain that

@@ -71,9 +71,17 @@ __device__ __forceinline__ double gibbs_row_tv(double x, double od, int t, bool 
   return rp.nh * row_resid2(x, od, fma(rp.tfac, T, rp.init + P), rp.b, rp.d, s_tab);
 }
 
-// One chain's parameters into a warp's shared-memory slot (all 32 lanes call it):
-//   s_th[0..12] theta13, [13], [14] -1/(2 sigma^2) of N / S, [15], [16] logit p / p_waner,
-//   [17], [18] sigmoid of those, [19], [20], [21] log p, log(1 - p), p; s_pw[0] = rho_n^k, s_pw[1] = rho_s^k.
+// A warp's per-chain parameter block s_th: theta13 in [0, 13) (enum Theta), then these.  k_gibbs keeps 20 doubles
+// per warp (it reads no slot past TH_SIG_PW), the other kernels 24.
+enum GibbsTh {
+  TH_NH_N = 13, TH_NH_S,        // -1/(2 sigma^2) of the N / S rows
+  TH_LOGIT_P, TH_LOGIT_PW,      // logit p, logit p_waner
+  TH_SIG_P, TH_SIG_PW,          // sigmoid of those: the heat-bath threshold of a prior-only bit
+  TH_LOG_P, TH_LOG1M_P, TH_P    // log p, log(1 - p), p
+};
+
+// One chain's parameters into a warp's shared-memory slot (all 32 lanes call it): s_th as above,
+// s_pw[0] = rho_n^k, s_pw[1] = rho_s^k.
 template <typename M = uint32_t>
 __device__ __forceinline__ void gibbs_load_chain(const double* __restrict__ theta, int theta_is_q,
                                                  const double* __restrict__ p_arr, const double* __restrict__ pw_arr,
@@ -82,12 +90,12 @@ __device__ __forceinline__ void gibbs_load_chain(const double* __restrict__ thet
   fill_pow_warp(load_param(theta, theta_is_q, c, N_RHO), G, lane, s_pw[0], nullptr);
   fill_pow_warp(load_param(theta, theta_is_q, c, S_RHO), G, lane, s_pw[1], nullptr);
   if (lane < 13) s_th[lane] = load_param(theta, theta_is_q, c, lane);
-  if (lane == 13 || lane == 14) {
-    const double sg = load_param(theta, theta_is_q, c, lane == 13 ? N_SIGMA : S_SIGMA);
+  if (lane == TH_NH_N || lane == TH_NH_S) {
+    const double sg = load_param(theta, theta_is_q, c, lane == TH_NH_N ? N_SIGMA : S_SIGMA);
     s_th[lane] = -0.5 / (sg * sg);
   }
-  if (lane == 15 || lane == 16) {
-    const int which = lane - 15;
+  if (lane == TH_LOGIT_P || lane == TH_LOGIT_PW) {
+    const int which = lane - TH_LOGIT_P;
     double lo, pv;
     if (theta_is_q) {  // logit of a logodds-transformed value is the value itself
       lo = theta[(size_t)c * 17 + (which ? kQ_PW : kQ_P)];
@@ -97,11 +105,11 @@ __device__ __forceinline__ void gibbs_load_chain(const double* __restrict__ thet
       lo = log(pv) - log1p(-pv);
     }
     s_th[lane] = lo;
-    s_th[lane + 2] = 1.0 / (1.0 + exp(-lo));  // the heat-bath threshold of a prior-only bit: sigmoid(logit)
+    s_th[TH_SIG_P + which] = 1.0 / (1.0 + exp(-lo));
     if (!which) {
-      s_th[19] = log(pv);
-      s_th[20] = log1p(-pv);
-      s_th[21] = pv;
+      s_th[TH_LOG_P] = log(pv);
+      s_th[TH_LOG1M_P] = log1p(-pv);
+      s_th[TH_P] = pv;
     }
   }
   __syncwarp();
@@ -174,7 +182,7 @@ struct GibbsRows {
     rp.tfac = is_s ? 1.0 : s_th[N_TEMP];
     rp.b = s_th[is_s ? S_B : N_B];
     rp.d = s_th[is_s ? S_D : N_D];
-    rp.nh = s_th[is_s ? 14 : 13];
+    rp.nh = s_th[is_s ? TH_NH_S : TH_NH_N];
     return rp;
   }
   __device__ __forceinline__ double ll(M inf_, M vac, int w_) const {
@@ -196,6 +204,126 @@ struct GibbsRows {
   }
 };
 
+// The binary state of (chain c, individual n) as a warp reads it: the resident packed entry (one broadcast load,
+// constraints already applied) or else the int8 column col = i_raw + c G N + n (gap t at col[t N]; gap 32 s + lane
+// in ballot s) and the constraints.  The caller forms col once and keeps it for warp_store_state: formed
+// again in each helper, the 64-register sweep kernels spill more.
+template <typename M>
+__device__ __forceinline__ void warp_load_state(const DevCohort& dc, const PackedState<M>* pack, const int8_t* col,
+                                                const int8_t* waner, int c, int n, M pcr, int lane, M& raw, M& inf, int& w) {
+  const int G = dc.G, N = dc.N;
+  if (pack) {
+    const PackedState<M> ps = pack[(size_t)c * N + n];
+    raw = ps.raw();
+    w = ps.waner();
+    inf = ps.inf;
+  } else {
+    raw = 0;
+#pragma unroll
+    for (int s = 0; s < (int)sizeof(M) / 4; ++s) {
+      const int t = lane + 32 * s;
+      const int8_t b = (t < G) ? col[(size_t)t * N] : (int8_t)0;
+      raw |= (M)__ballot_sync(0xffffffffu, b != 0) << (32 * s);
+    }
+    w = waner[(size_t)c * N + n] != 0;
+    inf = constrain<M>(raw, pcr, dc.ch);
+  }
+}
+
+// The sweep's result for (c, n) back into the state it was read from (raw_in, w_in): only what changed.
+template <typename M>
+__device__ __forceinline__ void warp_store_state(const DevCohort& dc, PackedState<M>* pack, int8_t* col, int8_t* waner,
+                                                 int c, int n, int lane, M raw, M raw_in, int w, int w_in, M inf) {
+  const int G = dc.G, N = dc.N;
+  const M changed = raw ^ raw_in;
+#pragma unroll
+  for (int s = 0; s < (int)sizeof(M) / 4; ++s) {
+    const int t = lane + 32 * s;
+    if (t < G && ((changed >> t) & 1)) col[(size_t)t * N] = (int8_t)((raw >> t) & 1);
+  }
+  if (lane == 0 && w != w_in) waner[(size_t)c * N + n] = (int8_t)w;
+  if (pack && lane == 0 && (changed != 0 || w != w_in)) pack[(size_t)c * N + n] = PackedState<M>(raw, w, inf);
+}
+
+// Persistent warps over one work queue per chain (individuals by decreasing OD-row count, so the tail at the end of
+// the launch is one short job).  A warp starts at the chain its global index points to and moves on when that queue is
+// empty, so it (re)loads chain parameters once or twice per sweep instead of once per chain (a single chain-major
+// queue walked every warp through all C chains: ~6 % of the sweep's instructions).  The warp counts its proposals and
+// accepted flips per chain and adds them to stats[c][0 / 1] (if not null) when it leaves chain c.
+struct ChainQueues {
+  unsigned* queue;
+  unsigned long long* stats;
+  int C, N, cq, cur_c = -1, exhausted = 0;
+  unsigned n_prop = 0, n_acc = 0;
+
+  __device__ __forceinline__ ChainQueues(unsigned* queue_, unsigned long long* stats_, int C_, int N_, unsigned gwarp)
+      : queue(queue_), stats(stats_), C(C_), N(N_), cq((int)(gwarp % (unsigned)C_)) {}
+  // claims the warp's next item of chain `c`: false when the queue was empty (the warp moves to the next chain; the
+  // caller stops once done()).  One claim per call, so the kernel's loop stays a single loop: a claim-until-found
+  // loop inside it made the compiler run the item in two diverged halves of the warp, 2.5x slower.
+  __device__ __forceinline__ bool claim(int lane, int& c, unsigned& item) {
+    unsigned it = 0;
+    if (lane == 0) it = atomicAdd(queue + cq, 1u);
+    it = __shfl_sync(0xffffffffu, it, 0);
+    if (it >= (unsigned)N) {
+      ++exhausted;
+      cq = (cq + 1 == C) ? 0 : cq + 1;
+      return false;
+    }
+    exhausted = 0;
+    c = cq, item = it;
+    return true;
+  }
+  __device__ __forceinline__ bool done() const { return exhausted >= C; }
+  // true when c is not the chain of the previous item: the counts so far are flushed, the caller loads c's parameters
+  __device__ __forceinline__ bool enter(int c, int lane) {
+    if (c == cur_c) return false;
+    flush(lane);
+    n_prop = n_acc = 0;
+    cur_c = c;
+    return true;
+  }
+  __device__ __forceinline__ void flush(int lane) const {
+    if (cur_c >= 0 && stats && lane == 0) {
+      atomicAdd(&stats[(size_t)cur_c * 2], (unsigned long long)n_prop);
+      atomicAdd(&stats[(size_t)cur_c * 2 + 1], (unsigned long long)n_acc);
+    }
+  }
+};
+
+// Time chunks (k_gibbs_blk, k_infprob_accum): lane o < n holds the constrained infections inf_own of one option of a
+// chunk ("first raw 1 at ..."); returns that option's log-likelihood (other lanes: ll_none, the chunk without a 1).
+// An option the data cannot tell from none -- it differs from inf_none only after the individual's last sample,
+// t_last -- takes ll_none, one equal to the current state (inf, w) takes its ll; the others are evaluated by
+// ll_of(infections, w), the kernel's log-likelihood of the individual.
+template <typename M, typename LL>
+__device__ __forceinline__ double chunk_options_ll(M inf_own, int n, M inf_none, double ll_none, M inf, int w, double ll,
+                                                   int t_last, int lane, LL&& ll_of) {
+  double llv = ll_none;
+  for (int o = 0; o < n; ++o) {
+    const M io = shfl_mask(inf_own, o);
+    const M diff = io ^ inf_none;
+    if (diff != 0 && ctz(diff) <= t_last) {
+      const double v = (io == inf) ? ll : ll_of(io, w);
+      if (lane == o) llv = v;
+    }
+  }
+  return llv;
+}
+
+// The exact conditional log-odds of ab_s_waner = 1 versus 0 at (inf, w) into d10, and ll2 = ll_of(inf, w ^ 1).
+// Returns false when no S row follows the first exposure: then d10 = logit p_w and ll2 = ll.
+template <typename M, typename LL>
+__device__ __forceinline__ bool waner_logodds(M inf, M vac, int w, double ll, int t_last_s, const double* s_th,
+                                              LL&& ll_of, double& d10, double& ll2) {
+  const M ex = inf | vac;
+  d10 = s_th[TH_LOGIT_PW], ll2 = ll;
+  if (!(ex != 0 && ctz(ex | top_bit<M>()) < t_last_s)) return false;
+  ll2 = ll_of(inf, w ^ 1);
+  d10 += w ? (ll - ll2) : (ll2 - ll);
+  return true;
+}
+
 // a[i] of a per-lane array of proposal slots (i uniform over the warp), by selects: a dynamic index would put the
 // array in local memory
 template <int NS, typename T>
@@ -210,11 +338,10 @@ __device__ __forceinline__ T slot(const T (&a)[NS], int i) {
   }
 }
 
-// (k_gibbs below keeps its own hand-inlined copy of these two: going through the helpers costs it
-// 4 % -- 274 instead of 264 us per sweep, a few more spilled registers under its 64-register cap.)
-// Persistent warps: every warp repeatedly claims the next (chain, individual) from a global
-// counter.  Items are ordered chain-major and, inside a chain, by decreasing OD-row count
-// (longest job first), so the tail at the end of the launch is one short job.
+// Single-site sweep (Metropolis or heat bath) or the conditional log-odds of every bit, over ChainQueues.  It shares
+// the state load / write-back and the queues with k_gibbs_blk but keeps its own hand-inlined copies of
+// gibbs_load_chain and GibbsRows: going through those costs it 4 % -- 274 instead of 264 us per sweep, a few more
+// spilled registers under its 64-register cap.
 // 4 CTAs/SM (64 registers, a few spills) is 3 % faster than 3 x 80 registers; 5 is slower.  Also
 // measured and dropped: patching each row's decaying response for a candidate instead of summing
 // it again (no gain: the extra live registers cost what the shorter loops save).
@@ -241,43 +368,27 @@ k_gibbs(const DevCohort dc, const int* __restrict__ order, const int C,
   __syncthreads();
 
   const int nprop = G + 1;  // proposal j < G flips i_raw[j, n]; j == G flips waner[n]
-  unsigned n_prop = 0, n_acc = 0;
-  int cur_c = -1;
-
-  // One work queue per chain (individuals by decreasing OD-row count); a warp starts at the chain its global index
-  // points to and moves on when that queue is empty, so it (re)loads chain parameters once or twice per sweep instead
-  // of once per chain (a single chain-major queue walked every warp through all C chains: ~6 % of the sweep's instructions).
-  int cq = (int)((blockIdx.x * kGibbsWarps + warp) % (unsigned)C), exhausted = 0;
+  ChainQueues q(queue, cfg.stats, C, N, blockIdx.x * kGibbsWarps + warp);
   while (true) {
-    unsigned item = 0;
-    if (lane == 0) item = atomicAdd(queue + cq, 1u);
-    item = __shfl_sync(0xffffffffu, item, 0);
-    if (item >= (unsigned)N) {
-      if (++exhausted >= C) break;
-      cq = (cq + 1 == C) ? 0 : cq + 1;
+    int c;
+    unsigned item;
+    if (!q.claim(lane, c, item)) {
+      if (q.done()) break;
       continue;
     }
-    exhausted = 0;
-    const int c = cq;
     const int n = order[item];
 
-    if (c != cur_c) {  // (re)load this chain's parameters into the warp's shared-memory slot
-      if (cur_c >= 0 && cfg.stats && lane == 0) {
-        atomicAdd(&cfg.stats[(size_t)cur_c * 2], (unsigned long long)n_prop);
-        atomicAdd(&cfg.stats[(size_t)cur_c * 2 + 1], (unsigned long long)n_acc);
-      }
-      n_prop = n_acc = 0;
-      cur_c = c;
+    if (q.enter(c, lane)) {  // (re)load this chain's parameters into the warp's shared-memory slot
       __syncwarp();
       fill_pow_warp(load_param(theta, theta_is_q, c, N_RHO), G, lane, s_pw_all[warp][0], nullptr);
       fill_pow_warp(load_param(theta, theta_is_q, c, S_RHO), G, lane, s_pw_all[warp][1], nullptr);
       if (lane < 13) s_th[lane] = load_param(theta, theta_is_q, c, lane);
-      if (lane == 13 || lane == 14) {
-        const double sg = load_param(theta, theta_is_q, c, lane == 13 ? N_SIGMA : S_SIGMA);
+      if (lane == TH_NH_N || lane == TH_NH_S) {
+        const double sg = load_param(theta, theta_is_q, c, lane == TH_NH_N ? N_SIGMA : S_SIGMA);
         s_th[lane] = -0.5 / (sg * sg);
       }
-      if (lane == 15 || lane == 16) {
-        const int which = lane - 15;
+      if (lane == TH_LOGIT_P || lane == TH_LOGIT_PW) {
+        const int which = lane - TH_LOGIT_P;
         double lo;
         if (theta_is_q) {  // logit of a logodds-transformed value is the value itself
           lo = theta[(size_t)c * 17 + (which ? kQ_PW : kQ_P)];
@@ -286,31 +397,17 @@ k_gibbs(const DevCohort dc, const int* __restrict__ order, const int C,
           lo = log(p) - log1p(-p);
         }
         s_th[lane] = lo;
-        s_th[lane + 2] = 1.0 / (1.0 + exp(-lo));
+        s_th[TH_SIG_P + which] = 1.0 / (1.0 + exp(-lo));
       }
       __syncwarp();
     }
 
-    // ---- this individual's column of i_raw (lane t reads gap t), waner, masks, rows ----
-    int8_t* col = i_raw + (size_t)c * G * N + n;
+    // ---- this individual's state, masks, rows ----
     const M pcr = reinterpret_cast<const M*>(dc.pcr)[n];
-    M raw = 0, inf;
+    M raw, inf;
     int w;
-    if (pack) {  // resident state: one broadcast load instead of G strided bytes, constraints already applied
-      const PackedState<M> ps = pack[(size_t)c * N + n];
-      raw = ps.rw & ~top_bit<M>();
-      w = (ps.rw & top_bit<M>()) != 0;
-      inf = ps.inf;
-    } else {
-#pragma unroll
-      for (int sl = 0; sl < NSLOT; ++sl) {
-        const int t = lane + 32 * sl;
-        const int8_t b = (t < G) ? col[(size_t)t * N] : (int8_t)0;
-        raw |= (M)__ballot_sync(0xffffffffu, b != 0) << (32 * sl);
-      }
-      w = waner[(size_t)c * N + n] != 0;
-      inf = constrain<M>(raw, pcr, dc.ch);
-    }
+    int8_t* col = i_raw + (size_t)c * G * N + n;
+    warp_load_state<M>(dc, pack, col, waner, c, n, pcr, lane, raw, inf, w);
     const M raw_in = raw;
     const int w_in = w;
     const M vac = reinterpret_cast<const M*>(dc.vac)[n];
@@ -339,7 +436,7 @@ k_gibbs(const DevCohort dc, const int* __restrict__ order, const int C,
       rp.tfac = is_s ? 1.0 : s_th[N_TEMP];
       rp.b = s_th[is_s ? S_B : N_B];
       rp.d = s_th[is_s ? S_D : N_D];
-      rp.nh = s_th[is_s ? 14 : 13];
+      rp.nh = s_th[is_s ? TH_NH_S : TH_NH_N];
       return rp;
     };
     double x0, od0;
@@ -460,11 +557,11 @@ k_gibbs(const DevCohort dc, const int* __restrict__ order, const int C,
         }
         bool flip0;
         if (cfg.mode == ABD_GIBBS_METROPOLIS) {
-          const double lo = s_th[is_w ? 16 : 15];
+          const double lo = s_th[is_w ? TH_LOGIT_PW : TH_LOGIT_P];
           const double delta = cur_bit ? -lo : lo;
           flip0 = isfinite(delta) && (acc_u[sl] < delta);
         } else {
-          flip0 = ((acc_u[sl] <= s_th[is_w ? 18 : 17]) ? 1 : 0) != cur_bit;  // s_th[17 / 18] = sigmoid(logit)
+          flip0 = ((acc_u[sl] <= s_th[is_w ? TH_SIG_PW : TH_SIG_P]) ? 1 : 0) != cur_bit;
         }
         code_own[sl] = affected ? 2 : (flip0 ? 1 : 0);
       }
@@ -479,7 +576,7 @@ k_gibbs(const DevCohort dc, const int* __restrict__ order, const int C,
       const int code = __shfl_sync(0xffffffffu, slot(code_own, jb), owner);
       const bool is_w = (jp == G);
       if (cfg.mode >= 0) {
-        ++n_prop;
+        ++q.n_prop;
         if (code == 0) continue;
       }
       const M inf2 = shfl_mask(slot(inf2_own, jb), owner);
@@ -489,7 +586,7 @@ k_gibbs(const DevCohort dc, const int* __restrict__ order, const int C,
       if (code == 2 || cfg.mode < 0) {
         const int cur_bit = is_w ? w : (int)((raw >> jp) & 1);
         if (code == 2) ll2 = indiv_ll(inf2, w2);
-        const double lo = s_th[is_w ? 16 : 15];
+        const double lo = s_th[is_w ? TH_LOGIT_PW : TH_LOGIT_P];
         const double d10 = cur_bit ? (ll - ll2 + lo) : (ll2 - ll + lo);  // log-odds of 1 versus 0
         if (cfg.mode < 0) {
           if (lane == 0) {
@@ -508,7 +605,7 @@ k_gibbs(const DevCohort dc, const int* __restrict__ order, const int C,
         }
       }
       if (flip) {
-        ++n_acc;
+        ++q.n_acc;
         ll = ll2;
         if (is_w) {
           w = w2;
@@ -520,26 +617,9 @@ k_gibbs(const DevCohort dc, const int* __restrict__ order, const int C,
       }
     }
 
-    if (cfg.mode >= 0) {  // write back only what changed
-      const M changed = raw ^ raw_in;
-#pragma unroll
-      for (int sl = 0; sl < NSLOT; ++sl) {
-        const int t = lane + 32 * sl;
-        if (t < G && ((changed >> t) & 1)) col[(size_t)t * N] = (int8_t)((raw >> t) & 1);
-      }
-      if (lane == 0 && w != w_in) waner[(size_t)c * N + n] = (int8_t)w;
-      if (pack && lane == 0 && (changed != 0 || w != w_in)) {
-        PackedState<M> ps;
-        ps.rw = raw | (w ? top_bit<M>() : (M)0);
-        ps.inf = inf;
-        pack[(size_t)c * N + n] = ps;
-      }
-    }
+    if (cfg.mode >= 0) warp_store_state<M>(dc, pack, col, waner, c, n, lane, raw, raw_in, w, w_in, inf);
   }
-  if (cfg.mode >= 0 && cfg.stats && lane == 0 && cur_c >= 0) {
-    atomicAdd(&cfg.stats[(size_t)cur_c * 2], (unsigned long long)n_prop);
-    atomicAdd(&cfg.stats[(size_t)cur_c * 2 + 1], (unsigned long long)n_acc);
-  }
+  q.flush(lane);
 }
 
 }  // namespace

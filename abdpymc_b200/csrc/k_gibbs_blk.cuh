@@ -45,52 +45,23 @@ k_gibbs_blk(const DevCohort dc, const int* __restrict__ order, const int C,
   for (int k = lane; k < kGapTab<M>; k += 32) s_pw_all[warp][2][k] = 1.0;
   __syncthreads();
 
-  unsigned n_prop = 0, n_acc = 0;
-  int cur_c = -1;
-
-  // One work queue per chain (individuals by decreasing OD-row count); a warp starts at the chain its global index
-  // points to and moves on when that queue is empty, so it (re)loads chain parameters once or twice per sweep instead
-  // of once per chain (a single chain-major queue walked every warp through all C chains: ~6 % of the sweep's instructions).
-  int cq = (int)((blockIdx.x * kGibbsWarps + warp) % (unsigned)C), exhausted = 0;
+  ChainQueues q(queue, cfg.stats, C, N, blockIdx.x * kGibbsWarps + warp);
   while (true) {
-    unsigned item = 0;
-    if (lane == 0) item = atomicAdd(queue + cq, 1u);
-    item = __shfl_sync(FULL, item, 0);
-    if (item >= (unsigned)N) {
-      if (++exhausted >= C) break;
-      cq = (cq + 1 == C) ? 0 : cq + 1;
+    int c;
+    unsigned item;
+    if (!q.claim(lane, c, item)) {
+      if (q.done()) break;
       continue;
     }
-    exhausted = 0;
-    const int c = cq;
     const int n = order[item];
+    if (q.enter(c, lane)) gibbs_load_chain(theta, theta_is_q, p_arr, pw_arr, c, G, lane, s_th, s_pw_all[warp]);
 
-    if (c != cur_c) {  // (re)load this chain's parameters into the warp's shared-memory slot
-      if (cur_c >= 0 && cfg.stats && lane == 0) {
-        atomicAdd(&cfg.stats[(size_t)cur_c * 2], (unsigned long long)n_prop);
-        atomicAdd(&cfg.stats[(size_t)cur_c * 2 + 1], (unsigned long long)n_acc);
-      }
-      n_prop = n_acc = 0;
-      cur_c = c;
-      gibbs_load_chain(theta, theta_is_q, p_arr, pw_arr, c, G, lane, s_th, s_pw_all[warp]);
-    }
-
-    // ---- this individual's column of i_raw (lane t reads gap t), waner, masks, rows ----
-    int8_t* col = i_raw + (size_t)c * G * N + n;
+    // ---- this individual's state, masks, rows ----
     const M pcr = reinterpret_cast<const M*>(dc.pcr)[n];
     M raw, inf;
     int w;
-    if (pack) {  // resident state: one broadcast load, constraints already applied
-      const PackedState<M> ps = pack[(size_t)c * N + n];
-      raw = ps.rw & ~top_bit<M>();
-      w = (ps.rw & top_bit<M>()) != 0;
-      inf = ps.inf;
-    } else {
-      const int8_t b0 = (lane < G) ? col[(size_t)lane * N] : (int8_t)0;
-      raw = __ballot_sync(FULL, b0 != 0);
-      w = waner[(size_t)c * N + n] != 0;
-      inf = constrain<M>(raw, pcr, dc.ch);
-    }
+    int8_t* col = i_raw + (size_t)c * G * N + n;
+    warp_load_state<M>(dc, pack, col, waner, c, n, pcr, lane, raw, inf, w);
     const M raw_in = raw;
     const int w_in = w;
     const M vac = reinterpret_cast<const M*>(dc.vac)[n];
@@ -106,14 +77,14 @@ k_gibbs_blk(const DevCohort dc, const int* __restrict__ order, const int C,
     const uint4 rnd = philox4x32_10(
         make_uint4((uint32_t)lane, (uint32_t)n + dc.ind_offset, (uint32_t)c + dc.chain_offset, (uint32_t)cfg.sweep),
         make_uint2((uint32_t)cfg.seed, (uint32_t)(cfg.seed >> 32) ^ (uint32_t)(cfg.sweep >> 32)));
-    const double pv = s_th[21], lp1 = s_th[19], lp0 = s_th[20];
+    const double pv = s_th[TH_P], lp1 = s_th[TH_LOG_P], lp0 = s_th[TH_LOG1M_P];
     const M fresh = __ballot_sync(FULL, lane < G && u01(rnd.x) <= pv);
     const double u_cat = u01(rnd.y);
 
     for (int k = 0; k < dc.ch.n; ++k) {
       const M cm = (M)dc.ch.mask[k];
       if (cm == 0) continue;
-      ++n_prop;
+      ++q.n_prop;
       if (pcr & cm) {  // the chunk is the PCR+ column: its raw bits are free
         raw = (raw & ~cm) | (fresh & cm);
         continue;
@@ -123,15 +94,7 @@ k_gibbs_blk(const DevCohort dc, const int* __restrict__ order, const int C,
       const M inf_own = constrain<M>(base | ((lane < len) ? ((M)1 << (c0 + lane)) : (M)0), pcr, dc.ch);
       const M inf_none = __shfl_sync(FULL, inf_own, len);
       const double ll_none = (inf_none == inf) ? ll : indiv_ll(inf_none, w);
-      double llv = ll_none;  // lane o: log-likelihood under option o
-      for (int o = 0; o < len; ++o) {
-        const M io = __shfl_sync(FULL, inf_own, o);
-        const M diff = io ^ inf_none;
-        if (diff != 0 && ctz(diff) <= t_last) {  // otherwise the data cannot tell it from "none"
-          const double v = (io == inf) ? ll : indiv_ll(io, w);
-          if (lane == o) llv = v;
-        }
-      }
+      const double llv = chunk_options_ll<M>(inf_own, len, inf_none, ll_none, inf, w, ll, t_last, lane, indiv_ll);
       // categorical draw over the len + 1 options: inclusive scan of exp(log weight - max)
       double lw = (lane < len) ? llv + (double)lane * lp0 + lp1 : llv + (double)len * lp0;
       if (lane > len || !(lw == lw)) lw = -INFINITY;
@@ -154,7 +117,7 @@ k_gibbs_blk(const DevCohort dc, const int* __restrict__ order, const int C,
         newbits = bit | (fresh & cm & ~((bit << 1) - 1));
       }
       const M new_first = newbits & (~newbits + 1);
-      if (new_first != old_first) ++n_acc;
+      if (new_first != old_first) ++q.n_acc;
       raw = base | newbits;
       inf = __shfl_sync(FULL, inf_own, pick);
       ll = __shfl_sync(FULL, llv, pick);
@@ -162,40 +125,22 @@ k_gibbs_blk(const DevCohort dc, const int* __restrict__ order, const int C,
 
     // ---- waner: exact conditional ----
     {
-      ++n_prop;
-      const M ex = inf | vac;
-      const bool affected = ex != 0 && ctz(ex | top_bit<M>()) < t_last_s;
-      double d10 = s_th[16], ll2 = ll;
-      if (affected) {
-        ll2 = indiv_ll(inf, w ^ 1);
-        d10 += w ? (ll - ll2) : (ll2 - ll);  // log-odds of 1 versus 0
-      }
+      ++q.n_prop;
+      double d10, ll2;
+      waner_logodds<M>(inf, vac, w, ll, t_last_s, s_th, indiv_ll, d10, ll2);
       const double p1 = 1.0 / (1.0 + exp(-d10));
       const int w_new = (__shfl_sync(FULL, u01(rnd.z), 0) <= p1) ? 1 : 0;
       if (w_new != w) {
         w = w_new;
         rows.set_w(vac, w);
         ll = ll2;
-        ++n_acc;
+        ++q.n_acc;
       }
     }
 
-    {  // write back only what changed
-      const M changed = raw ^ raw_in;
-      if (lane < G && ((changed >> lane) & 1)) col[(size_t)lane * N] = (int8_t)((raw >> lane) & 1);
-      if (lane == 0 && w != w_in) waner[(size_t)c * N + n] = (int8_t)w;
-      if (pack && lane == 0 && (changed != 0 || w != w_in)) {
-        PackedState<M> ps;
-        ps.rw = raw | (w ? top_bit<M>() : (M)0);
-        ps.inf = inf;
-        pack[(size_t)c * N + n] = ps;
-      }
-    }
+    warp_store_state<M>(dc, pack, col, waner, c, n, lane, raw, raw_in, w, w_in, inf);
   }
-  if (cfg.stats && lane == 0 && cur_c >= 0) {
-    atomicAdd(&cfg.stats[(size_t)cur_c * 2], (unsigned long long)n_prop);
-    atomicAdd(&cfg.stats[(size_t)cur_c * 2 + 1], (unsigned long long)n_acc);
-  }
+  q.flush(lane);
 }
 
 }  // namespace

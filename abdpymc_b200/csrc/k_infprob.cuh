@@ -71,24 +71,9 @@ k_infprob_accum(const DevCohort dc, const int* __restrict__ order, const int C, 
     __syncthreads();
     if (!active) continue;
 
-    M raw = 0, inf;
+    M raw, inf;
     int w;
-    if (pack) {
-      const PackedState<M> ps = pack[(size_t)c * N + n];
-      raw = ps.rw & ~top_bit<M>();
-      w = (ps.rw & top_bit<M>()) != 0;
-      inf = ps.inf;
-    } else {
-      const int8_t* col = i_raw + (size_t)c * G * N + n;
-#pragma unroll
-      for (int s = 0; s < NSLOT; ++s) {
-        const int t = lane + 32 * s;
-        const int8_t b = (t < G) ? col[(size_t)t * N] : (int8_t)0;
-        raw |= (M)__ballot_sync(FULL, b != 0) << (32 * s);
-      }
-      w = waner[(size_t)c * N + n] != 0;
-      inf = constrain<M>(raw, pcr, dc.ch);
-    }
+    warp_load_state<M>(dc, pack, i_raw + (size_t)c * G * N + n, waner, c, n, pcr, lane, raw, inf, w);
     GibbsRows<M> rows(dc, n, lane, s_th, s_pw, s_tab);
     const int t_last = rows.t_last;
     rows.set_w(vac, w);
@@ -115,7 +100,7 @@ k_infprob_accum(const DevCohort dc, const int* __restrict__ order, const int C, 
         const int b1 = (int)((inf1 >> t) & 1), b0 = (int)((inf0 >> t) & 1);
         double v = (double)b1;
         if (b1 != b0) {
-          const double d = s_th[15] + (cur ? ll - ll_alt : ll_alt - ll);  // log-odds of raw_t = 1 versus 0
+          const double d = s_th[TH_LOGIT_P] + (cur ? ll - ll_alt : ll_alt - ll);  // log-odds of raw_t = 1 versus 0
           const double p1 = 1.0 / (1.0 + exp(-d));
           v = (p1 == p1) ? (b1 ? p1 : 1.0 - p1) : (double)((inf >> t) & 1);
         }
@@ -123,7 +108,7 @@ k_infprob_accum(const DevCohort dc, const int* __restrict__ order, const int C, 
       }
     } else {
       // ---- time chunks: the position of the chunk's first raw 1, or none ----
-      const double lp1 = s_th[19], lp0 = s_th[20];
+      const double lp1 = s_th[TH_LOG_P], lp0 = s_th[TH_LOG1M_P];
       for (int k = 0; k < dc.ch.n; ++k) {
         const M cm = chunk_mask<M>(dc.ch, k);
         if (cm == 0) continue;
@@ -149,16 +134,8 @@ k_infprob_accum(const DevCohort dc, const int* __restrict__ order, const int C, 
           if (32 * g >= len) continue;
           const int o_own = 32 * g + lane;
           const M inf_own = (o_own < len) ? constrain<M>(base | ((M)1 << (c0 + o_own)), pcr, dc.ch) : inf_none;
-          double llv = ll_none;
-          const int n_in = min(32, len - 32 * g);
-          for (int j = 0; j < n_in; ++j) {
-            const M io = shfl_mask(inf_own, j);
-            const M diff = io ^ inf_none;
-            if (diff != 0 && ctz(diff) <= t_last) {  // otherwise the data cannot tell it from "none"
-              const double v = (io == inf) ? ll : indiv_ll(io, w);
-              if (lane == j) llv = v;
-            }
-          }
+          const double llv =
+              chunk_options_ll<M>(inf_own, min(32, len - 32 * g), inf_none, ll_none, inf, w, ll, t_last, lane, indiv_ll);
           double lw = (o_own < len) ? llv + (double)o_own * lp0 + lp1 : -INFINITY;
           if (!(lw == lw)) lw = -INFINITY;
           double gm = lw;
@@ -192,11 +169,8 @@ k_infprob_accum(const DevCohort dc, const int* __restrict__ order, const int C, 
 
     // ---- waner ----
     {
-      const M ex = inf | vac;
-      double p1 = s_th[18];
-      if (ex != 0 && ctz(ex | top_bit<M>()) < rows.t_last_s) {
-        const double ll2 = indiv_ll(inf, w ^ 1);
-        const double d10 = s_th[16] + (w ? ll - ll2 : ll2 - ll);  // log-odds of 1 versus 0
+      double d10, ll2, p1 = s_th[TH_SIG_PW];
+      if (waner_logodds<M>(inf, vac, w, ll, rows.t_last_s, s_th, indiv_ll, d10, ll2)) {
         p1 = 1.0 / (1.0 + exp(-d10));
         if (!(p1 == p1)) p1 = (double)w;
       }

@@ -232,10 +232,8 @@ k_pack(const DevCohort dc, const int8_t* __restrict__ i_raw, const int8_t* __res
   const int G = dc.G, N = dc.N;
   if (n >= N) return;
   const M raw = load_column<M>(i_raw + (size_t)c * G * N + n, G, N);
-  PackedState<M> ps;
-  ps.inf = constrain<M>(raw, reinterpret_cast<const M*>(dc.pcr)[n], dc.ch);
-  ps.rw = raw | (waner[(size_t)c * N + n] != 0 ? top_bit<M>() : (M)0);
-  pack[(size_t)c * N + n] = ps;
+  const M inf = constrain<M>(raw, reinterpret_cast<const M*>(dc.pcr)[n], dc.ch);
+  pack[(size_t)c * N + n] = PackedState<M>(raw, waner[(size_t)c * N + n] != 0, inf);
 }
 
 // pinned host memory -> device memory by the SMs (see copy_state_h2d); n16 16-byte words + rem bytes

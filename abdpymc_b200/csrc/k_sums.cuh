@@ -370,12 +370,12 @@ k_sums(const DevCohort dc, const TileDesc* __restrict__ tiles, const SumsCfg cfg
       // resident state, packed (PackedState): one coalesced 8 / 16-byte load per individual, the
       // constraints were applied when the state was written
       const PackedState<M> ps = pack[(size_t)c * N + i0 + tid];
-      const M w = ps.rw & top_bit<M>();
+      const M w = ps.waner_bit();
       IndState<M> st;
       st.inf = ps.inf;
       st.vacw = my_vac | w;
       s_ind[tid] = st;
-      cnt_i = (double)popc(ps.rw & ~top_bit<M>());
+      cnt_i = (double)popc(ps.raw());
       cnt_w = w ? 1.0 : 0.0;
     } else if (tid < ni) {
       // (unpredicated loads, all in flight: see load_column; without them the column costs 5 memory round trips)
